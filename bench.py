@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- utterances/sec of the SIF hot path (embed + PC removal) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[3], SURVEY.md §8d "Config 4", the shape the roofline is
@@ -19,6 +19,10 @@ measured HBM copy bandwidth; `cpu_baseline` = the oracle port of the reference's
 sklearn path timed on this box's host cores (bounded sample).
 
 `--impl reference` times that CPU port instead (rank 0 only) and prints the same line shape.
+
+`--dump-outputs DIR` writes what the last timed step returned, after the timed region, as float32 .npy
+files (see dump_outputs).  The inputs depend only on the arguments and the MMB_BENCH_* variables, so two
+builds run with the same ones can be compared output for output.
 """
 import argparse
 import json
@@ -414,6 +418,33 @@ def verify_run(ctx):
     return {'ok': int(flag.item()) == 0, 'rank0': checks, 'ranks_failed': int(flag.item()), 'failed': failed}
 
 
+DUMP_ROWS = 32768      # 32768 x 300 float32 = 39 MB: the whole N x d output would be 12 GB
+
+
+def dump_rows(n):
+    """The embedding rows --dump-outputs writes: a fixed, seeded sample of the n global rows, ascending."""
+    rng = np.random.default_rng(0)
+    return np.sort(rng.choice(n, size=min(DUMP_ROWS, n), replace=False))
+
+
+def dump_outputs(out_dir, emb, pc, lo, world, rank):
+    """Write the last timed step's outputs under out_dir: pc.npy, the (npc, d) principal component, and
+    embeddings.npy, the projected embedding rows dump_rows(N_UTT) of the (N, d) result, both float32.  With
+    several ranks each rank contributes the sampled rows of its shard and rank 0 writes."""
+    import torch.distributed as dist
+    rows = dump_rows(N_UTT)
+    mine = rows[(rows >= lo) & (rows < lo + emb.shape[0])] - lo
+    part = emb[torch.as_tensor(mine, device=emb.device)].cpu().numpy()
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, part)
+        part = np.concatenate(parts)              # shards are contiguous in rank order: rows stay ascending
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, 'embeddings.npy'), part.astype(np.float32))
+        np.save(os.path.join(out_dir, 'pc.npy'), pc.cpu().numpy().astype(np.float32))
+
+
 def mmb_secondary(steps=50):
     """SURVEY.md 8(d) secondary metric, recorded by the driver's own bench run: one MMB2 latent-optimisation
     step (heads -> word + 6 Gaussian terms -> backward -> SGD) at the MOSI and the real-POM layouts, as this
@@ -447,7 +478,13 @@ def main():
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-verify', action='store_true')
     ap.add_argument('--no-secondary', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one returned to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the GPU path\'s outputs; --impl reference has none')
     args.warmup = max(args.warmup, 0)
     # stdout carries exactly ONE JSON line: keep the real stdout for it and point fd 1 at stderr, so that
     # whatever else writes to fd 1 (NCCL's version banner at NCCL_DEBUG >= VERSION, library prints, the
@@ -545,6 +582,8 @@ def main():
     ms_per_step = float(t.item()) / args.steps
     value = N_UTT / (ms_per_step * 1e-3)
     clocks = sampler.window(t_wall0, t_wall1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, emb, pc, lo, world, rank)
 
     # ---- end to end: pinned host ids in, float32 embeddings out, copies inside the region --
     e2e = None

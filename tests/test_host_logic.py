@@ -255,9 +255,10 @@ def test_id_dataset_and_moment_batches_keep_the_reference_tuple_layout():
     assert isinstance(data['text'], losses.TokenIds) and isinstance(data['textaudio'].parts[0], losses.MomentStats)
 
 
-def test_loaders_read_the_reference_file_layout(tmp_path, monkeypatch):
+def test_loaders_read_the_reference_file_layout(tmp_path, monkeypatch, golden_dir):
     """utils.load_data and its parts (reference utils.py:10-128): the id / vocabulary / table files by their
-    reference paths, the h5 splits through h5py (a stand-in module here: the image has no h5py)."""
+    reference paths, the h5 splits through h5py (a stand-in module here: the image has no h5py), and the real
+    POM id matrices (kept in tests/golden/sif_pom_full.npz) laid out as the reference ships them."""
     import pickle
     import sys
     import types
@@ -305,11 +306,15 @@ def test_loaders_read_the_reference_file_layout(tmp_path, monkeypatch):
         utils.load_data({'dataset': 'nope'})
     with pytest.raises(FileNotFoundError):
         utils.load_data({'dataset': 'iemocap', 'emotion': 'happy', 'data_root': str(root)})
-    ref_root = '/root/reference'
-    if os.path.exists(os.path.join(ref_root, 'pom', 'pom_test_ids.npy')):       # the real fixtures, when present
-        v, t = utils.load_text_ids('pom', ref_root, ('valid', 'test'))
-        assert v.shape == (100, 1089) and t.shape == (203, 1357) and t.dtype == np.int64
-        assert max(utils.load_word2ix('mosi', ref_root).values()) == 3015
+    g = np.load(os.path.join(golden_dir, 'sif_pom_full.npz'))
+    real = tmp_path / 'real'
+    (real / 'pom').mkdir(parents=True)
+    for s in ('valid', 'test'):
+        np.save(real / 'pom' / ('pom_%s_ids.npy' % s), g[s + '_ids'].astype(np.int64))
+    v, t = utils.load_text_ids('pom', str(real), ('valid', 'test'))
+    assert v.shape == (100, 1089) and t.shape == (203, 1357) and t.dtype == np.int64
+    np.testing.assert_array_equal(v, g['valid_ids'])
+    np.testing.assert_array_equal(t, g['test_ids'])
 
 
 def test_batched_regressors_equal_sequential_ones(capsys):

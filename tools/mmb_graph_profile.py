@@ -1,5 +1,5 @@
 import os, sys
-ROOT = '/root/repo'
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'multimodal-baselines_b200')); sys.path.insert(0, os.path.join(ROOT, 'tools'))
 import torch, bench_mmb as bm, models, simplesif, utils
 name = os.environ.get('SHAPE', 'mosi')
