@@ -115,6 +115,20 @@ MMB_API int mmb_sif_embed_ws(const float* table, int64_t V, int d, const float* 
                              int64_t N, int64_t L, float* emb, int* status, void* ws, size_t ws_bytes,
                              mmb_stream_t stream);
 
+/* SIF sweep: seq2weight + get_weighted_average (sif_functions.py:8-15, 28-56) for K vocabulary-weight vectors
+ * over one gather of the table rows.  vocab_w is (K, V) row-major; emb is (K, N, d), so every emb[k] is a dense
+ * (N, d) matrix that mmb_gram / mmb_remove_pc take as it is.  emb[k] is bit-identical to mmb_sif_embed with
+ * vocab_w = vocab_w[k] (the general kernel, not the pre-scaled one of mmb_sif_embed_ws): the same variant rule,
+ * duplicate-row merging, summation order and per-vector divisor count_nonzero(w_k[i, :]).  Negative ids wrap
+ * and weigh 0 for every k; ids outside [-V, V) set MMB_STATUS_BAD_INDEX.  Rows are read once per group of up to
+ * Kg vectors (Kg = 8 for d <= 256, 4 for d <= 512, 2 for d <= 1024); any K >= 1 runs as ceil(K / Kg) passes.
+ * ws: mmb_sif_embed_multi_workspace_bytes(V, K) bytes, 32-byte aligned (the weights, laid out per token);
+ * too small a ws is MMB_E_INVALID.  The kernel of the last call is mmb_last_kernel(1).                  */
+MMB_API size_t mmb_sif_embed_multi_workspace_bytes(int64_t V, int K);
+MMB_API int mmb_sif_embed_multi(const float* table, int64_t V, int d, const float* vocab_w, int K, const int64_t* x,
+                                int64_t N, int64_t L, float* emb, int* status, void* ws, size_t ws_bytes,
+                                mmb_stream_t stream);
+
 /* get_weighted_average + the Gram that compute_pc needs (sif_functions.py:28-67) of one block in one call.
  * With option "overlap_sms" = S > 0 (mmb_set_option; default 0) the Gram is taken BESIDE the embed: the block
  * is cut into "overlap_chunks" chunks and chunk c's tcgen05 Gram runs on S SMs from an internal

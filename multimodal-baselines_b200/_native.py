@@ -43,6 +43,8 @@ SIGNATURES = {
     'mmb_sif_embed': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _p, _p, _p]),
     'mmb_sif_embed_workspace_bytes': (_sz, [_i64, _i, _i64, _i64]),
     'mmb_sif_embed_ws': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _p, _p, _p, _sz, _p]),
+    'mmb_sif_embed_multi_workspace_bytes': (_sz, [_i64, _i]),
+    'mmb_sif_embed_multi': (_i, [_p, _i64, _i, _p, _i, _p, _i64, _i64, _p, _p, _p, _sz, _p]),
     'mmb_sif_embed_gram_workspace_bytes': (_sz, [_i64, _i, _i64, _i64, _i]),
     'mmb_sif_embed_gram': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _p, _p, _p, _p, _sz, _i, _p]),
     'mmb_sif_embed_ragged': (_i, [_p, _i64, _i, _p, _p, _p, _i64, _i64, _i64, _p, _p, _p]),

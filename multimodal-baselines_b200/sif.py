@@ -1,7 +1,8 @@
 """Drop-in for the reference's ``sif.py`` (SURVEY.md §2 #2, §8 row A5): word weights and
 ``get_sentence_embeddings``, the call ``simplesif.main`` makes per split (reference
 simplesif.py:296-311).  The embedding itself runs through ``mmb_sif_embedding_host`` /
-``mmb_sif_embedding`` of libmmb_b200.so.
+``mmb_sif_embedding`` of libmmb_b200.so.  ``get_sentence_embeddings_sweep`` (no reference counterpart) does the
+same for K word-weight vectors and several numbers of removed components in one gather (``mmb_sif_embed_multi``).
 """
 import ctypes as C
 import os
@@ -12,6 +13,7 @@ import torch
 import _native as nv
 from _native import lib
 from sif_functions import Params, seq2weight, SIF_embedding, start_block, sif_embedding_device  # noqa: F401
+from sif_functions import sif_embedding_sweep  # noqa: F401
 from sif_functions import RaggedIds, sif_embedding_ragged, to_ragged  # noqa: F401
 
 # ---- word weights a / (a + p(w)) (host-side file handling; the arithmetic that matters runs in the kernels) ----
@@ -130,3 +132,45 @@ def get_sentence_embeddings(word_embeddings, weights, text, out=None):
                                         nv.np_ptr(omega), nv.np_ptr(out), int(out.dtype == np.float64),
                                         None, nv.GRAM_AUTO, 0))
     return out
+
+
+def get_sentence_embeddings_sweep(word_embeddings, weights, text, npcs=(1,)):
+    """``get_sentence_embeddings`` for K word-weight vectors at once (e.g. ``get_word_weights(file, a)`` for
+    several ``a``) and P numbers of removed principal components: ``out[k, j]`` is the SIF embedding with
+    ``weights[k]`` and ``npcs[j]`` components removed (0 = the raw weighted average).  The table rows are
+    gathered once for all K vectors (``sif_functions.sif_embedding_sweep``).
+
+    ``weights`` is a (K, V) array or a sequence of K vectors; a vector shorter than the table is padded with
+    zeros, and an id beyond it raises ``IndexError``, as in ``get_sentence_embeddings``.  NumPy in -> float64
+    (K, P, N, d) NumPy out; CUDA tensors in -> float32 CUDA tensor out.  The ids are uploaded once and the
+    result downloaded once."""
+    dev = nv.require_cuda()
+    as_np = not (isinstance(text, torch.Tensor) and text.is_cuda)
+    table_t = nv.to_device(word_embeddings, torch.float32, dev)
+    V, d = table_t.shape
+    if isinstance(weights, torch.Tensor):
+        vecs = [weights.reshape(-1)] if weights.dim() == 1 else list(weights)
+    elif isinstance(weights, np.ndarray) and weights.ndim == 2:
+        vecs = list(weights)
+    else:
+        vecs = [weights] if np.ndim(weights[0]) == 0 else list(weights)
+    if as_np:
+        ids = np.ascontiguousarray(np.asarray(text), dtype=np.int64)
+        if ids.ndim != 2:
+            raise ValueError('text must be (n_samples, seq_len)')
+        ids_t = nv.to_device(ids, torch.int64, dev)
+        id_max = int(ids.max()) if ids.size else None
+    else:
+        ids_t = text.contiguous()
+        id_max = int(ids_t.max().item()) if ids_t.numel() else None
+    rows = []
+    for vec in vecs:
+        w_t = nv.to_device(vec if isinstance(vec, torch.Tensor) else np.asarray(vec).reshape(-1),
+                           torch.float32, dev).reshape(-1)
+        if w_t.numel() < V:
+            if id_max is not None and id_max >= w_t.numel():
+                raise IndexError('index %d is out of bounds for axis 0 with size %d' % (id_max, w_t.numel()))
+            w_t = torch.cat([w_t, w_t.new_zeros(V - w_t.numel())])
+        rows.append(w_t[:V])
+    out = sif_embedding_sweep(table_t, torch.stack(rows).contiguous(), ids_t, npcs=npcs)
+    return out.double().cpu().numpy() if as_np else out

@@ -6,6 +6,9 @@ the arithmetic runs in libmmb_b200.so (hand-written sm_100a CUDA behind the C AB
 include/mmb_b200.h).  NumPy in -> NumPy out, like the reference; every function also takes
 CUDA torch tensors and then returns a CUDA tensor without touching the host.
 
+``sif_embedding_sweep`` (no reference counterpart) embeds with K word-weight vectors over one gather and
+removes several numbers of principal components: a sweep over SIF's ``a`` and ``npc``.
+
 There is no CPU fallback: without the built library or without a CUDA device these raise.
 """
 import numpy as np
@@ -16,7 +19,7 @@ from _native import lib
 
 __all__ = ['seq2weight', 'Params', 'get_weighted_average', 'compute_pc', 'remove_pc',
            'SIF_embedding', 'start_block', 'gram', 'pc_from_gram', 'project_out',
-           'sif_embedding_device', 'RaggedIds', 'to_ragged', 'sif_embedding_ragged']
+           'sif_embedding_device', 'sif_embedding_sweep', 'RaggedIds', 'to_ragged', 'sif_embedding_ragged']
 
 
 def _is_np(*xs):
@@ -239,6 +242,54 @@ def sif_embedding_device(table_t, vocab_w_t, ids_t, npc=1, gram_mode=nv.GRAM_AUT
     if check:
         nv.raise_on_status(st, V)
     return (emb, pc) if return_pc else emb
+
+
+def sif_embedding_sweep(table_t, vocab_w_t, ids_t, npcs=(1,), gram_mode=nv.GRAM_AUTO):
+    """SIF embeddings for K word-weight vectors x P principal-component counts (a sweep over the smoothing
+    constant ``a`` of ``a / (a + p(w))`` and over ``npc``).  All arguments are CUDA tensors: table (V, d) f32,
+    vocab_w (K, V) f32, ids (N, L) int64.  Returns float32 (K, P, N, d), P = ``len(npcs)``.
+
+    One ``mmb_sif_embed_multi`` call gathers every token's row once for all K weight vectors (``emb[k]`` is bit
+    for bit ``mmb_sif_embed`` with ``vocab_w[k]``); then per k one Gram, and per (k, npc) one ``pc_from_gram``
+    (with that k's own start block when N < d) and one projection.  ``npc = 0`` is the raw weighted average.
+    With a single ``npc`` the projection runs in place: peak memory is the (K, N, d) output."""
+    npcs = tuple(int(p) for p in npcs)
+    if not npcs:
+        raise ValueError('npcs must name at least one number of components')
+    for p in npcs:
+        if p < 0 or p + 10 > 32:
+            raise ValueError('npc must be in 0..22')
+    if vocab_w_t.dim() != 2 or ids_t.dim() != 2:
+        raise ValueError('vocab_w must be (K, V) and ids (n_samples, seq_len)')
+    n, L = ids_t.shape
+    V, d = table_t.shape
+    K = vocab_w_t.shape[0]
+    if vocab_w_t.shape[1] != V:
+        raise ValueError('vocab_w has %d columns, the table %d rows' % (vocab_w_t.shape[1], V))
+    dev = table_t.device
+    emb = torch.empty((K, n, d), dtype=torch.float32, device=dev)
+    st = _status(dev)
+    nbytes = lib.mmb_sif_embed_multi_workspace_bytes(V, K)
+    ws = torch.empty(max(nbytes, 32), dtype=torch.uint8, device=dev)
+    nv.check(lib.mmb_sif_embed_multi(nv.ptr(table_t), V, d, nv.ptr(vocab_w_t), K, nv.ptr(ids_t), n, L, nv.ptr(emb),
+                                     nv.ptr(st), nv.ptr(ws), nbytes, nv.stream_ptr()))
+    nv.raise_on_status(st, V)
+    del ws
+    in_place = len(npcs) == 1
+    out = emb.unsqueeze(1) if in_place else torch.empty((K, len(npcs), n, d), dtype=torch.float32, device=dev)
+    if n == 0:
+        return out
+    for k in range(K):
+        E = emb[k]
+        G = gram(E, gram_mode) if any(npcs) else None
+        for j, p in enumerate(npcs):
+            if p == 0:
+                if not in_place:
+                    out[k, j].copy_(E)
+                continue
+            pc = pc_from_gram(G, p, n, X_t=E)
+            project_out(E, pc, out=out[k, j])
+    return out
 
 
 # --------------------------------------------------------------------------- ragged ids (SURVEY.md 8f N3)
