@@ -70,14 +70,6 @@ MMB_API int mmb_device_info(int* sm_count, int* cc_major, int* cc_minor);
  * mmb_weighted_average).  bench.py derives `gpu_launches` and `roofline.kernel` from these. */
 MMB_API unsigned long long mmb_launch_count(void);
 MMB_API const char* mmb_last_kernel(int tag);
-/* Run-time switches for experiments and tests (the defaults are what the benchmarks use):
- *   "embed_prescale"  1 (default) / 0: fold the vocabulary weights into a scratch table for large batches
- *   "embed_hot"       0 / 1: the tensor-core hot-row embed path for very large batches (d = 300)
- *   "embed_warm"      K in 0..512: keep only the K most frequent rows cacheable in L1 (experiment, 0 = off)
- *   "overlap_sms"     S: SMs given to the Gram beside the embed in mmb_sif_embed_gram (0 = off, default)
- *   "overlap_chunks"  chunks per call of that pipeline (2..64, default 10)
- *   "overlap_grid"    embed CTAs per SM of that pipeline (4..256, default 32)                          */
-MMB_API int mmb_set_option(const char* name, int value);
 /* Pinned host memory for the *_host entry points and for e2e benchmarks. */
 MMB_API int mmb_host_alloc(void** ptr, size_t bytes);
 /* Write-combined pinned memory: for buffers the host only WRITES and the device reads (the ids of the
@@ -128,20 +120,6 @@ MMB_API size_t mmb_sif_embed_multi_workspace_bytes(int64_t V, int K);
 MMB_API int mmb_sif_embed_multi(const float* table, int64_t V, int d, const float* vocab_w, int K, const int64_t* x,
                                 int64_t N, int64_t L, float* emb, int* status, void* ws, size_t ws_bytes,
                                 mmb_stream_t stream);
-
-/* get_weighted_average + the Gram that compute_pc needs (sif_functions.py:28-67) of one block in one call.
- * With option "overlap_sms" = S > 0 (mmb_set_option; default 0) the Gram is taken BESIDE the embed: the block
- * is cut into "overlap_chunks" chunks and chunk c's tcgen05 Gram runs on S SMs from an internal
- * higher-priority stream while chunk c + 1 is embedded on the others.  Measured slower than one stage after
- * the other on a B200 (33.6 vs 31.4 ms per 10 M utterances, tools/overlap_probe.py), hence off: the call is
- * then mmb_sif_embed_ws followed by mmb_gram.  emb (N, d) and G (d, d) = emb^T emb are complete when the
- * work enqueued on `stream` by this call completes; chunk Grams are added in chunk order (deterministic,
- * within 2e-6 relative of mmb_gram's grouping).
- * ws: mmb_sif_embed_gram_workspace_bytes(V, d, N, L, gram_mode) bytes, 256-byte aligned.               */
-MMB_API size_t mmb_sif_embed_gram_workspace_bytes(int64_t V, int d, int64_t N, int64_t L, int gram_mode);
-MMB_API int mmb_sif_embed_gram(const float* table, int64_t V, int d, const float* vocab_w, const int64_t* x,
-                               int64_t N, int64_t L, float* emb, int* status, float* G, void* ws,
-                               size_t ws_bytes, int gram_mode, mmb_stream_t stream);
 
 /* Ragged (CSR) ids, SURVEY.md 8f N3 -- the same result as mmb_sif_embed on the right-padded (N, L_pad)
  * matrix the reference builds (utils.py:77-80; sif_functions.py:28-56), without walking the padding:

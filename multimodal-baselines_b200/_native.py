@@ -32,7 +32,6 @@ SIGNATURES = {
     'mmb_version': (_i, []),
     'mmb_last_error': (C.c_char_p, []),
     'mmb_device_info': (_i, [C.POINTER(_i)] * 3),
-    'mmb_set_option': (_i, [C.c_char_p, _i]),
     'mmb_launch_count': (C.c_ulonglong, []),
     'mmb_last_kernel': (C.c_char_p, [_i]),
     'mmb_host_alloc': (_i, [C.POINTER(_p), _sz]),
@@ -45,8 +44,6 @@ SIGNATURES = {
     'mmb_sif_embed_ws': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _p, _p, _p, _sz, _p]),
     'mmb_sif_embed_multi_workspace_bytes': (_sz, [_i64, _i]),
     'mmb_sif_embed_multi': (_i, [_p, _i64, _i, _p, _i, _p, _i64, _i64, _p, _p, _p, _sz, _p]),
-    'mmb_sif_embed_gram_workspace_bytes': (_sz, [_i64, _i, _i64, _i64, _i]),
-    'mmb_sif_embed_gram': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _p, _p, _p, _p, _sz, _i, _p]),
     'mmb_sif_embed_ragged': (_i, [_p, _i64, _i, _p, _p, _p, _i64, _i64, _i64, _p, _p, _p]),
     'mmb_ids_lengths': (_i, [_p, _i64, _i64, _i64, _p, _p, _p]),
     'mmb_ids_compact': (_i, [_p, _i64, _i64, _p, _p, _p]),

@@ -3,7 +3,6 @@
 #include <stdarg.h>
 #include <string.h>
 
-#include <mutex>
 #include <vector>
 
 #include "common.cuh"
@@ -36,42 +35,6 @@ void note_kernel(int tag, const char* name) {
   strncpy(g_last_kernel[tag], name, sizeof(g_last_kernel[tag]) - 1);
 }
 
-// Run-time switches (mmb_set_option); -1 = unset -> the environment variable / built-in default decides.
-static int g_opt_embed_hot = -1, g_opt_embed_prescale = -1, g_opt_embed_warm = -1;
-static int g_opt_overlap_sms = -1, g_opt_overlap_chunks = -1, g_opt_overlap_grid = -1;
-static int env_int(const char* name, int dflt) { return getenv(name) ? atoi(getenv(name)) : dflt; }
-// Gram beside the embed (mmb_sif_embed_gram): SMs given to the Gram (0 = no overlap, one stage after the other),
-// chunks per call, embed CTAs per SM.
-static int option_overlap_sms() {
-  static const int env = env_int("MMB_OVERLAP_SMS", 0);   // measured slower than one stage after the other: off
-  return g_opt_overlap_sms >= 0 ? g_opt_overlap_sms : env;
-}
-static int option_overlap_chunks() {
-  static const int env = env_int("MMB_OVERLAP_CHUNKS", 10);
-  const int v = g_opt_overlap_chunks > 0 ? g_opt_overlap_chunks : env;
-  return v < 2 ? 2 : (v > 64 ? 64 : v);
-}
-static int option_overlap_grid() {
-  static const int env = env_int("MMB_OVERLAP_GRID", 32);
-  const int v = g_opt_overlap_grid > 0 ? g_opt_overlap_grid : env;
-  return v < 4 ? 4 : (v > 256 ? 256 : v);
-}
-int option_embed_warm() {
-  if (g_opt_embed_warm >= 0) return g_opt_embed_warm;
-  static const int env = getenv("MMB_EMBED_WARM") ? atoi(getenv("MMB_EMBED_WARM")) : 0;
-  return env < 0 ? 0 : (env > 512 ? 512 : env);
-}
-int option_embed_hot() {
-  if (g_opt_embed_hot >= 0) return g_opt_embed_hot;
-  static const int env = getenv("MMB_EMBED_HOT") ? atoi(getenv("MMB_EMBED_HOT")) : 0;
-  return env;
-}
-int option_embed_prescale() {
-  if (g_opt_embed_prescale >= 0) return g_opt_embed_prescale;
-  static const int env = getenv("MMB_EMBED_PRESCALE") ? atoi(getenv("MMB_EMBED_PRESCALE")) : 1;
-  return env;
-}
-
 int sm_count() {
   static thread_local int cached_dev = -1, cached = 148;
   int dev = 0;
@@ -90,7 +53,7 @@ int sm_count() {
 size_t gram_fp32_workspace_bytes(int64_t N, int d);
 int gram_fp32(const float* X, int64_t N, int d, float* G, void* ws, size_t ws_bytes, cudaStream_t st);
 size_t gram_tc_workspace_bytes(int64_t N, int d);
-int gram_tc(const float* X, int64_t N, int d, float* G, void* ws, size_t ws_bytes, cudaStream_t st, int max_cta = 0);
+int gram_tc(const float* X, int64_t N, int d, float* G, void* ws, size_t ws_bytes, cudaStream_t st);
 bool gram_tc_supported(int64_t N, int d);
 
 static int resolve_gram_mode(int64_t N, int d, int mode) {
@@ -116,28 +79,13 @@ __global__ void f32_to_f64_kernel(const float* __restrict__ in, double* __restri
 
 using namespace mmb;
 
-extern "C" int mmb_version(void) { return 100; }
+extern "C" int mmb_version(void) { return 101; }
 
 extern "C" const char* mmb_last_error(void) { return g_err; }
 
 extern "C" unsigned long long mmb_launch_count(void) { return __atomic_load_n(&g_launches, __ATOMIC_RELAXED); }
 
 extern "C" const char* mmb_last_kernel(int tag) { return (tag >= 0 && tag < 8) ? g_last_kernel[tag] : ""; }
-
-extern "C" int mmb_set_option(const char* name, int value) {
-  MMB_REQUIRE(name, "null pointer");
-  if (!strcmp(name, "embed_hot")) g_opt_embed_hot = value;
-  else if (!strcmp(name, "embed_prescale")) g_opt_embed_prescale = value;
-  else if (!strcmp(name, "embed_warm")) g_opt_embed_warm = value < 0 ? 0 : (value > 512 ? 512 : value);
-  else if (!strcmp(name, "overlap_sms")) g_opt_overlap_sms = value;
-  else if (!strcmp(name, "overlap_chunks")) g_opt_overlap_chunks = value;
-  else if (!strcmp(name, "overlap_grid")) g_opt_overlap_grid = value;
-  else {
-    set_error("mmb_set_option: unknown option '%s'", name);
-    return MMB_E_INVALID;
-  }
-  return MMB_OK;
-}
 
 extern "C" int mmb_device_info(int* sm, int* cc_major, int* cc_minor) {
   int dev = 0;
@@ -199,112 +147,8 @@ extern "C" int mmb_gram(const float* X, int64_t N, int d, float* G, void* ws, si
 namespace mmb {   // implemented in sif_embed.cu
 int sif_prescale(const float* table, int64_t V, int d, const float* vocab_w, void* ws, cudaStream_t st);
 int sif_embed_prescaled(const float* table, int64_t V, int d, const float* vocab_w, const void* ws, const int64_t* x,
-                        int64_t N, int64_t L, float* emb, int* status, cudaStream_t st, int grid_mult = 8);
+                        int64_t N, int64_t L, float* emb, int* status, cudaStream_t st);
 }  // namespace mmb
-
-
-// ---- embed + Gram of a block, the Gram of chunk c beside the embed of chunk c + 1 (experiment, OFF by default) --
-// Idea: the embed is bound by the L2->SM fabric, the tcgen05 Gram by the tensor pipe and shared memory of the SMs
-// it runs on, so on DISJOINT SMs the two should barely compete.  The block is cut into chunks; chunk c's Gram runs
-// on `overlap_sms` SMs (one persistent CTA each, launched first from a higher-priority stream so that it gets its
-// SMs at the chunk boundary -- a Gram CTA's registers and shared memory leave no room for an embed CTA beside it,
-// so the partition is the block scheduler's own) while chunk c + 1 is embedded on the others; only the last
-// chunk's Gram (whole GPU) is exposed.  Chunk Grams are added in chunk order: deterministic.
-// Measured (tools/overlap_probe.py, profiles/r02_overlap_probe.jsonl, 10 M utterances): 31.4 ms one stage after
-// the other, 33.6 ms at best overlapped (40 SMs, 5 chunks) -- the embed slows down in proportion to the SMs it
-// loses (its per-SM L1 pipe is at 75 % too), so a partition of the SMs cannot win.  overlap_sms = 0 keeps
-// mmb_sif_embed_ws + mmb_gram; the entry point stays for the probe.
-namespace {
-struct SideStream {
-  cudaStream_t st = nullptr;
-};
-SideStream g_side[64];
-
-int side_stream(cudaStream_t* out) {
-  static std::mutex mu;
-  std::lock_guard<std::mutex> lock(mu);
-  int dev = 0;
-  MMB_CUDA(cudaGetDevice(&dev));
-  MMB_REQUIRE(dev >= 0 && dev < 64, "device ordinal out of range");
-  if (!g_side[dev].st) {
-    int lo = 0, hi = 0;
-    MMB_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));   // hi = numerically lowest = greatest priority
-    MMB_CUDA(cudaStreamCreateWithPriority(&g_side[dev].st, cudaStreamNonBlocking, hi));
-  }
-  *out = g_side[dev].st;
-  return MMB_OK;
-}
-struct EventPair {
-  cudaEvent_t fork = nullptr, join = nullptr;
-  int init() {
-    MMB_CUDA(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
-    MMB_CUDA(cudaEventCreateWithFlags(&join, cudaEventDisableTiming));
-    return MMB_OK;
-  }
-  ~EventPair() {
-    if (fork) cudaEventDestroy(fork);
-    if (join) cudaEventDestroy(join);
-  }
-};
-}  // namespace
-
-static bool embed_gram_overlaps(int64_t V, int d, int64_t N, int64_t L, int gram_mode) {
-  if (option_overlap_sms() <= 0 || option_overlap_sms() >= sm_count()) return false;
-  if (resolve_gram_mode(N, d, gram_mode) != MMB_GRAM_TF32X3 || !gram_tc_supported(N, d)) return false;
-  if (mmb_sif_embed_workspace_bytes(V, d, N, L) == 0) return false;
-  return N >= (int64_t)option_overlap_chunks() * 32768;     // chunks long enough to amortise their boundaries
-}
-
-extern "C" size_t mmb_sif_embed_gram_workspace_bytes(int64_t V, int d, int64_t N, int64_t L, int gram_mode) {
-  return align_up(mmb_sif_embed_workspace_bytes(V, d, N, L)) + align_up(mmb_gram_workspace_bytes(N > 0 ? N : 1, d, gram_mode)) +
-         align_up((size_t)d * d * sizeof(float));
-}
-
-extern "C" int mmb_sif_embed_gram(const float* table, int64_t V, int d, const float* vocab_w, const int64_t* x,
-                                  int64_t N, int64_t L, float* emb, int* status, float* G, void* ws, size_t ws_bytes,
-                                  int gram_mode, mmb_stream_t stream) {
-  MMB_REQUIRE(table && vocab_w && x && emb && status && G && ws, "null pointer");
-  MMB_REQUIRE(N > 0, "empty block");
-  MMB_REQUIRE(ws_bytes >= mmb_sif_embed_gram_workspace_bytes(V, d, N, L, gram_mode), "workspace too small");
-  MMB_REQUIRE((uintptr_t)ws % 256 == 0, "ws must be 256-byte aligned");
-  const size_t scaled_bytes = mmb_sif_embed_workspace_bytes(V, d, N, L);
-  const size_t gram_bytes = align_up(mmb_gram_workspace_bytes(N, d, gram_mode));
-  char* ws_scaled = (char*)ws;
-  char* ws_gram = ws_scaled + align_up(scaled_bytes);
-  float* gchunk = (float*)(ws_gram + gram_bytes);
-  cudaStream_t st = as_stream(stream);
-  if (!embed_gram_overlaps(V, d, N, L, gram_mode)) {
-    int rc = mmb_sif_embed_ws(table, V, d, vocab_w, x, N, L, emb, status, ws_scaled, scaled_bytes, stream);
-    if (rc) return rc;
-    return mmb_gram(emb, N, d, G, ws_gram, gram_bytes, gram_mode, stream);
-  }
-  MMB_REQUIRE(((uintptr_t)table % 16 == 0) && ((uintptr_t)emb % 16 == 0), "table / emb must be 16-byte aligned");
-  cudaStream_t side;
-  int rc = side_stream(&side);
-  if (rc) return rc;
-  EventPair ev;
-  if ((rc = ev.init())) return rc;
-  const int nch = option_overlap_chunks(), gram_sms = option_overlap_sms(), grid_mult = option_overlap_grid();
-  const int64_t chunk = ceil_div(ceil_div(N, (int64_t)nch), (int64_t)16) * 16;
-  if ((rc = sif_prescale(table, V, d, vocab_w, ws_scaled, st))) return rc;
-  for (int64_t r0 = 0, c = 0; r0 < N; r0 += chunk, ++c) {
-    const int64_t rows = (N - r0) < chunk ? (N - r0) : chunk;
-    const bool last = r0 + rows >= N;
-    rc = sif_embed_prescaled(table, V, d, vocab_w, ws_scaled, x + r0 * L, rows, L, emb + r0 * d, status, st, grid_mult);
-    if (rc) return rc;
-    MMB_CUDA(cudaEventRecord(ev.fork, st));
-    MMB_CUDA(cudaStreamWaitEvent(side, ev.fork, 0));
-    rc = gram_tc(emb + r0 * d, rows, d, c == 0 ? G : gchunk, ws_gram, gram_bytes, side, last ? 0 : gram_sms);
-    if (rc) return rc;
-    if (c > 0) {
-      accumulate_kernel<<<(d * d + 255) / 256, 256, 0, side>>>(G, gchunk, d * d, 0);
-      MMB_LAUNCH_CHECK("accumulate");
-    }
-  }
-  MMB_CUDA(cudaEventRecord(ev.join, side));
-  MMB_CUDA(cudaStreamWaitEvent(st, ev.join, 0));
-  return MMB_OK;
-}
 
 struct SifWs {
   size_t gram, pc, s0, G, pcv, total;

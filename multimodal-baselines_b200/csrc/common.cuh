@@ -26,9 +26,6 @@ int sm_count();
 // instead of asserting a constant.
 void count_launch(const char* name);
 void note_kernel(int tag, const char* name);
-int option_embed_hot();        // 1: the tensor-core hot-row embed path for very large batches (sif_embed_hot.cu)
-int option_embed_warm();       // K > 0: keep only the K most frequent rows cacheable in L1 (sif_embed_prescaled_warm_kernel)
-int option_embed_prescale();   // 0: never fold the weights into a scratch table (always the general kernel)
 
 #define MMB_LAUNCH_CHECK(name)                                    \
   do {                                                            \
@@ -86,12 +83,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
       "}" ::"r"(bar), "r"(parity) : "memory");
 }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-// 1-D bulk copy global -> shared (TMA engine, no tensor map): src, dst and bytes 16-byte aligned;
-// completion is signalled on `bar` as `bytes` of transaction count.
-__device__ __forceinline__ void bulk_copy_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
 
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 

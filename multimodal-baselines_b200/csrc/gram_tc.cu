@@ -17,19 +17,19 @@
 //              pipe idled whenever a flush put the workers behind.  The MMA ignores the low 13 mantissa bits of its FP32
 //              operands (verified bit-for-bit on B200), so "hi" is the raw TMA tile.
 //   MMA      : one elected thread issues tcgen05.mma (M = 128) for the upper-triangular blocks
-//                 tile A  rows   0..127 x cols   0..303   (N = 256 + 48)   TMEM cols   0..303
+//                 tile A  rows   0..127 x cols   0..303   (N = 160 + 144)  TMEM cols   0..303
 //                 tile B  rows 128..255 x cols 128..303   (N = 176)        TMEM cols 304..479
 //              with three products (hi*lo, hi*hi, lo*hi) per 8-row K step: 18 MMAs per stage, issued BY A TILE
 //              (hi rows 0..127 x {lo, hi}, hi rows 128..255 x {lo, hi}, lo rows 0..127 x hi, lo rows 128..255 x
 //              hi) with .collector::a::fill/use/lastuse, so an A tile is fetched from shared memory once per
-//              K step instead of once per MMA; tile A's 304 columns go as N = 160 + 144.  (Shared-memory
+//              K step instead of once per MMA.  (Shared-memory
 //              bandwidth -- operand fetch + the workers below -- is what bounds this kernel.)
 //   block C  : the remaining 44x44 block (rows/cols 256..299) does not fit in the 512 TMEM
 //              columns next to A and B (it would need 48 more), so the worker warps compute
 //              it on the CUDA cores in exact FP32 from the raw tile, 4x4 register blocks.
 //   flush    : the tensor core adds each MMA into the FP32 accumulator with truncation, a bias
 //              of ~1e-7 per MMA that grows linearly with the K chain (measured 1e-4 relative
-//              over 6.7 k rows); every `seg` stages (default 64 = 1024 rows) the workers drain
+//              over 6.7 k rows); every kSeg = 64 stages (1024 rows) the workers drain
 //              TMEM (tcgen05.ld) into the CTA's FP32 partial tile in global memory (L2-resident,
 //              column-major so that lane = row gives coalesced lines) with round-to-nearest
 //              adds, which bounds the bias at ~2e-5 relative.  The partial is read and written with an
@@ -55,16 +55,11 @@ constexpr int kBoxBytes = kBK * 128;            // one box: kBK rows x 128 B
 constexpr int kHiBytes = kBoxes * kBoxBytes;    // 20480
 constexpr int kStageBytes = 2 * kHiBytes;       // hi + lo
 constexpr int kSmemBytes = kStages * kStageBytes + 1024 /*align*/ + 256 /*barriers*/;
-constexpr int kSegDefault = 64;                 // 1024 rows between TMEM flushes
+constexpr int kSeg = 64;                        // K blocks (1024 rows) accumulated in TMEM between two flushes
 constexpr int kThreads = 320;                   // warp0 TMA, warp1 MMA, warps 2-5 split + TMEM flush, warps 6-9 corner block
 constexpr int kColsAB = 480, kColsC = 48;
 constexpr int kPartialStride = 128 * kColsAB + kColsC * kColsC;   // floats per CTA: tiles A|B, then block C
 
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-      ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar) : "memory");
-}
 __device__ __forceinline__ void tma_load_2d_hint(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar,
                                                  uint64_t policy) {
   asm volatile(
@@ -167,13 +162,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
 struct Params {
   int64_t N;
   int n_cta;
-  int passes;         // 3 = 3xTF32, 1 = plain TF32 (debug)
-  int seg;            // K blocks accumulated in TMEM between two flushes to the FP32 partial
-  int prefetch;       // K blocks of L2 prefetch distance (0 = off)
-  int opt;            // bit 0: flush skips warp-chunks below the diagonal; bit 1: L2 eviction hints (X evict_first,
-                      // partial evict_last); bit 2: block C pairs packed into full warps; bit 3: tile A's 304
-                      // columns as N = 160 + 144 instead of 256 + 48
-  int collect;        // 1: A-sharing MMA order with collector reuse hints; 0: pass order
   uint32_t lbo, sbo;  // descriptor strides in bytes
   float* partial;
 };
@@ -200,7 +188,7 @@ __global__ void __launch_bounds__(kThreads, 1)
   int64_t kb1 = kb0 + per;
   if (kb1 > kblocks) kb1 = kblocks;
   const int64_t nkb = kb1 > kb0 ? kb1 - kb0 : 0;
-  const int64_t nseg = (nkb + prm.seg - 1) / prm.seg;
+  const int64_t nseg = (nkb + kSeg - 1) / kSeg;
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < kStages; ++s) {
@@ -229,29 +217,18 @@ __global__ void __launch_bounds__(kThreads, 1)
       for (int64_t i = 0; i < nkb; ++i) {
         const int s = (int)(i % kStages);
         const uint32_t ph = (uint32_t)((i / kStages) & 1);
-        if (prm.prefetch > 0 && i + prm.prefetch < nkb) {   // warm L2 ahead of the ring
-          const int prow = (int)((kb0 + i + prm.prefetch) * kBK);
-          for (int b = 0; b < kBoxes; ++b)
-            asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(&tmap),
-                         "r"(b * 32), "r"(prow) : "memory");
-        }
         mbar_wait(bar_empty + 8 * s, ph ^ 1);
         mbar_expect_tx(bar_full + 8 * s, (uint32_t)kHiBytes);
         const uint32_t dst = smem_base + s * kStageBytes;
         const int row = (int)((kb0 + i) * kBK);
-        if (prm.opt & 2) {
-          for (int b = 0; b < kBoxes; ++b)
-            tma_load_2d_hint(dst + b * kBoxBytes, &tmap, b * 32, row, bar_full + 8 * s, pol_stream);
-        } else {
-          for (int b = 0; b < kBoxes; ++b)
-            tma_load_2d(dst + b * kBoxBytes, &tmap, b * 32, row, bar_full + 8 * s);
-        }
+        for (int b = 0; b < kBoxes; ++b)
+          tma_load_2d_hint(dst + b * kBoxBytes, &tmap, b * 32, row, bar_full + 8 * s, pol_stream);
       }
     }
   } else if (warp == 1) {
     // ===== MMA issuer =====
     if (lane == 0) {
-      constexpr uint32_t idesc256 = make_idesc(128, 256), idesc48 = make_idesc(128, 48),
+      constexpr uint32_t idesc160 = make_idesc(128, 160), idesc144 = make_idesc(128, 144),
                          idesc176 = make_idesc(128, 176);
       const uint32_t blk = prm.lbo;  // byte distance between 32-column blocks
       const uint64_t dbase = make_desc(0, prm.lbo, prm.sbo);
@@ -261,7 +238,7 @@ __global__ void __launch_bounds__(kThreads, 1)
           mbar_wait(bar_free, (uint32_t)((sg - 1) & 1));
           tc_fence_after();
         }
-        int64_t iend = i + prm.seg;
+        int64_t iend = i + kSeg;
         if (iend > nkb) iend = nkb;
         bool first = true;
         for (; i < iend; ++i) {
@@ -273,55 +250,24 @@ __global__ void __launch_bounds__(kThreads, 1)
 #pragma unroll
           for (int ks = 0; ks < kBK / 8; ++ks) {
             const uint32_t koff = ks * 1024;  // 8 K rows = two 4-row swizzle atoms of 512 B
-            if (prm.passes == 3 && prm.collect != 0) {
-              // The nine MMAs of a K step ordered by A tile, so that each of the four A tiles (hi / lo x rows
-              // 0..127 / 128..255) is fetched from shared memory once instead of 9 times in total: the A
-              // collector keeps it across the MMAs that share it.  Sums are the same terms in another order.
-              const uint32_t z = (first && ks == 0) ? 0u : 1u;
-              const uint64_t h0 = desc_at(dbase, hi + koff), h4 = desc_at(dbase, hi + koff + 4 * blk),
-                             h8 = desc_at(dbase, hi + koff + 8 * blk);
-              const uint64_t l0 = desc_at(dbase, lo + koff), l4 = desc_at(dbase, lo + koff + 4 * blk),
-                             l8 = desc_at(dbase, lo + koff + 8 * blk);
-              if (prm.opt & 8) {
-                // tile A's 304 columns as N = 160 + 144 instead of 256 + 48: no 24-clock MMA between the long
-                // ones (-2.6 %, same bits)
-                constexpr uint32_t idesc160 = make_idesc(128, 160), idesc144 = make_idesc(128, 144);
-                const uint64_t h5 = desc_at(dbase, hi + koff + 5 * blk), l5 = desc_at(dbase, lo + koff + 5 * blk);
-                umma_tf32_c<kCollectFill>(tmem + 0, h0, l0, idesc160, z);
-                umma_tf32_c<kCollectUse>(tmem + 160, h0, l5, idesc144, z);
-                umma_tf32_c<kCollectUse>(tmem + 0, h0, h0, idesc160, 1u);
-                umma_tf32_c<kCollectLastUse>(tmem + 160, h0, h5, idesc144, 1u);
-                umma_tf32_c<kCollectFill>(tmem + 304, h4, l4, idesc176, z);
-                umma_tf32_c<kCollectLastUse>(tmem + 304, h4, h4, idesc176, 1u);
-                umma_tf32_c<kCollectFill>(tmem + 0, l0, h0, idesc160, 1u);
-                umma_tf32_c<kCollectLastUse>(tmem + 160, l0, h5, idesc144, 1u);
-                umma_tf32_c<kCollectDiscard>(tmem + 304, l4, h4, idesc176, 1u);
-              } else {
-                umma_tf32_c<kCollectFill>(tmem + 0, h0, l0, idesc256, z);        // hi[0:128]   x lo[0:256]
-                umma_tf32_c<kCollectUse>(tmem + 256, h0, l8, idesc48, z);        //             x lo[256:304]
-                umma_tf32_c<kCollectUse>(tmem + 0, h0, h0, idesc256, 1u);        //             x hi[0:256]
-                umma_tf32_c<kCollectLastUse>(tmem + 256, h0, h8, idesc48, 1u);   //             x hi[256:304]
-                umma_tf32_c<kCollectFill>(tmem + 304, h4, l4, idesc176, z);      // hi[128:256] x lo[128:304]
-                umma_tf32_c<kCollectLastUse>(tmem + 304, h4, h4, idesc176, 1u);  //             x hi[128:304]
-                umma_tf32_c<kCollectFill>(tmem + 0, l0, h0, idesc256, 1u);       // lo[0:128]   x hi[0:256]
-                umma_tf32_c<kCollectLastUse>(tmem + 256, l0, h8, idesc48, 1u);   //             x hi[256:304]
-                umma_tf32_c<kCollectDiscard>(tmem + 304, l4, h4, idesc176, 1u);  // lo[128:256] x hi[128:304]
-              }
-              continue;
-            }
-            for (int p = 0; p < prm.passes; ++p) {
-              // small terms first (lo*hi, hi*lo), then hi*hi; the MMA ignores the low 13
-              // mantissa bits of its FP32 operands, so "hi" is the raw TMA tile.
-              const uint32_t abase = ((prm.passes == 3 && p == 0) ? lo : hi) + koff;
-              const uint32_t bbase = ((prm.passes == 3 && p == 1) ? lo : hi) + koff;
-              const uint32_t acc = (first && ks == 0 && p == 0) ? 0u : 1u;
-              const uint64_t a0 = desc_at(dbase, abase), a4 = desc_at(dbase, abase + 4 * blk);
-              const uint64_t b0 = desc_at(dbase, bbase), b4 = desc_at(dbase, bbase + 4 * blk),
-                             b8 = desc_at(dbase, bbase + 8 * blk);
-              umma_tf32(tmem + 0, a0, b0, idesc256, acc);     // rows 0..127   x cols 0..255
-              umma_tf32(tmem + 256, a0, b8, idesc48, acc);    // rows 0..127   x cols 256..303
-              umma_tf32(tmem + 304, a4, b4, idesc176, acc);   // rows 128..255 x cols 128..303
-            }
+            // The nine MMAs of a K step ordered by A tile, so that each of the four A tiles (hi / lo x rows
+            // 0..127 / 128..255) is fetched from shared memory once instead of 9 times in total: the A
+            // collector keeps it across the MMAs that share it.  Tile A's 304 columns go as N = 160 + 144
+            // rather than 256 + 48: no 24-clock MMA between the long ones (-2.6 %, same bits).
+            const uint32_t z = (first && ks == 0) ? 0u : 1u;
+            const uint64_t h0 = desc_at(dbase, hi + koff), h4 = desc_at(dbase, hi + koff + 4 * blk),
+                           h5 = desc_at(dbase, hi + koff + 5 * blk);
+            const uint64_t l0 = desc_at(dbase, lo + koff), l4 = desc_at(dbase, lo + koff + 4 * blk),
+                           l5 = desc_at(dbase, lo + koff + 5 * blk);
+            umma_tf32_c<kCollectFill>(tmem + 0, h0, l0, idesc160, z);          // hi[0:128]   x lo[0:160]
+            umma_tf32_c<kCollectUse>(tmem + 160, h0, l5, idesc144, z);         //             x lo[160:304]
+            umma_tf32_c<kCollectUse>(tmem + 0, h0, h0, idesc160, 1u);          //             x hi[0:160]
+            umma_tf32_c<kCollectLastUse>(tmem + 160, h0, h5, idesc144, 1u);    //             x hi[160:304]
+            umma_tf32_c<kCollectFill>(tmem + 304, h4, l4, idesc176, z);        // hi[128:256] x lo[128:304]
+            umma_tf32_c<kCollectLastUse>(tmem + 304, h4, h4, idesc176, 1u);    //             x hi[128:304]
+            umma_tf32_c<kCollectFill>(tmem + 0, l0, h0, idesc160, 1u);         // lo[0:128]   x hi[0:160]
+            umma_tf32_c<kCollectLastUse>(tmem + 160, l0, h5, idesc144, 1u);    //             x hi[160:304]
+            umma_tf32_c<kCollectDiscard>(tmem + 304, l4, h4, idesc176, 1u);    // lo[128:256] x hi[128:304]
           }
           first = false;
           umma_commit(bar_empty + 8 * s);   // frees the stage when these MMAs have read it
@@ -339,7 +285,7 @@ __global__ void __launch_bounds__(kThreads, 1)
     const uint64_t pol_keep = l2_policy_evict_last();   // the partial is re-read at every flush: keep it in L2
     int64_t i = 0;
     for (int64_t sg = 0; sg < nseg; ++sg) {
-      int64_t iend = i + prm.seg;
+      int64_t iend = i + kSeg;
       if (iend > nkb) iend = nkb;
       for (; i < iend; ++i) {
         const int s = (int)(i % kStages);
@@ -371,36 +317,21 @@ __global__ void __launch_bounds__(kThreads, 1)
       for (int c = 0; c < kColsAB; c += 32) {
         // warp-chunks entirely below the diagonal are never read by the reduce kernel: tile A (rows 32 q ..,
         // columns c ..) when c + 32 <= 32 q; tile B (rows 128 + 32 q .., columns 128 + c - 304 ..) likewise
-        if ((prm.opt & 1) && (c + 32 <= 32 * q || (c >= 320 && c - 304 + 32 <= 32 * q))) continue;
+        if (c + 32 <= 32 * q || (c >= 320 && c - 304 + 32 <= 32 * q)) continue;
         float* o = outT + (size_t)c * 128;
         float old[32];
         uint32_t r[32];
-        if (prm.opt & 2) {
-          if (sg > 0) {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) old[j] = ld_hint(o + (size_t)j * 128, pol_keep);
-          }
-          tmem_ld32(tmem + ((uint32_t)(q * 32) << 16) + c, r);
-          if (sg == 0) {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) st_hint(o + (size_t)j * 128, __uint_as_float(r[j]), pol_keep);
-          } else {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) st_hint(o + (size_t)j * 128, old[j] + __uint_as_float(r[j]), pol_keep);
-          }
-          continue;
-        }
         if (sg > 0) {
 #pragma unroll
-          for (int j = 0; j < 32; ++j) old[j] = o[(size_t)j * 128];
+          for (int j = 0; j < 32; ++j) old[j] = ld_hint(o + (size_t)j * 128, pol_keep);
         }
         tmem_ld32(tmem + ((uint32_t)(q * 32) << 16) + c, r);
         if (sg == 0) {
 #pragma unroll
-          for (int j = 0; j < 32; ++j) o[(size_t)j * 128] = __uint_as_float(r[j]);
+          for (int j = 0; j < 32; ++j) st_hint(o + (size_t)j * 128, __uint_as_float(r[j]), pol_keep);
         } else {
 #pragma unroll
-          for (int j = 0; j < 32; ++j) o[(size_t)j * 128] = old[j] + __uint_as_float(r[j]);
+          for (int j = 0; j < 32; ++j) st_hint(o + (size_t)j * 128, old[j] + __uint_as_float(r[j]), pol_keep);
         }
       }
       tc_fence_before();
@@ -413,9 +344,9 @@ __global__ void __launch_bounds__(kThreads, 1)
     // ===== corner warps: block C (rows/cols 256..299, does not fit in TMEM) in exact FP32 from the
     // raw tile; 11 x 11 grid of 4x4 blocks, upper triangle (66 pairs), dealt round-robin =====
     float* part = prm.partial + (size_t)blockIdx.x * kPartialStride;
-    // pair index: dealt over the four warps, or (opt bit 2) packed into two full warps + 2 lanes -- the cost of a
+    // pair index: packed into two full warps + 2 lanes rather than dealt over the four warps -- the cost of a
     // warp-wide LDS.128 here is its 2-3 shared-memory wavefronts whatever the number of active lanes
-    const int pidx = (prm.opt & 4) ? (warp - 6) * 32 + lane : lane * 4 + (warp - 6);
+    const int pidx = (warp - 6) * 32 + lane;
     int ti = 0, tj = 0;
     const bool has_c = pidx < 66;
     if (has_c) {
@@ -546,10 +477,9 @@ static EncodeTiledFn encode_fn() {
   return fn;
 }
 
-static int plan(int64_t N, int max_cta = 0) {
+static int plan(int64_t N) {
   const int64_t kblocks = (N + kBK - 1) / kBK;
-  int sms = sm_count();
-  if (max_cta > 0 && max_cta < sms) sms = max_cta;   // leave the other SMs to a concurrent kernel (api.cu)
+  const int sms = sm_count();
   return (int)(kblocks < sms ? (kblocks > 0 ? kblocks : 1) : sms);
 }
 
@@ -572,12 +502,11 @@ size_t gram_tc_workspace_bytes(int64_t N, int d) {
   return (size_t)tc::plan(N) * tc::kPartialStride * sizeof(float);
 }
 
-static int gram_tc_main(const float* X, int64_t N, int d, void* ws, size_t ws_bytes, cudaStream_t st, int* n_cta_out,
-                        int max_cta = 0) {
+static int gram_tc_main(const float* X, int64_t N, int d, void* ws, size_t ws_bytes, cudaStream_t st, int* n_cta_out) {
   using namespace tc;
   MMB_REQUIRE(d == kD, "tcgen05 Gram is specialised for d == 300");
   MMB_REQUIRE(N < ((int64_t)1 << 31) - 64, "N too large for 32-bit TMA coordinates");
-  const int n_cta = plan(N, max_cta);
+  const int n_cta = plan(N);
   MMB_REQUIRE(ws_bytes >= (size_t)n_cta * kPartialStride * sizeof(float), "workspace too small");
   EncodeTiledFn enc = encode_fn();
   if (!enc) {
@@ -604,18 +533,8 @@ static int gram_tc_main(const float* X, int64_t N, int d, void* ws, size_t ws_by
   Params prm;
   prm.N = N;
   prm.n_cta = n_cta;
-  prm.passes = 3;
-  prm.seg = kSegDefault;
-  prm.prefetch = 0;     // measured: L2 prefetch ahead of the 5-stage ring does not help
   prm.lbo = kBoxBytes;  // 32-column blocks are kBK*128 bytes apart
   prm.sbo = 512;        // 4-row K atoms (4 x 128 B) are 512 bytes apart
-  if (const char* e = getenv("MMB_TC_PASSES")) prm.passes = atoi(e) == 1 ? 1 : 3;
-  if (const char* e = getenv("MMB_TC_SEG")) prm.seg = atoi(e) > 0 ? atoi(e) : kSegDefault;
-  if (const char* e = getenv("MMB_TC_PREFETCH")) prm.prefetch = atoi(e);
-  prm.opt = 15;         // measured (tools/gram_probe.py, profiles/r02_gram_probe.jsonl): each of the four helps
-  if (const char* e = getenv("MMB_TC_OPT")) prm.opt = atoi(e);
-  prm.collect = 1;      // A-sharing MMA order + collector hints: -4 ... -7 % (same probe)
-  if (const char* e = getenv("MMB_TC_COLLECT")) prm.collect = atoi(e);
   prm.partial = (float*)ws;
   gram_tc_kernel<<<n_cta, kThreads, kSmemBytes, st>>>(tmap, prm);
   MMB_LAUNCH_CHECK("gram_tc");
@@ -623,11 +542,10 @@ static int gram_tc_main(const float* X, int64_t N, int d, void* ws, size_t ws_by
   return MMB_OK;
 }
 
-// max_cta > 0: at most that many CTAs (= SMs; one persistent CTA per SM), for a Gram that runs beside another kernel.
-int gram_tc(const float* X, int64_t N, int d, float* G, void* ws, size_t ws_bytes, cudaStream_t st, int max_cta) {
+int gram_tc(const float* X, int64_t N, int d, float* G, void* ws, size_t ws_bytes, cudaStream_t st) {
   using namespace tc;
   int n_cta = 0;
-  const int rc = gram_tc_main(X, N, d, ws, ws_bytes, st, &n_cta, max_cta);
+  const int rc = gram_tc_main(X, N, d, ws, ws_bytes, st, &n_cta);
   if (rc) return rc;
   gram_tc_reduce_kernel<<<(kD * kD + 255) / 256, 256, 0, st>>>((const float*)ws, n_cta, G);
   MMB_LAUNCH_CHECK("gram_tc_reduce");

@@ -188,7 +188,7 @@ __global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
 
 template <int NCH, bool EXPLICIT_W, int UNROLL, int MINB, bool WIDE>
 __global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
-    sif_embed_warp_kernel(const float4* __restrict__ table4, int V, int d4, int stride4,
+    sif_embed_warp_kernel(const float4* __restrict__ table4, int V, int d4,
                           const float* __restrict__ wsrc, const int64_t* __restrict__ ids,
                           int64_t N, int64_t L, float4* __restrict__ emb4,
                           int* __restrict__ status) {
@@ -196,7 +196,7 @@ __global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
   const int64_t warp0 = (int64_t)blockIdx.x * kEmbedWarps + (threadIdx.x >> 5);
   const int64_t nwarps = (int64_t)gridDim.x * kEmbedWarps;
   const char* lane_base = (const char*)(table4 + lane);
-  const unsigned row_bytes = (unsigned)stride4 * 16u;   // table row pitch (>= d4 float4)
+  const unsigned row_bytes = (unsigned)d4 * 16u;
   const typename Live<NCH>::type tail = make_live<NCH>(lane, d4);
   bool bad = false;
   for (int64_t i = warp0; i < N; i += nwarps) {
@@ -316,114 +316,6 @@ __global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
             fma_row<NCH>(acc, vv, (float)(pj >> kRowBits), tail);
           }
         }
-      }
-    }
-    store_row<NCH>(emb4 + (size_t)i * d4, acc, cnt, lane, d4);
-  }
-  if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, MMB_STATUS_BAD_INDEX);
-}
-
-// The same kernel with an L1 allocation policy per row.  After the pre-scale the kernel is bound by the L2 -> SM
-// fabric (ncu r02b: 25 KB per utterance at 11.2 TB/s = 91 % of the LTS cap): every row that misses L1 crosses it,
-// and under LRU the cold rows (each read once, 10 lines) keep evicting the few hundred warm rows that would be
-// read again.  A sample histogram of the ids (sif_embed_hot.cu: hot_hist / hot_select) names the K most frequent
-// rows; each CTA keeps a 64 Kbit Bloom filter of them in shared memory, and rows that are NOT in it are loaded with
-// ld.global.nc.L1::no_allocate (SASS LDG.E.NA): the L1 is left to the rows that will hit again.  Results are
-// bit-identical to sif_embed_prescaled_kernel (only the cache policy differs).
-constexpr int kBloomWords = 2048;      // 8 KB per CTA
-constexpr int kWarmRowBits = 25;       // row index below 2^25, multiplicity (<= 32) in 6 bits, warm flag in bit 31
-__device__ __forceinline__ unsigned bloom_hash(unsigned row) { return (row * 2654435761u) >> 16; }
-
-template <int NCH>
-__device__ __forceinline__ void load_row_na(float4 (&v)[NCH], const char* __restrict__ lane_base, size_t off,
-                                            typename Live<NCH>::type live) {
-  const float4* p = (const float4*)(lane_base + off);
-#pragma unroll
-  for (int c = 0; c < NCH; ++c)
-    if (chunk_on<NCH>(live, c))
-      asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];"
-                   : "=f"(v[c].x), "=f"(v[c].y), "=f"(v[c].z), "=f"(v[c].w) : "l"(p + 32 * c));
-}
-
-template <int NCH, int UNROLL, int MINB>
-__global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
-    sif_embed_prescaled_warm_kernel(const float4* __restrict__ tp4, int V, int d4, const int* __restrict__ flags,
-                                    const int* __restrict__ warm_ids, int n_warm, const int64_t* __restrict__ ids,
-                                    int64_t N, int64_t L, float4* __restrict__ emb4, int* __restrict__ status) {
-  if (__ldg(flags) & 1) return;        // a zero vocabulary weight: the general kernel behind this one runs
-  __shared__ unsigned bloom[kBloomWords];
-  for (int i = threadIdx.x; i < kBloomWords; i += blockDim.x) bloom[i] = 0u;
-  __syncthreads();
-  for (int i = threadIdx.x; i < n_warm; i += blockDim.x) {
-    const int id = __ldg(warm_ids + i);
-    if (id >= 0) {
-      const unsigned h = bloom_hash((unsigned)id);
-      atomicOr(&bloom[h >> 5], 1u << (h & 31u));
-    }
-  }
-  __syncthreads();
-  const int lane = threadIdx.x & 31;
-  const int64_t warp0 = (int64_t)blockIdx.x * kEmbedWarps + (threadIdx.x >> 5);
-  const int64_t nwarps = (int64_t)gridDim.x * kEmbedWarps;
-  const char* lane_base = (const char*)(tp4 + lane);
-  const unsigned row_bytes = (unsigned)d4 * 16u;
-  const typename Live<NCH>::type tail = make_live<NCH>(lane, d4);
-  constexpr unsigned kRowMask = (1u << kWarmRowBits) - 1u;
-  bool bad = false;
-  int64_t nid = (warp0 < N && lane < L) ? __ldcs(ids + warp0 * L + lane) : 0;
-  for (int64_t i = warp0; i < N; i += nwarps) {
-    RowAcc<NCH> acc;
-    acc.clear();
-    int cnt = 0;
-    for (int64_t base = 0; base < L; base += 32) {
-      const int64_t id = nid;
-      const bool same = base + 32 < L;
-      const int64_t ni = same ? i : i + nwarps;
-      const int64_t nb = same ? base + 32 : 0;
-      nid = (ni < N && nb + lane < L) ? __ldcs(ids + ni * L + nb + lane) : 0;
-      int row = -1;
-      bool counts = false;
-      unsigned warm = 0u;
-      if (base + lane < L) {
-        const int64_t r = id < 0 ? id + V : id;
-        if (r >= 0 && r < V) {
-          row = (int)r;
-          counts = id >= 0;
-          const unsigned h = bloom_hash((unsigned)row);
-          warm = (bloom[h >> 5] >> (h & 31u)) & 1u;
-        } else {
-          bad = true;
-        }
-      }
-      const unsigned nn = __ballot_sync(0xffffffffu, counts);
-      cnt += __popc(nn);
-      const unsigned grp = __match_any_sync(0xffffffffu, row);
-      const bool head = (row >= 0) && (lane == __ffs(grp) - 1);
-      const unsigned packed = (unsigned)row | ((unsigned)__popc(grp & nn) << kWarmRowBits) | (warm << 31);
-      unsigned heads = __ballot_sync(0xffffffffu, head);
-      while (heads) {
-        int j[UNROLL];
-        int n = 0;
-#pragma unroll
-        for (int u = 0; u < UNROLL; ++u) {
-          j[u] = heads ? (__ffs(heads) - 1) : 0;
-          if (heads) { heads &= heads - 1; ++n; }
-        }
-        float mj[UNROLL];
-        float4 v[UNROLL][NCH];
-#pragma unroll
-        for (int u = 0; u < UNROLL; ++u) {
-          if (u < n) {
-            const unsigned pj = __shfl_sync(0xffffffffu, packed, j[u]);
-            mj[u] = (float)((pj >> kWarmRowBits) & 63u);
-            const unsigned off = (pj & kRowMask) * row_bytes;
-            if (pj >> 31) load_row<NCH>(v[u], lane_base, off, tail);       // warm: keep it in L1
-            else load_row_na<NCH>(v[u], lane_base, off, tail);             // cold: do not displace the warm rows
-          }
-        }
-#pragma unroll
-        for (int u = 0; u < UNROLL; ++u)
-          if (u < n) fma_row<NCH>(acc, v[u], mj[u], tail);
       }
     }
     store_row<NCH>(emb4 + (size_t)i * d4, acc, cnt, lane, d4);
@@ -652,26 +544,16 @@ static int launch_embed(const float* table, int64_t V, int d, const float* wsrc,
         (const float4*)table, (int)V, d4, wsrc, ids, N, L, (float4*)emb, status);
   } else {
     // Persistent-style grid: a multiple of the SM count, grid-stride over utterances.
-    int64_t blocks = ceil_div(N, kEmbedWarps);
-    int64_t cap = (int64_t)sms * 8;
-    int grid = (int)(blocks < cap ? blocks : cap);
-    // default: ids of the next chunk prefetched (variant 6) for the fused lookup; measured on B200, 4 M
-    // utterances: 11.83 ms plain (variant 0) -> 11.56 ms; also prefetching the next chunk's weight lookups
-    // (two chunks ahead) spills at the 64-register budget and takes 16.5 ms -- not kept
-    static const int variant = getenv("MMB_EMBED_VARIANT") ? atoi(getenv("MMB_EMBED_VARIANT")) : (EXPLICIT_W ? 0 : 6);
-    static const int waves = getenv("MMB_EMBED_WAVES") ? atoi(getenv("MMB_EMBED_WAVES")) : 8;
-    cap = (int64_t)sms * waves;
-    grid = (int)(blocks < cap ? blocks : cap);
+    const int64_t blocks = ceil_div(N, kEmbedWarps);
+    const int grid = (int)(blocks < (int64_t)sms * 8 ? blocks : (int64_t)sms * 8);
     // Row pitch = d (dense table).  A 128-byte-aligned pitch (1280 B at d = 300) was measured on
     // B200 and changes nothing (11.88 vs 11.93 ms per 4 M utterances): the L1 wavefront count is
     // not sensitive to where the 512-byte warp reads start.
-    const float* tbl = table;
-    const int stride4 = d4;
-    const bool wide = (uint64_t)V * (uint64_t)stride4 * 16u >= ((uint64_t)1 << 32);
+    const bool wide = (uint64_t)V * (uint64_t)d4 * 16u >= ((uint64_t)1 << 32);
 #define EMBED_LAUNCH(U, B, W)                                                                \
   do {                                                                                       \
     sif_embed_warp_kernel<NCH, EXPLICIT_W, U, B, W><<<grid, kEmbedWarps * 32, 0, st>>>(      \
-        (const float4*)tbl, (int)V, d4, stride4, wsrc, ids, N, L, (float4*)emb, status);     \
+        (const float4*)table, (int)V, d4, wsrc, ids, N, L, (float4*)emb, status);            \
     snprintf(kname, sizeof(kname), "sif_embed_warp_kernel<%d,%s,%d,%d,%s>", NCH,             \
              EXPLICIT_W ? "true" : "false", U, B, W ? "true" : "false");                     \
   } while (0)
@@ -682,24 +564,15 @@ static int launch_embed(const float* table, int64_t V, int d, const float* wsrc,
       else EMBED_LAUNCH(1, 2, false);
     } else if (wide) {
       EMBED_LAUNCH(2, 4, true);
+    } else if constexpr (!EXPLICIT_W) {
+      // fused lookup: ids of the next chunk prefetched; measured on B200, 4 M utterances: 11.83 ms
+      // without the prefetch -> 11.56 ms; also prefetching the next chunk's weight lookups (two chunks
+      // ahead) spills at the 64-register budget and takes 16.5 ms -- not kept
+      sif_embed_warp_prefetch_kernel<NCH, 2, 4><<<grid, kEmbedWarps * 32, 0, st>>>(
+          (const float4*)table, (int)V, d4, wsrc, ids, N, L, (float4*)emb, status);
+      snprintf(kname, sizeof(kname), "sif_embed_warp_prefetch_kernel<%d,2,4>", NCH);
     } else {
-      switch (variant) {
-        case 1: EMBED_LAUNCH(4, 3, false); break;
-        case 2: EMBED_LAUNCH(2, 5, false); break;
-        case 3: EMBED_LAUNCH(1, 6, false); break;
-        case 4: EMBED_LAUNCH(4, 2, false); break;
-        case 5: EMBED_LAUNCH(2, 3, false); break;
-        case 6:
-          if constexpr (!EXPLICIT_W && NCH <= 4) {
-            sif_embed_warp_prefetch_kernel<NCH, 2, 4><<<grid, kEmbedWarps * 32, 0, st>>>(
-                (const float4*)tbl, (int)V, d4, wsrc, ids, N, L, (float4*)emb, status);
-            snprintf(kname, sizeof(kname), "sif_embed_warp_prefetch_kernel<%d,2,4>", NCH);
-            break;
-          }
-          EMBED_LAUNCH(2, 4, false);
-          break;
-        default: EMBED_LAUNCH(2, 4, false); break;   // variant 0
-      }
+      EMBED_LAUNCH(2, 4, false);
     }
 #undef EMBED_LAUNCH
   }
@@ -826,24 +699,13 @@ extern "C" int mmb_ids_compact(const int64_t* ids, int64_t N, int64_t L, const i
   return MMB_OK;
 }
 
-namespace mmb {   // sif_embed_hot.cu
-size_t sif_embed_hot_extra_bytes(int64_t V);
-bool sif_embed_hot_eligible(int64_t V, int d, int64_t N, int64_t L);
-int sif_embed_hot(const float* tp, const int* flags, int64_t V, const int64_t* x, int64_t N, int64_t L, float* emb,
-                  int* status, void* ws_hot, cudaStream_t st);
-int sif_select_frequent_rows(const int64_t* x, int64_t N, int64_t L, int64_t V, int k, void* ws_hot, int** ids_out,
-                             cudaStream_t st);
-}  // namespace mmb
-
 extern "C" size_t mmb_sif_embed_workspace_bytes(int64_t V, int d, int64_t N, int64_t L) {
   // pre-scaled table + flag word; 0 = the batch is too small for the pre-scale pass to pay (or out of range)
-  const bool off = option_embed_prescale() == 0;
-  if (off || d <= 0 || d % 4 != 0 || d > 512 || V <= 0 || V >= ((int64_t)1 << kRowBits)) return 0;
+  if (d <= 0 || d % 4 != 0 || d > 512 || V <= 0 || V >= ((int64_t)1 << kRowBits)) return 0;
   if ((uint64_t)V * (uint64_t)d * 4u >= ((uint64_t)1 << 32)) return 0;
   if (L >= 256 && N < (int64_t)sm_count() * 16) return 0;     // few long rows: the CTA-per-utterance kernel
   if (N * L < 8 * V) return 0;
-  // (+ the sample histogram and hot-id list of the tensor-core hot-row path; unused below its threshold)
-  return (size_t)V * d * sizeof(float) + 256 + sif_embed_hot_extra_bytes(V);
+  return (size_t)V * d * sizeof(float) + 256;
 }
 
 namespace mmb {
@@ -858,64 +720,24 @@ int sif_prescale(const float* table, int64_t V, int d, const float* vocab_w, voi
 }
 
 // The embed pass on a pre-scaled table (ws from sif_prescale) with the general kernel standing by.
-// grid_mult: CTAs per SM of the grid-stride launch (4 are resident).  8 for a kernel that owns the GPU; the
-// Gram-overlap pipeline (api.cu) asks for more, smaller CTAs so that SMs freed by the Gram are refilled.
 int sif_embed_prescaled(const float* table, int64_t V, int d, const float* vocab_w, const void* ws, const int64_t* x,
-                        int64_t N, int64_t L, float* emb, int* status, cudaStream_t st, int grid_mult) {
+                        int64_t N, int64_t L, float* emb, int* status, cudaStream_t st) {
   if (N == 0) return MMB_OK;
   const int d4 = d / 4;
   const int* flags = (const int*)ws;
   const float4* tp4 = (const float4*)((const char*)ws + 256);
   const int sms = sm_count();
   const int64_t blocks = ceil_div(N, kEmbedWarps);
-  if (grid_mult < 1) grid_mult = 8;
-  const int grid = (int)(blocks < (int64_t)sms * grid_mult ? blocks : (int64_t)sms * grid_mult);
-  if (sif_embed_hot_eligible(V, d, N, L)) {
-    // very large batches: the most frequent rows on the tensor cores (sif_embed_hot.cu); the general kernel
-    // still stands by for the zero-weight case
-    void* ws_hot = (void*)((char*)ws + 256 + (size_t)V * d * sizeof(float));
-    int rc = sif_embed_hot((const float*)tp4, flags, V, x, N, L, emb, status, ws_hot, st);
-    if (rc) return rc;
-    sif_embed_warp_prefetch_kernel<3, 2, 4><<<grid, kEmbedWarps * 32, 0, st>>>(
-        (const float4*)table, (int)V, d4, vocab_w, x, N, L, (float4*)emb, status, flags);
-    MMB_LAUNCH_CHECK("sif_embed_general_standby");
-    return MMB_OK;
-  }
-  const int n_warm = option_embed_warm();
-  if (n_warm > 0 && d == 300 && V < ((int64_t)1 << kWarmRowBits) && N * L >= 64 * V) {
-    // L1 allocation policy per row: the K most frequent rows of a sample of the ids stay cacheable, the rest
-    // are read with L1::no_allocate
-    void* ws_hot = (void*)((char*)ws + 256 + (size_t)V * d * sizeof(float));
-    int* warm_ids = nullptr;
-    int rc = sif_select_frequent_rows(x, N, L, V, n_warm, ws_hot, &warm_ids, st);
-    if (rc) return rc;
-    sif_embed_prescaled_warm_kernel<3, 2, 4><<<grid, kEmbedWarps * 32, 0, st>>>(tp4, (int)V, d4, flags, warm_ids, n_warm,
-                                                                              x, N, L, (float4*)emb, status);
-    MMB_LAUNCH_CHECK("sif_embed_prescaled_warm");
-    sif_embed_warp_prefetch_kernel<3, 2, 4><<<grid, kEmbedWarps * 32, 0, st>>>(
-        (const float4*)table, (int)V, d4, vocab_w, x, N, L, (float4*)emb, status, flags);
-    MMB_LAUNCH_CHECK("sif_embed_general_standby");
-    note_kernel(0, "sif_embed_prescaled_warm_kernel<3,2,4>");
-    return MMB_OK;
-  }
-  static const int variant = getenv("MMB_EMBED_PS_VARIANT") ? atoi(getenv("MMB_EMBED_PS_VARIANT")) : 0;
-#define PS_KERNEL(NCH, U, B)                                                                                   \
-  sif_embed_prescaled_kernel<NCH, U, B><<<grid, kEmbedWarps * 32, 0, st>>>(tp4, (int)V, d4, flags, x, N, L,    \
-                                                                           (float4*)emb, status)
+  const int grid = (int)(blocks < (int64_t)sms * 8 ? blocks : (int64_t)sms * 8);
 #define PRESCALED_LAUNCH(NCH)                                                                                  \
   do {                                                                                                         \
-    if (variant == 1) PS_KERNEL(NCH, 3, 4);                                                                    \
-    else if (variant == 2) PS_KERNEL(NCH, 3, 3);                                                               \
-    else if (variant == 3) PS_KERNEL(NCH, 4, 3);                                                               \
-    else PS_KERNEL(NCH, 2, 4);                                                                                 \
+    sif_embed_prescaled_kernel<NCH, 2, 4><<<grid, kEmbedWarps * 32, 0, st>>>(tp4, (int)V, d4, flags, x, N, L,  \
+                                                                             (float4*)emb, status);            \
     MMB_LAUNCH_CHECK("sif_embed_prescaled");                                                                   \
     sif_embed_warp_prefetch_kernel<NCH, 2, 4><<<grid, kEmbedWarps * 32, 0, st>>>(                              \
         (const float4*)table, (int)V, d4, vocab_w, x, N, L, (float4*)emb, status, flags);                      \
     MMB_LAUNCH_CHECK("sif_embed_general_standby");                                                             \
-    note_kernel(0, variant == 1 ? "sif_embed_prescaled_kernel<" #NCH ",3,4>"                                  \
-                   : variant == 2 ? "sif_embed_prescaled_kernel<" #NCH ",3,3>"                                \
-                   : variant == 3 ? "sif_embed_prescaled_kernel<" #NCH ",4,3>"                                \
-                                  : "sif_embed_prescaled_kernel<" #NCH ",2,4>");                              \
+    note_kernel(0, "sif_embed_prescaled_kernel<" #NCH ",2,4>");                                               \
   } while (0)
   switch ((d4 + 31) / 32) {
     case 1: PRESCALED_LAUNCH(1); break;
@@ -924,7 +746,6 @@ int sif_embed_prescaled(const float* table, int64_t V, int d, const float* vocab
     default: PRESCALED_LAUNCH(4); break;
   }
 #undef PRESCALED_LAUNCH
-#undef PS_KERNEL
   return MMB_OK;
 }
 }  // namespace mmb
@@ -940,5 +761,5 @@ extern "C" int mmb_sif_embed_ws(const float* table, int64_t V, int d, const floa
               "table / emb / ws must be 16-byte aligned");
   int rc = sif_prescale(table, V, d, vocab_w, ws, as_stream(stream));
   if (rc) return rc;
-  return sif_embed_prescaled(table, V, d, vocab_w, ws, x, N, L, emb, status, as_stream(stream), 8);
+  return sif_embed_prescaled(table, V, d, vocab_w, ws, x, N, L, emb, status, as_stream(stream));
 }

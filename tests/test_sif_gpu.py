@@ -508,55 +508,6 @@ def test_device_masks_equal_reference_masks(mods, capsys):
     capsys.readouterr()
 
 
-@pytest.mark.gpu
-def test_embed_gram_beside_each_other_equals_the_two_stages(mods):
-    """mmb_sif_embed_gram: embed + Gram of a block in one call.  With overlap_sms = 0 (default) it IS
-    mmb_sif_embed_ws + mmb_gram; with the Gram of chunk c running on a few SMs beside the embed of chunk c + 1
-    (experiment, DESIGN.md section 4) the embeddings are bit-identical and the Gram -- chunk Grams added in
-    chunk order -- equals the float64 Gram of those embeddings within the tensor-core path's bound."""
-    import torch
-    nv, sf, sif = mods
-    lib = nv.lib
-    dev = torch.device('cuda')
-    rng = np.random.default_rng(21)
-    V, d, n, L = 20000, 300, 131072 + 37, 16                # N * L >= 8 V; 4 chunks of >= 32768 rows
-    We = cases.table(V, d, seed=5)
-    ids, p = cases.zipf_ids(rng, n, L, V)
-    weights = cases.sif_weights(p).astype(np.float32)
-    t_We, t_ids, t_w = torch.tensor(We, device=dev), torch.tensor(ids, device=dev), torch.tensor(weights, device=dev)
-    nbytes = lib.mmb_sif_embed_gram_workspace_bytes(V, d, n, L, 0)
-    ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-
-    def run(sms):
-        nv.check(lib.mmb_set_option(b'overlap_sms', sms))
-        nv.check(lib.mmb_set_option(b'overlap_chunks', 4))
-        emb = torch.zeros((n, d), dtype=torch.float32, device=dev)
-        G = torch.zeros((d, d), dtype=torch.float32, device=dev)
-        st = torch.zeros(1, dtype=torch.int32, device=dev)
-        nv.check(lib.mmb_sif_embed_gram(nv.ptr(t_We), V, d, nv.ptr(t_w), nv.ptr(t_ids), n, L, nv.ptr(emb), nv.ptr(st),
-                                        nv.ptr(G), nv.ptr(ws), nbytes, 0, nv.stream_ptr()))
-        torch.cuda.synchronize()
-        assert int(st.item()) == 0
-        return emb, G
-
-    try:
-        emb0, G0 = run(0)
-        emb1, G1 = run(40)
-        emb2, G2 = run(40)
-    finally:
-        nv.check(lib.mmb_set_option(b'overlap_sms', 0))
-        nv.check(lib.mmb_set_option(b'overlap_chunks', 10))
-    assert torch.equal(emb0, emb1) and torch.equal(G1, G2)   # same embeddings; deterministic
-    want = (emb0.double().T @ emb0.double()).cpu().numpy()
-    scale = np.abs(want).max()
-    assert np.abs(G0.double().cpu().numpy() - want).max() / scale < 2e-5
-    assert np.abs(G1.double().cpu().numpy() - want).max() / scale < 2e-5
-    rows = np.arange(0, n, 997)
-    w = so.seq2weight(ids[rows], np.ones(ids[rows].shape), weights.astype(np.float64))
-    assert rel_err(emb1[torch.as_tensor(rows, device=dev)].double().cpu().numpy(),
-                   so.get_weighted_average(We, ids[rows], w)) < EMB_RTOL
-
-
 def test_prescaled_table_path_equals_general_kernel(mods):
     """Large batches fold the vocabulary weights into a scratch copy of the table (mmb_sif_embed_ws): same
     averages as the general kernel and the oracle (one extra rounding per term); a zero vocabulary weight
@@ -610,51 +561,6 @@ def test_prescaled_table_path_equals_general_kernel(mods):
     assert stb & nv.STATUS_BAD_INDEX
     # too small a batch: no scratch requested, plain kernel
     assert lib.mmb_sif_embed_workspace_bytes(V, d, 10, L) == 0
-
-
-def test_embed_experimental_paths_are_correct(mods):
-    """The two round-2 experiments on the embed kernel stay selectable (mmb_set_option) and correct: the
-    tensor-core hot-row path (tcgen05 kind::tf32 over the 64 most frequent rows) and the per-row L1 allocation
-    policy.  Neither is the default (both measured slower, DESIGN.md section 4)."""
-    import torch
-    nv, sf, sif = mods
-    lib = nv.lib
-    dev = torch.device('cuda')
-    rng = np.random.default_rng(21)
-    V, d, n, L = 2000, 300, 4500, 64
-    We = cases.table(V, d, seed=5)
-    ids, p = cases.zipf_ids(rng, n, L, V)
-    ids[9, 4] = -3
-    weights = cases.sif_weights(p).astype(np.float32)
-    t_We, t_w, t_ids = torch.tensor(We, device=dev), torch.tensor(weights, device=dev), torch.tensor(ids, device=dev)
-
-    def run():
-        emb = torch.empty((n, d), dtype=torch.float32, device=dev)
-        st = torch.zeros(1, dtype=torch.int32, device=dev)
-        nbytes = lib.mmb_sif_embed_workspace_bytes(V, d, n, L)
-        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        nv.check(lib.mmb_sif_embed_ws(nv.ptr(t_We), V, d, nv.ptr(t_w), nv.ptr(t_ids), n, L, nv.ptr(emb), nv.ptr(st),
-                                      nv.ptr(ws), nbytes, nv.stream_ptr()))
-        assert int(st.item()) == 0
-        return emb, (lib.mmb_last_kernel(0) or b'').decode()
-    try:
-        ref, k0 = run()
-        assert 'prescaled_kernel' in k0
-        nv.check(lib.mmb_set_option(b'embed_warm', 128))
-        warm, k1 = run()
-        assert 'warm' in k1 and torch.equal(warm, ref)               # only the cache policy differs
-        nv.check(lib.mmb_set_option(b'embed_warm', 0))
-        nv.check(lib.mmb_set_option(b'embed_hot', 1))
-        hot, k2 = run()
-        assert 'hot' in k2
-        assert rel_err(hot.double().cpu().numpy(), ref.double().cpu().numpy()) < 5e-6
-        w = so.seq2weight(ids, np.ones(ids.shape), weights.astype(np.float64))
-        assert rel_err(hot.double().cpu().numpy(), so.get_weighted_average(We, ids, w)) < EMB_RTOL
-        with pytest.raises(ValueError):
-            nv.check(lib.mmb_set_option(b'no_such_option', 1))
-    finally:
-        lib.mmb_set_option(b'embed_warm', 0)
-        lib.mmb_set_option(b'embed_hot', 0)
 
 
 def test_ragged_equals_padded_at_bench_shape(mods):

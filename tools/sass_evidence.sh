@@ -3,7 +3,7 @@
 # Blackwell-native kernel"): counts per object file of libmmb_b200.so.  Runs on the CPU box (no GPU needed).
 cd "$(dirname "$0")/../multimodal-baselines_b200" || exit 1
 python build.py > /dev/null
-for f in gram_tc sif_embed sif_embed_hot remove_pc peer_comm pc_solve mmb_step; do
+for f in gram_tc sif_embed remove_pc peer_comm pc_solve mmb_step; do
   echo "== csrc/$f.cu"
   cuobjdump -sass build/$f.o 2>/dev/null | grep -oE "\b(UTC[A-Z]*MMA[.A-Z0-9_]*|UTMALDG[.A-Z0-9_]*|UTMAPF[.A-Z0-9_]*|UTCBAR[.A-Z0-9_]*|UTCATOMSWS[.A-Z0-9_]*|LDTM[.A-Z0-9_x]*|STTM[.A-Z0-9_x]*|SYNCS[.A-Z0-9_]*|FFMA2|MATCH\.ANY|LDG\.E\.NA\.128[.A-Z]*|LDG\.E\.128[.A-Z]*|DFMA|ACQBULK|HMMA[.A-Z0-9_]*|ATOMG[.A-Z0-9_]*|LD\.E\.[A-Z0-9.]*SYS[.A-Z0-9]*|ST\.E\.[A-Z0-9.]*SYS[.A-Z0-9]*)" | sort | uniq -c | sort -rn
 done

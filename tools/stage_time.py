@@ -1,7 +1,8 @@
-"""Per-stage device times of the SIF path on a slice of the bench workload, plus correctness of
-the Gram and the component solve against float64 torch.  Variants are selected by the same
-environment switches the library reads (MMB_EMBED_PAD, MMB_PC_SOLVER, MMB_TC_SEG ...), so run
-it once per variant:   PROFILE_N=4000000 MMB_EMBED_PAD=1 python tools/stage_time.py"""
+"""Per-stage device times of the SIF path (embed, tcgen05 Gram, component solve, projection) on a
+slice of the bench workload, plus correctness of the Gram and the component solve against float64
+torch.  PROFILE_N sets the number of utterances (default 4 M); IDS=uniform draws the ids uniformly
+instead of from the bench's Zipf law.  Every output line is tagged with IDS and any MMB_* variable
+set, such as MMB_PC_SOLVER:   PROFILE_N=4000000 python tools/stage_time.py"""
 import os
 import sys
 
