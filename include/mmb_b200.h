@@ -120,6 +120,17 @@ MMB_API size_t mmb_sif_embed_multi_workspace_bytes(int64_t V, int K);
 MMB_API int mmb_sif_embed_multi(const float* table, int64_t V, int d, const float* vocab_w, int K, const int64_t* x,
                                 int64_t N, int64_t L, float* emb, int* status, void* ws, size_t ws_bytes,
                                 mmb_stream_t stream);
+/* mmb_sif_embed_multi on ragged (CSR) ids (tokens, offsets, L_pad, pad_id as for mmb_sif_embed_ragged below): emb
+ * is (K, N, d) and emb[k] is bit-identical to mmb_sif_embed_ragged with vocab_w = vocab_w[k].  The pad run of each
+ * utterance is added in closed form per k (n_pad * vocab_w[k][pad_id] * table[pad_id] to the sum, n_pad to the
+ * divisor when that weight is non-zero), so padding is neither stored nor walked.  d <= 512.  The same workspace
+ * (mmb_sif_embed_multi_workspace_bytes(V, K)) and variant rule (L_pad >= 256 and N < 16 SMs: a CTA per utterance)
+ * as mmb_sif_embed_multi.  MMB_STATUS_BAD_INDEX: a token outside [-V, V), an utterance longer than L_pad, or a
+ * pad_id outside [-V, V) where padding is present.  mmb_last_kernel(1) names a *_ragged_* kernel.          */
+MMB_API int mmb_sif_embed_multi_ragged(const float* table, int64_t V, int d, const float* vocab_w, int K,
+                                       const int64_t* tokens, const int64_t* offsets, int64_t N, int64_t L_pad,
+                                       int64_t pad_id, float* emb, int* status, void* ws, size_t ws_bytes,
+                                       mmb_stream_t stream);
 
 /* Ragged (CSR) ids, SURVEY.md 8f N3 -- the same result as mmb_sif_embed on the right-padded (N, L_pad)
  * matrix the reference builds (utils.py:77-80; sif_functions.py:28-56), without walking the padding:

@@ -44,6 +44,7 @@ SIGNATURES = {
     'mmb_sif_embed_ws': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _p, _p, _p, _sz, _p]),
     'mmb_sif_embed_multi_workspace_bytes': (_sz, [_i64, _i]),
     'mmb_sif_embed_multi': (_i, [_p, _i64, _i, _p, _i, _p, _i64, _i64, _p, _p, _p, _sz, _p]),
+    'mmb_sif_embed_multi_ragged': (_i, [_p, _i64, _i, _p, _i, _p, _p, _i64, _i64, _i64, _p, _p, _p, _sz, _p]),
     'mmb_sif_embed_ragged': (_i, [_p, _i64, _i, _p, _p, _p, _i64, _i64, _i64, _p, _p, _p]),
     'mmb_ids_lengths': (_i, [_p, _i64, _i64, _i64, _p, _p, _p]),
     'mmb_ids_compact': (_i, [_p, _i64, _i64, _p, _p, _p]),

@@ -15,6 +15,8 @@
 //   * the divisor is counted per k (count_nonzero of that vector's token weights), stored with __fdiv_rn: a
 //     vector with zero entries gets its own count, an all-zero row its own inf/NaN.
 // Negative ids wrap like NumPy and get weight 0 for every k; ids outside [-V, V) raise MMB_STATUS_BAD_INDEX.
+// mmb_sif_embed_multi_ragged does the same on ragged (CSR) ids: emb[k] is mmb_sif_embed_ragged(vocab_w = W[k]) bit
+// for bit (chunks of the CSR run, then the pad run in closed form; the same variant rule).
 #include "sif_rows.cuh"
 
 namespace mmb {
@@ -172,9 +174,49 @@ __global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
   if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, MMB_STATUS_BAD_INDEX);
 }
 
-// CTA per utterance (few, long utterances): the 8 warps take 32-token chunks round-robin; per output k the warp
-// partials go through shared memory and are summed in warp order (sif_embed_cta_kernel, one k at a time so the
-// shared footprint is the single-vector kernel's).
+// The CTA-per-utterance epilogue: per output k the warp partials go through shared memory and are summed in warp
+// order, then divided by the utterance's count (sif_embed_cta_kernel, one k at a time so the shared footprint is the
+// single-vector kernel's).  Output k of utterance i is row (k * N + i) of emb4.
+template <int NCH, int KG>
+__device__ __forceinline__ void cta_store_multi(float4 (&part)[kEmbedWarps][NCH * 32], int (&part_cnt)[kEmbedWarps],
+                                                const RowAcc<NCH> (&acc)[KG], const int (&cnt)[KG], int kn,
+                                                typename Live<NCH>::type tail, int lane, int warp, int d4,
+                                                float4* __restrict__ emb4, int64_t N, int64_t i) {
+#pragma unroll
+  for (int k = 0; k < KG; ++k) {
+    if (k >= kn) break;
+#pragma unroll
+    for (int c = 0; c < NCH; ++c) {
+      float4 r = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (chunk_on<NCH>(tail, c)) {
+        unpack2(acc[k].a[c][0], r.x, r.y);
+        unpack2(acc[k].a[c][1], r.z, r.w);
+      }
+      part[warp][lane + 32 * c] = r;
+    }
+    if (lane == 0) part_cnt[warp] = cnt[k];
+    __syncthreads();
+    int total = 0;
+#pragma unroll
+    for (int w = 0; w < kEmbedWarps; ++w) total += part_cnt[w];
+    const float div = (float)total;
+    float4* out = emb4 + ((size_t)k * N + i) * d4;
+    for (int e = threadIdx.x; e < d4; e += blockDim.x) {
+      float4 s = part[0][e];
+#pragma unroll
+      for (int w = 1; w < kEmbedWarps; ++w) {
+        float4 p = part[w][e];
+        s.x += p.x; s.y += p.y; s.z += p.z; s.w += p.w;
+      }
+      s.x = __fdiv_rn(s.x, div); s.y = __fdiv_rn(s.y, div);
+      s.z = __fdiv_rn(s.z, div); s.w = __fdiv_rn(s.w, div);
+      st_stream(out + e, s);
+    }
+    __syncthreads();
+  }
+}
+
+// CTA per utterance (few, long utterances): the 8 warps take 32-token chunks round-robin, then cta_store_multi.
 template <int NCH, int KG, int UNROLL>
 __global__ void __launch_bounds__(kEmbedWarps * 32, 1)
     sif_embed_multi_cta_kernel(const float4* __restrict__ table4, int V, int d4, const float* __restrict__ wg,
@@ -197,47 +239,113 @@ __global__ void __launch_bounds__(kEmbedWarps * 32, 1)
     for (int64_t base = 32 * (int64_t)warp; base < L; base += 32 * kEmbedWarps)
       accumulate_chunk_multi<NCH, KG, UNROLL, true, false>(acc, cnt, lane_base, V, row_bytes, tail, wg, row_ids, base,
                                                            L, lane, bad, 0);
-#pragma unroll
-    for (int k = 0; k < KG; ++k) {
-      if (k >= kn) break;
-#pragma unroll
-      for (int c = 0; c < NCH; ++c) {
-        float4 r = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (chunk_on<NCH>(tail, c)) {
-          unpack2(acc[k].a[c][0], r.x, r.y);
-          unpack2(acc[k].a[c][1], r.z, r.w);
-        }
-        part[warp][lane + 32 * c] = r;
-      }
-      if (lane == 0) part_cnt[warp] = cnt[k];
-      __syncthreads();
-      int total = 0;
-#pragma unroll
-      for (int w = 0; w < kEmbedWarps; ++w) total += part_cnt[w];
-      const float div = (float)total;
-      float4* out = emb4 + ((size_t)k * N + i) * d4;
-      for (int e = threadIdx.x; e < d4; e += blockDim.x) {
-        float4 s = part[0][e];
-#pragma unroll
-        for (int w = 1; w < kEmbedWarps; ++w) {
-          float4 p = part[w][e];
-          s.x += p.x; s.y += p.y; s.z += p.z; s.w += p.w;
-        }
-        s.x = __fdiv_rn(s.x, div); s.y = __fdiv_rn(s.y, div);
-        s.z = __fdiv_rn(s.z, div); s.w = __fdiv_rn(s.w, div);
-        st_stream(out + e, s);
-      }
-      __syncthreads();
-    }
+    cta_store_multi<NCH, KG>(part, part_cnt, acc, cnt, kn, tail, lane, warp, d4, emb4, N, i);
   }
   if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, MMB_STATUS_BAD_INDEX);
 }
 
-// One gather pass: kn (<= KG) vectors whose weights are the (V, KG) block wg, outputs from emb.
+// ---- ragged (CSR) ids -----------------------------------------------------------------------------------------
+// Utterance i is tokens[offsets[i] .. offsets[i+1]) followed by n_pad = L_pad - length copies of pad_id, added in
+// closed form after the chunks as mmb_sif_embed_ragged does: n_pad * w_k[pad] * table[pad] to sum k, n_pad to
+// count k when w_k[pad] != 0.  The FMA runs even when w_k[pad] == 0 (it can still turn -0 into +0, or an inf/NaN
+// pad row into NaN), so emb[k] is mmb_sif_embed_ragged(vocab_w = W[k]) bit for bit.  pad_row is pad_id wrapped
+// like a negative token; a negative pad_id weighs 0.  Returns false (a bad index) when the utterance is longer than
+// L_pad, or pads with a row outside [0, V).
 template <int NCH, int KG>
-static int launch_multi_group(const float* table, int64_t V, int d, const float* wg, const int64_t* ids, int64_t N,
-                              int64_t L, int kn, float* emb, int* status, bool few_long, bool wide, int grid,
-                              cudaStream_t st, char* kname, size_t kname_len) {
+__device__ __forceinline__ bool add_pad_run_multi(RowAcc<NCH> (&acc)[KG], int (&cnt)[KG],
+                                                  const char* __restrict__ lane_base, unsigned row_bytes,
+                                                  typename Live<NCH>::type tail, const float* __restrict__ wg,
+                                                  int V, int64_t pad_id, int64_t n_pad) {
+  if (n_pad == 0) return true;
+  const int64_t pad_row = pad_id < 0 ? pad_id + V : pad_id;
+  if (n_pad < 0 || pad_row < 0 || pad_row >= V) return false;
+  float w[KG];
+#pragma unroll
+  for (int k = 0; k < KG; ++k) w[k] = 0.f;
+  if (pad_id >= 0) load_wk<KG>(w, wg + (size_t)pad_id * KG);
+  float4 v[NCH] = {};    // defined where the row has no chunk: otherwise ptxas carries it across utterances (spills)
+  load_row<NCH>(v, lane_base, (size_t)pad_row * row_bytes, tail);
+#pragma unroll
+  for (int k = 0; k < KG; ++k) {
+    fma_row<NCH>(acc[k], v, (float)n_pad * w[k], tail);
+    if (w[k] != 0.f) cnt[k] += (int)n_pad;
+  }
+  return true;
+}
+
+// Warp per utterance on ragged ids (sif_embed_ragged_kernel for KG vectors): the chunks of the CSR run with 64-bit
+// row offsets, then the pad run.
+template <int NCH, int KG, int UNROLL, int MINB>
+__global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
+    sif_embed_multi_ragged_warp_kernel(const float4* __restrict__ table4, int V, int d4, const float* __restrict__ wg,
+                                       const int64_t* __restrict__ tokens, const int64_t* __restrict__ offsets,
+                                       int64_t N, int64_t L_pad, int64_t pad_id, int kn, float4* __restrict__ emb4,
+                                       int* __restrict__ status) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp0 = (int64_t)blockIdx.x * kEmbedWarps + (threadIdx.x >> 5);
+  const int64_t nwarps = (int64_t)gridDim.x * kEmbedWarps;
+  const char* lane_base = (const char*)(table4 + lane);
+  const unsigned row_bytes = (unsigned)d4 * 16u;
+  const typename Live<NCH>::type tail = make_live<NCH>(lane, d4);
+  bool bad = false;
+  for (int64_t i = warp0; i < N; i += nwarps) {
+    RowAcc<NCH> acc[KG];
+    int cnt[KG];
+#pragma unroll
+    for (int k = 0; k < KG; ++k) { acc[k].clear(); cnt[k] = 0; }
+    const int64_t o0 = __ldg(offsets + i), len = __ldg(offsets + i + 1) - o0;
+    const int64_t* row_ids = tokens + o0;
+    // the chunks by pointer and remaining length: one 64-bit induction variable fewer than base / len
+    for (int64_t rem = len; rem > 0; rem -= 32, row_ids += 32)
+      accumulate_chunk_multi<NCH, KG, UNROLL, true, false>(acc, cnt, lane_base, V, row_bytes, tail, wg, row_ids, 0,
+                                                           rem, lane, bad, 0);
+    if (!add_pad_run_multi<NCH, KG>(acc, cnt, lane_base, row_bytes, tail, wg, V, pad_id, L_pad - len)) bad = true;
+#pragma unroll
+    for (int k = 0; k < KG; ++k)
+      if (k < kn) store_row<NCH>(emb4 + ((size_t)k * N + i) * d4, acc[k], cnt[k], lane, d4);
+  }
+  if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, MMB_STATUS_BAD_INDEX);
+}
+
+// CTA per utterance on ragged ids (sif_embed_cta_kernel with offsets, for KG vectors): warp 0 adds the pad run after
+// its own chunks, then the warp partials are summed in warp order.
+template <int NCH, int KG, int UNROLL>
+__global__ void __launch_bounds__(kEmbedWarps * 32, 1)
+    sif_embed_multi_ragged_cta_kernel(const float4* __restrict__ table4, int V, int d4, const float* __restrict__ wg,
+                                      const int64_t* __restrict__ tokens, const int64_t* __restrict__ offsets,
+                                      int64_t N, int64_t L_pad, int64_t pad_id, int kn, float4* __restrict__ emb4,
+                                      int* __restrict__ status) {
+  __shared__ float4 part[kEmbedWarps][NCH * 32];
+  __shared__ int part_cnt[kEmbedWarps];
+  const int lane = threadIdx.x & 31;
+  const int warp = threadIdx.x >> 5;
+  const char* lane_base = (const char*)(table4 + lane);
+  const unsigned row_bytes = (unsigned)d4 * 16u;
+  const typename Live<NCH>::type tail = make_live<NCH>(lane, d4);
+  bool bad = false;
+  for (int64_t i = blockIdx.x; i < N; i += gridDim.x) {
+    RowAcc<NCH> acc[KG];
+    int cnt[KG];
+#pragma unroll
+    for (int k = 0; k < KG; ++k) { acc[k].clear(); cnt[k] = 0; }
+    const int64_t o0 = __ldg(offsets + i), len = __ldg(offsets + i + 1) - o0;
+    for (int64_t base = 32 * (int64_t)warp; base < len; base += 32 * kEmbedWarps)
+      accumulate_chunk_multi<NCH, KG, UNROLL, true, false>(acc, cnt, lane_base, V, row_bytes, tail, wg, tokens + o0,
+                                                           base, len, lane, bad, 0);
+    if (warp == 0 && !add_pad_run_multi<NCH, KG>(acc, cnt, lane_base, row_bytes, tail, wg, V, pad_id, L_pad - len))
+      bad = true;
+    cta_store_multi<NCH, KG>(part, part_cnt, acc, cnt, kn, tail, lane, warp, d4, emb4, N, i);
+  }
+  if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, MMB_STATUS_BAD_INDEX);
+}
+
+// One gather pass: kn (<= KG) vectors whose weights are the (V, KG) block wg, outputs from emb.  With offsets (ragged
+// ids, d <= 512) ids are the CSR tokens and L is L_pad.
+template <int NCH, int KG>
+static int launch_multi_group(const float* table, int64_t V, int d, const float* wg, const int64_t* ids,
+                              const int64_t* offsets, int64_t N, int64_t L, int64_t pad_id, int kn, float* emb,
+                              int* status, bool few_long, bool wide, int grid, cudaStream_t st, char* kname,
+                              size_t kname_len) {
   const int d4 = d / 4;
   // 64 accumulator registers (KG * NCH = 16): one row in flight instead of two (spills otherwise); d > 512 also
   // takes the whole register file (one CTA per SM), as the single-vector kernel's one-row configuration spills.
@@ -245,6 +353,24 @@ static int launch_multi_group(const float* table, int64_t V, int d, const float*
   // (B200, 10 M x 64 tokens, d = 300, K = 2: 53.9 ms at 2 CTAs per SM)
   constexpr int UNROLL = (NCH > 4 || KG * NCH >= 16) ? 1 : 2;
   constexpr int MINB = NCH > 4 ? 1 : (KG * NCH <= 2 ? 4 : (KG * NCH <= 6 ? 3 : 2));
+  if constexpr (NCH <= 4) {
+    if (offsets) {
+      if (few_long) {
+        sif_embed_multi_ragged_cta_kernel<NCH, KG, UNROLL><<<grid, kEmbedWarps * 32, 0, st>>>(
+            (const float4*)table, (int)V, d4, wg, ids, offsets, N, L, pad_id, kn, (float4*)emb, status);
+        snprintf(kname, kname_len, "sif_embed_multi_ragged_cta_kernel<%d,%d,%d>", NCH, KG, UNROLL);
+      } else {
+        // the CSR walk and the pad run need a few more registers than the padded kernel: at NCH = 4, KG = 1 they
+        // do not fit 80 (3 CTAs per SM) without a spill
+        constexpr int RMINB = (NCH == 4 && MINB == 3) ? 2 : MINB;
+        sif_embed_multi_ragged_warp_kernel<NCH, KG, UNROLL, RMINB><<<grid, kEmbedWarps * 32, 0, st>>>(
+            (const float4*)table, (int)V, d4, wg, ids, offsets, N, L, pad_id, kn, (float4*)emb, status);
+        snprintf(kname, kname_len, "sif_embed_multi_ragged_warp_kernel<%d,%d,%d,%d>", NCH, KG, UNROLL, RMINB);
+      }
+      MMB_LAUNCH_CHECK("sif_embed_multi_ragged");
+      return MMB_OK;
+    }
+  }
   if (few_long) {
     sif_embed_multi_cta_kernel<NCH, KG, UNROLL><<<grid, kEmbedWarps * 32, 0, st>>>(
         (const float4*)table, (int)V, d4, wg, ids, N, L, kn, (float4*)emb, status);
@@ -264,7 +390,8 @@ static int launch_multi_group(const float* table, int64_t V, int d, const float*
 
 template <int NCH>
 static int launch_multi(const float* table, int64_t V, int d, const float* vocab_w, int K, const int64_t* ids,
-                        int64_t N, int64_t L, float* emb, int* status, float* ws, cudaStream_t st) {
+                        const int64_t* offsets, int64_t N, int64_t L, int64_t pad_id, float* emb, int* status,
+                        float* ws, cudaStream_t st) {
   constexpr int KG = multi_group(NCH);
   const int sms = sm_count();
   const int ngroups = (K + KG - 1) / KG;
@@ -277,7 +404,7 @@ static int launch_multi(const float* table, int64_t V, int d, const float* vocab
   multi_weights_kernel<<<pgrid, 256, 0, st>>>(vocab_w, V, K, KG, ngroups, last_w, total, ws);
   MMB_LAUNCH_CHECK("sif_multi_weights");
 
-  // launch_embed's variant rule and grid (sif_embed.cu)
+  // launch_embed's (and mmb_sif_embed_ragged's) variant rule and grid (sif_embed.cu)
   const bool few_long = (L >= 256) && (N < (int64_t)sms * 16);
   const bool wide = (uint64_t)V * (uint64_t)(d / 4) * 16u >= ((uint64_t)1 << 32);
   const int64_t cap = (int64_t)sms * 8;
@@ -291,8 +418,8 @@ static int launch_multi(const float* table, int64_t V, int d, const float* vocab
     float* out = emb + (size_t)g * KG * N * d;
     int rc = MMB_OK;
 #define MULTI_GROUP(W) \
-  rc = launch_multi_group<NCH, W>(table, V, d, wg, ids, N, L, kn, out, status, few_long, wide, grid, st, kname, \
-                                  sizeof(kname))
+  rc = launch_multi_group<NCH, W>(table, V, d, wg, ids, offsets, N, L, pad_id, kn, out, status, few_long, wide, \
+                                  grid, st, kname, sizeof(kname))
     if (kw == 1) MULTI_GROUP(1);
     else if (kw == 2) MULTI_GROUP(2);
     else if constexpr (KG >= 4) {
@@ -331,10 +458,33 @@ extern "C" int mmb_sif_embed_multi(const float* table, int64_t V, int d, const f
   cudaStream_t st = as_stream(stream);
   float* wsf = (float*)ws;
   switch ((d / 4 + 31) / 32) {
-    case 1: return launch_multi<1>(table, V, d, vocab_w, K, x, N, L, emb, status, wsf, st);
-    case 2: return launch_multi<2>(table, V, d, vocab_w, K, x, N, L, emb, status, wsf, st);
-    case 3: return launch_multi<3>(table, V, d, vocab_w, K, x, N, L, emb, status, wsf, st);
-    case 4: return launch_multi<4>(table, V, d, vocab_w, K, x, N, L, emb, status, wsf, st);
-    default: return launch_multi<8>(table, V, d, vocab_w, K, x, N, L, emb, status, wsf, st);
+    case 1: return launch_multi<1>(table, V, d, vocab_w, K, x, nullptr, N, L, 0, emb, status, wsf, st);
+    case 2: return launch_multi<2>(table, V, d, vocab_w, K, x, nullptr, N, L, 0, emb, status, wsf, st);
+    case 3: return launch_multi<3>(table, V, d, vocab_w, K, x, nullptr, N, L, 0, emb, status, wsf, st);
+    case 4: return launch_multi<4>(table, V, d, vocab_w, K, x, nullptr, N, L, 0, emb, status, wsf, st);
+    default: return launch_multi<8>(table, V, d, vocab_w, K, x, nullptr, N, L, 0, emb, status, wsf, st);
+  }
+}
+
+extern "C" int mmb_sif_embed_multi_ragged(const float* table, int64_t V, int d, const float* vocab_w, int K,
+                                          const int64_t* tokens, const int64_t* offsets, int64_t N, int64_t L_pad,
+                                          int64_t pad_id, float* emb, int* status, void* ws, size_t ws_bytes,
+                                          mmb_stream_t stream) {
+  MMB_REQUIRE(d > 0 && d % 4 == 0 && d <= 512, "d must be a multiple of 4, <= 512");
+  MMB_REQUIRE(V > 0 && V < (int64_t)1 << 31, "V out of range");
+  MMB_REQUIRE(K >= 1, "K must be >= 1");
+  MMB_REQUIRE(N >= 0 && L_pad >= 0, "negative size");
+  if (N == 0) return MMB_OK;   // empty input: nothing to do (pointers may be null)
+  MMB_REQUIRE(table && vocab_w && offsets && emb && status && ws, "null pointer");
+  MMB_REQUIRE(ws_bytes >= mmb_sif_embed_multi_workspace_bytes(V, K), "workspace too small");
+  MMB_REQUIRE(((uintptr_t)table % 16 == 0) && ((uintptr_t)emb % 16 == 0) && ((uintptr_t)ws % 32 == 0),
+              "table / emb must be 16-byte aligned, ws 32-byte aligned");
+  cudaStream_t st = as_stream(stream);
+  float* wsf = (float*)ws;
+  switch ((d / 4 + 31) / 32) {
+    case 1: return launch_multi<1>(table, V, d, vocab_w, K, tokens, offsets, N, L_pad, pad_id, emb, status, wsf, st);
+    case 2: return launch_multi<2>(table, V, d, vocab_w, K, tokens, offsets, N, L_pad, pad_id, emb, status, wsf, st);
+    case 3: return launch_multi<3>(table, V, d, vocab_w, K, tokens, offsets, N, L_pad, pad_id, emb, status, wsf, st);
+    default: return launch_multi<4>(table, V, d, vocab_w, K, tokens, offsets, N, L_pad, pad_id, emb, status, wsf, st);
   }
 }

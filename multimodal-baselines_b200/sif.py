@@ -2,7 +2,8 @@
 ``get_sentence_embeddings``, the call ``simplesif.main`` makes per split (reference
 simplesif.py:296-311).  The embedding itself runs through ``mmb_sif_embedding_host`` /
 ``mmb_sif_embedding`` of libmmb_b200.so.  ``get_sentence_embeddings_sweep`` (no reference counterpart) does the
-same for K word-weight vectors and several numbers of removed components in one gather (``mmb_sif_embed_multi``).
+same for K word-weight vectors and several numbers of removed components in one gather (``mmb_sif_embed_multi``;
+``mmb_sif_embed_multi_ragged`` for ``RaggedIds``).
 """
 import ctypes as C
 import os
@@ -142,10 +143,12 @@ def get_sentence_embeddings_sweep(word_embeddings, weights, text, npcs=(1,)):
 
     ``weights`` is a (K, V) array or a sequence of K vectors; a vector shorter than the table is padded with
     zeros, and an id beyond it raises ``IndexError``, as in ``get_sentence_embeddings``.  NumPy in -> float64
-    (K, P, N, d) NumPy out; CUDA tensors in -> float32 CUDA tensor out.  The ids are uploaded once and the
-    result downloaded once."""
+    (K, P, N, d) NumPy out; CUDA tensors or ``RaggedIds`` in -> float32 CUDA tensor out.  The ids are uploaded
+    once and the result downloaded once.  For ``RaggedIds`` the ids are those of the padded matrix they stand
+    for: the tokens, and ``pad_id`` when an utterance is shorter than ``L_pad``."""
     dev = nv.require_cuda()
-    as_np = not (isinstance(text, torch.Tensor) and text.is_cuda)
+    ragged = isinstance(text, RaggedIds)
+    as_np = not (ragged or (isinstance(text, torch.Tensor) and text.is_cuda))
     table_t = nv.to_device(word_embeddings, torch.float32, dev)
     V, d = table_t.shape
     if isinstance(weights, torch.Tensor):
@@ -160,6 +163,12 @@ def get_sentence_embeddings_sweep(word_embeddings, weights, text, npcs=(1,)):
             raise ValueError('text must be (n_samples, seq_len)')
         ids_t = nv.to_device(ids, torch.int64, dev)
         id_max = int(ids.max()) if ids.size else None
+    elif ragged:
+        ids_t = text
+        n, L = text.shape
+        id_max = int(text.tokens.max().item()) if text.tokens.numel() else None
+        if n and bool((text.lengths() < L).any()):
+            id_max = text.pad_id if id_max is None else max(id_max, text.pad_id)
     else:
         ids_t = text.contiguous()
         id_max = int(ids_t.max().item()) if ids_t.numel() else None

@@ -246,20 +246,23 @@ def sif_embedding_device(table_t, vocab_w_t, ids_t, npc=1, gram_mode=nv.GRAM_AUT
 
 def sif_embedding_sweep(table_t, vocab_w_t, ids_t, npcs=(1,), gram_mode=nv.GRAM_AUTO):
     """SIF embeddings for K word-weight vectors x P principal-component counts (a sweep over the smoothing
-    constant ``a`` of ``a / (a + p(w))`` and over ``npc``).  All arguments are CUDA tensors: table (V, d) f32,
-    vocab_w (K, V) f32, ids (N, L) int64.  Returns float32 (K, P, N, d), P = ``len(npcs)``.
+    constant ``a`` of ``a / (a + p(w))`` and over ``npc``).  All arguments are on the device: table (V, d) f32,
+    vocab_w (K, V) f32, ids (N, L) int64 or ``RaggedIds``.  Returns float32 (K, P, N, d), P = ``len(npcs)``.
 
     One ``mmb_sif_embed_multi`` call gathers every token's row once for all K weight vectors (``emb[k]`` is bit
-    for bit ``mmb_sif_embed`` with ``vocab_w[k]``); then per k one Gram, and per (k, npc) one ``pc_from_gram``
-    (with that k's own start block when N < d) and one projection.  ``npc = 0`` is the raw weighted average.
-    With a single ``npc`` the projection runs in place: peak memory is the (K, N, d) output."""
+    for bit ``mmb_sif_embed`` with ``vocab_w[k]``); ``RaggedIds`` go through ``mmb_sif_embed_multi_ragged``
+    (``emb[k]`` is bit for bit ``mmb_sif_embed_ragged``, so ``out[k, j]`` is ``sif_embedding_ragged(table,
+    vocab_w[k], ids, npc=npcs[j])``), which walks no padding.  Then per k one Gram, and per (k, npc) one
+    ``pc_from_gram`` (with that k's own start block when N < d) and one projection.  ``npc = 0`` is the raw
+    weighted average.  With a single ``npc`` the projection runs in place: peak memory is the (K, N, d) output."""
     npcs = tuple(int(p) for p in npcs)
     if not npcs:
         raise ValueError('npcs must name at least one number of components')
     for p in npcs:
         if p < 0 or p + 10 > 32:
             raise ValueError('npc must be in 0..22')
-    if vocab_w_t.dim() != 2 or ids_t.dim() != 2:
+    ragged = isinstance(ids_t, RaggedIds)
+    if vocab_w_t.dim() != 2 or (not ragged and ids_t.dim() != 2):
         raise ValueError('vocab_w must be (K, V) and ids (n_samples, seq_len)')
     n, L = ids_t.shape
     V, d = table_t.shape
@@ -271,8 +274,13 @@ def sif_embedding_sweep(table_t, vocab_w_t, ids_t, npcs=(1,), gram_mode=nv.GRAM_
     st = _status(dev)
     nbytes = lib.mmb_sif_embed_multi_workspace_bytes(V, K)
     ws = torch.empty(max(nbytes, 32), dtype=torch.uint8, device=dev)
-    nv.check(lib.mmb_sif_embed_multi(nv.ptr(table_t), V, d, nv.ptr(vocab_w_t), K, nv.ptr(ids_t), n, L, nv.ptr(emb),
-                                     nv.ptr(st), nv.ptr(ws), nbytes, nv.stream_ptr()))
+    if ragged:
+        nv.check(lib.mmb_sif_embed_multi_ragged(nv.ptr(table_t), V, d, nv.ptr(vocab_w_t), K, nv.ptr(ids_t.tokens),
+                                                nv.ptr(ids_t.offsets), n, L, ids_t.pad_id, nv.ptr(emb), nv.ptr(st),
+                                                nv.ptr(ws), nbytes, nv.stream_ptr()))
+    else:
+        nv.check(lib.mmb_sif_embed_multi(nv.ptr(table_t), V, d, nv.ptr(vocab_w_t), K, nv.ptr(ids_t), n, L,
+                                         nv.ptr(emb), nv.ptr(st), nv.ptr(ws), nbytes, nv.stream_ptr()))
     nv.raise_on_status(st, V)
     del ws
     in_place = len(npcs) == 1
