@@ -173,6 +173,13 @@ MMB_API int mmb_start_block_xt(const float* X, int64_t N, int d, const double* O
  * out = X - (X pc^T) pc  (npc == 1: line 78; npc > 1: line 80).  out may alias X.      */
 MMB_API int mmb_remove_pc(const float* X, int64_t N, int d, const float* pc, int npc, float* out,
                   mmb_stream_t stream);
+/* mmb_remove_pc for P component sets against ONE read of X: out[j] = X - (X pc[j]^T) pc[j], each out[j]
+ * bit-identical to mmb_remove_pc(X, pc[j], npc[j]); npc[j] = 0 copies X (pc[j] may then be NULL).
+ * pc and out are HOST arrays of P DEVICE pointers (pc[j]: npc[j] x d, out[j]: N x d); npc is a HOST
+ * array.  Any P >= 1: one launch per group of up to 8 consecutive sets whose components fit 128 KB of
+ * shared memory.  out[j] may alias X only when P == 1.  N == 0 launches nothing (X, out[j] may be NULL). */
+MMB_API int mmb_remove_pc_multi(const float* X, int64_t N, int d, int P, const float* const* pc, const int* npc,
+                                float* const* out, mmb_stream_t stream);
 
 /* get_sentence_embeddings -- sif.py:84-94 on ONE device, everything resident in HBM:
  * embed -> Gram -> components (npc, 0 = skip PC removal) -> projection, no host sync.
@@ -213,6 +220,8 @@ MMB_API int mmb_host_pipeline_trim(size_t keep_bytes);
  * Sums are taken in rank order, so all ranks obtain identical bits.  A peer that never arrives
  * sets MMB_STATUS_COMM_TIMEOUT in `status` after ~4 s instead of hanging.                    */
 MMB_API size_t mmb_comm_bytes(void);
+/* Capacity of one exchange slot: the largest vector mmb_allreduce_peer sums in one call (4 MiB). */
+MMB_API size_t mmb_comm_slot_bytes(void);
 MMB_API int mmb_comm_alloc(void** buf);
 MMB_API int mmb_comm_free(void* buf);
 MMB_API int mmb_comm_export(void* buf, void* handle64);

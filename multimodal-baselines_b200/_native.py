@@ -56,6 +56,7 @@ SIGNATURES = {
     'mmb_pc_from_gram': (_i, [_p, _i, _p, _i, _i, _i, _i, _p, _p, _sz, _p]),
     'mmb_start_block_xt': (_i, [_p, _i64, _i, _p, _i, _p, _p]),
     'mmb_remove_pc': (_i, [_p, _i64, _i, _p, _i, _p, _p]),
+    'mmb_remove_pc_multi': (_i, [_p, _i64, _i, _i, _p, _p, _p, _p]),
     'mmb_sif_workspace_bytes': (_sz, [_i64, _i, _i]),
     'mmb_sif_embedding': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _i, _p, _p, _p, _p, _p, _sz, _i, _p, _p]),
     'mmb_sif_embedding_host': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _i, _p, _p, _i, _p, _i, _i64]),
@@ -64,6 +65,7 @@ SIGNATURES = {
     'mmb_host_pipeline_trim': (_i, [_sz]),
     'mmb_comm_abort': (_i, [_i, _i, _p, C.c_uint64, _p]),
     'mmb_comm_bytes': (_sz, []),
+    'mmb_comm_slot_bytes': (_sz, []),
     'mmb_comm_alloc': (_i, [C.POINTER(_p)]),
     'mmb_comm_free': (_i, [_p]),
     'mmb_comm_export': (_i, [_p, _p]),

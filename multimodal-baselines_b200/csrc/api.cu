@@ -79,7 +79,7 @@ __global__ void f32_to_f64_kernel(const float* __restrict__ in, double* __restri
 
 using namespace mmb;
 
-extern "C" int mmb_version(void) { return 102; }
+extern "C" int mmb_version(void) { return 103; }
 
 extern "C" const char* mmb_last_error(void) { return g_err; }
 

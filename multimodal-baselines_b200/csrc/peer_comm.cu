@@ -93,6 +93,8 @@ using namespace mmb;
 
 extern "C" size_t mmb_comm_bytes(void) { return kCommBytes; }
 
+extern "C" size_t mmb_comm_slot_bytes(void) { return kCommSlotBytes; }
+
 extern "C" int mmb_comm_alloc(void** buf) {
   MMB_REQUIRE(buf, "null pointer");
   MMB_CUDA(cudaMalloc(buf, kCommBytes));

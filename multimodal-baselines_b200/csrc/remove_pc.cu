@@ -10,6 +10,59 @@ namespace mmb {
 constexpr int kRmWarps = 8;
 constexpr int kRmMaxPc = 8;  // components kept in shared memory per pass
 
+// One warp per row: x[] (and its copy r[]) holds lane's float4 columns lane, lane + 32, ... (zero past d4).
+template <int NCH>
+__device__ __forceinline__ void load_row(const float4* X4, int64_t i, int d4, int lane, float4 (&x)[NCH],
+                                         float4 (&r)[NCH]) {
+#pragma unroll
+  for (int c = 0; c < NCH; ++c) {
+    const int k = lane + 32 * c;
+    x[c] = k < d4 ? ld_stream(X4 + (size_t)i * d4 + k) : make_float4(0.f, 0.f, 0.f, 0.f);
+    r[c] = x[c];
+  }
+}
+
+// r -= sum_p dot(x, pc[p]) pc[p] with every dot taken from x (pc: npc x d4 in shared memory); r enters as x.
+template <int NCH>
+__device__ __forceinline__ void subtract_pcs(const float4 (&x)[NCH], float4 (&r)[NCH], const float4* spc, int npc,
+                                             int d4, int lane) {
+  for (int p = 0; p < npc; ++p) {
+    float dot = 0.f;
+#pragma unroll
+    for (int c = 0; c < NCH; ++c) {
+      const int k = lane + 32 * c;
+      if (k < d4) {
+        const float4 v = spc[p * d4 + k];
+        dot = fmaf(x[c].x, v.x, dot);
+        dot = fmaf(x[c].y, v.y, dot);
+        dot = fmaf(x[c].z, v.z, dot);
+        dot = fmaf(x[c].w, v.w, dot);
+      }
+    }
+    dot = warp_sum(dot);
+#pragma unroll
+    for (int c = 0; c < NCH; ++c) {
+      const int k = lane + 32 * c;
+      if (k < d4) {
+        const float4 v = spc[p * d4 + k];
+        r[c].x = fmaf(-dot, v.x, r[c].x);
+        r[c].y = fmaf(-dot, v.y, r[c].y);
+        r[c].z = fmaf(-dot, v.z, r[c].z);
+        r[c].w = fmaf(-dot, v.w, r[c].w);
+      }
+    }
+  }
+}
+
+template <int NCH>
+__device__ __forceinline__ void store_row(float4* out4, int64_t i, int d4, int lane, const float4 (&r)[NCH]) {
+#pragma unroll
+  for (int c = 0; c < NCH; ++c) {
+    const int k = lane + 32 * c;
+    if (k < d4) st_stream(out4 + (size_t)i * d4 + k, r[c]);
+  }
+}
+
 template <int NCH>
 __global__ void __launch_bounds__(kRmWarps * 32)
     remove_pc_kernel(const float4* __restrict__ X4, int64_t N, int d4, const float4* __restrict__ pc4,
@@ -22,42 +75,58 @@ __global__ void __launch_bounds__(kRmWarps * 32)
   const int64_t nwarps = (int64_t)gridDim.x * kRmWarps;
   for (int64_t i = warp0; i < N; i += nwarps) {
     float4 x[NCH], r[NCH];
+    load_row<NCH>(X4, i, d4, lane, x, r);
+    subtract_pcs<NCH>(x, r, spc, npc, d4, lane);
+    store_row<NCH>(out4, i, d4, lane, r);
+  }
+}
+
+// Several component sets against one read of X: out[j] = X - (X pc_j^T) pc_j for every set j of the group,
+// each bit for bit what remove_pc_kernel writes for that set alone (npc_j = 0 copies X).
+constexpr int kRmMultiSets = 8;                     // sets per launch
+constexpr size_t kRmMultiSmemBytes = 128 * 1024;    // components per launch: one set of 32 x 1024 floats fits
+
+struct RmSets {
+  const float4* pc[kRmMultiSets];
+  float4* out[kRmMultiSets];
+  int npc[kRmMultiSets];
+  int off[kRmMultiSets];  // first float4 of set j's components in shared memory
+  int n;
+};
+
+template <int NCH>
+__global__ void __launch_bounds__(kRmWarps * 32)
+    remove_pc_multi_kernel(const float4* X4, int64_t N, int d4, const RmSets sets) {
+  extern __shared__ float4 spc[];
+  // the per-set table goes to shared memory: indexing the parameter arrays with a run-time j would copy them
+  // to local memory
+  __shared__ float4* s_out[kRmMultiSets];
+  __shared__ int s_npc[kRmMultiSets], s_off[kRmMultiSets];
 #pragma unroll
-    for (int c = 0; c < NCH; ++c) {
-      const int k = lane + 32 * c;
-      x[c] = k < d4 ? ld_stream(X4 + (size_t)i * d4 + k) : make_float4(0.f, 0.f, 0.f, 0.f);
-      r[c] = x[c];
-    }
-    for (int p = 0; p < npc; ++p) {
-      float dot = 0.f;
-#pragma unroll
-      for (int c = 0; c < NCH; ++c) {
-        const int k = lane + 32 * c;
-        if (k < d4) {
-          const float4 v = spc[p * d4 + k];
-          dot = fmaf(x[c].x, v.x, dot);
-          dot = fmaf(x[c].y, v.y, dot);
-          dot = fmaf(x[c].z, v.z, dot);
-          dot = fmaf(x[c].w, v.w, dot);
-        }
+  for (int j = 0; j < kRmMultiSets; ++j) {
+    if (j < sets.n) {
+      for (int k = threadIdx.x; k < sets.npc[j] * d4; k += blockDim.x) spc[sets.off[j] + k] = sets.pc[j][k];
+      if (threadIdx.x == 0) {
+        s_out[j] = sets.out[j];
+        s_npc[j] = sets.npc[j];
+        s_off[j] = sets.off[j];
       }
-      dot = warp_sum(dot);
-#pragma unroll
-      for (int c = 0; c < NCH; ++c) {
-        const int k = lane + 32 * c;
-        if (k < d4) {
-          const float4 v = spc[p * d4 + k];
-          r[c].x = fmaf(-dot, v.x, r[c].x);
-          r[c].y = fmaf(-dot, v.y, r[c].y);
-          r[c].z = fmaf(-dot, v.z, r[c].z);
-          r[c].w = fmaf(-dot, v.w, r[c].w);
-        }
-      }
     }
+  }
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  const int64_t warp0 = (int64_t)blockIdx.x * kRmWarps + (threadIdx.x >> 5);
+  const int64_t nwarps = (int64_t)gridDim.x * kRmWarps;
+  for (int64_t i = warp0; i < N; i += nwarps) {
+    float4 x[NCH], r[NCH];
+    load_row<NCH>(X4, i, d4, lane, x, r);
+    for (int j = 0; j < sets.n; ++j) {
+      if (j > 0) {
 #pragma unroll
-    for (int c = 0; c < NCH; ++c) {
-      const int k = lane + 32 * c;
-      if (k < d4) st_stream(out4 + (size_t)i * d4 + k, r[c]);
+        for (int c = 0; c < NCH; ++c) r[c] = x[c];
+      }
+      subtract_pcs<NCH>(x, r, spc + s_off[j], s_npc[j], d4, lane);
+      store_row<NCH>(s_out[j], i, d4, lane, r);
     }
   }
 }
@@ -96,5 +165,60 @@ extern "C" int mmb_remove_pc(const float* X, int64_t N, int d, const float* pc, 
   }
 #undef RM_LAUNCH
   MMB_LAUNCH_CHECK("remove_pc");
+  return MMB_OK;
+}
+
+extern "C" int mmb_remove_pc_multi(const float* X, int64_t N, int d, int P, const float* const* pc, const int* npc,
+                                   float* const* out, mmb_stream_t stream) {
+  // N == 0 touches no row, so X and out[j] may then be NULL (the data pointer of an empty tensor)
+  MMB_REQUIRE(pc && npc && out && (X || N == 0), "null pointer");
+  MMB_REQUIRE(d > 0 && d % 4 == 0 && d <= 1024, "d must be a multiple of 4, <= 1024");
+  MMB_REQUIRE(P > 0, "P must be >= 1");
+  MMB_REQUIRE(N >= 0, "negative size");
+  for (int j = 0; j < P; ++j) {
+    MMB_REQUIRE(npc[j] >= 0 && npc[j] <= 32, "npc must be in [0, 32]");
+    MMB_REQUIRE((out[j] || N == 0) && (pc[j] || npc[j] == 0), "null pointer");
+    MMB_REQUIRE(P == 1 || N == 0 || out[j] != X, "out may alias X only when P == 1");
+  }
+  if (N == 0) return MMB_OK;
+  const int d4 = d / 4, nch = (d4 + 31) / 32;
+  int64_t blocks = ceil_div(N, kRmWarps);
+  int64_t cap = (int64_t)sm_count() * 8;
+  const int grid = (int)(blocks < cap ? blocks : cap);
+  cudaStream_t st = as_stream(stream);
+  for (int j0 = 0; j0 < P;) {
+    // a group: up to kRmMultiSets consecutive sets whose components fit kRmMultiSmemBytes (a single set always does)
+    RmSets sets;
+    sets.n = 0;
+    size_t smem = 0;
+    while (j0 + sets.n < P && sets.n < kRmMultiSets) {
+      const int j = j0 + sets.n;
+      const size_t bytes = (size_t)npc[j] * d4 * sizeof(float4);
+      if (sets.n > 0 && smem + bytes > kRmMultiSmemBytes) break;
+      sets.pc[sets.n] = (const float4*)pc[j];
+      sets.out[sets.n] = (float4*)out[j];
+      sets.npc[sets.n] = npc[j];
+      sets.off[sets.n] = (int)(smem / sizeof(float4));
+      smem += bytes;
+      ++sets.n;
+    }
+#define RMM_LAUNCH(NCH)                                                                                       \
+  do {                                                                                                        \
+    if (smem > 48 * 1024)                                                                                     \
+      MMB_CUDA(cudaFuncSetAttribute(remove_pc_multi_kernel<NCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                    (int)kRmMultiSmemBytes));                                                 \
+    remove_pc_multi_kernel<NCH><<<grid, kRmWarps * 32, smem, st>>>((const float4*)X, N, d4, sets);            \
+  } while (0)
+    switch (nch) {
+      case 1: RMM_LAUNCH(1); break;
+      case 2: RMM_LAUNCH(2); break;
+      case 3: RMM_LAUNCH(3); break;
+      case 4: RMM_LAUNCH(4); break;
+      default: RMM_LAUNCH(8);
+    }
+#undef RMM_LAUNCH
+    MMB_LAUNCH_CHECK("remove_pc_multi");
+    j0 += sets.n;
+  }
   return MMB_OK;
 }

@@ -323,6 +323,83 @@ def sharded_sif_embedding(table_t, vocab_w_t, ids_local_t, n_global, lo, npc=1, 
     return emb, pc, st
 
 
+def exchange_sweep_(G, S0_blocks=(), comm=None, group=None, slot_bytes=None):
+    """Sum the sweep's stacked Grams G (K, d, d) float32 and its float64 start blocks over the ranks, in place.
+    With a ``PeerComm`` the Grams go in groups of floor(slot / (4 d^2)) (11 at d = 300) and the start blocks
+    (flattened back to back) in slot-sized pieces, one ``allreduce_`` per group; otherwise one
+    ``torch.distributed`` all-reduce for each of the two stacks.  The group sizes depend only on the shapes,
+    so every rank issues the same exchange sequence.  ``slot_bytes`` defaults to ``mmb_comm_slot_bytes()``."""
+    S0_blocks = list(S0_blocks)
+    flat = torch.cat([b.reshape(-1) for b in S0_blocks]) if S0_blocks else None
+    if comm is None:
+        allreduce_sum_(G, group)
+        if flat is not None:
+            allreduce_sum_(flat, group)
+    else:
+        if slot_bytes is None:
+            import _native as nv
+            slot_bytes = nv.lib.mmb_comm_slot_bytes()
+        K, d, _ = G.shape
+        per = slot_bytes // (4 * d * d)
+        if per < 1:
+            raise ValueError('a %d x %d Gram does not fit the %d-byte exchange slot' % (d, d, slot_bytes))
+        for k in range(0, K, per):
+            comm.allreduce_(G[k:k + per])
+        if flat is not None:
+            step = slot_bytes // 8
+            for i in range(0, flat.numel(), step):
+                comm.allreduce_(flat[i:i + step])
+    if flat is not None:
+        i = 0
+        for b in S0_blocks:
+            b.copy_(flat[i:i + b.numel()].view_as(b))
+            i += b.numel()
+    return G
+
+
+def sharded_sif_embedding_sweep(table_t, vocab_w_t, ids_local, n_global, lo, npcs=(1,), group=None, gram_mode=0,
+                                timers=None, comm='auto'):
+    """The SIF sweep (``sif_functions.sif_embedding_sweep``: K word-weight vectors x P component counts) on this
+    rank's block of a split of `n_global` utterances.
+
+    table_t (V, d) f32, vocab_w_t (K, V) f32, ids_local (n_local, L) int64 or ``RaggedIds`` of this rank's
+    block -- CUDA tensors on this rank's device.  Returns ``(out, pcs, st)``: out (K, P, n_local, d) float32
+    (in place over the embeddings when P = 1), ``pcs[k][j]`` the (npcs[j], d) components (None for npc = 0,
+    identical bits on every rank) and the status word, which this call does not read: check it afterwards
+    (``_native.raise_on_status(st, V)`` raises ``IndexError`` for a bad id), so that a bad id on one rank never
+    leaves its peers waiting in the exchange.
+
+    Stages (each followed by ``timers(name)`` when given, as in ``sharded_sif_embedding``): 'embed' (one
+    multi-vector gather), 'gram' (K local Grams), 'allreduce' (the stacked Grams, and for n_global < d the K x P
+    start blocks, summed over the ranks -- see ``exchange_sweep_``), 'pc' (replicated solves with the global
+    N), 'project' (one ``mmb_remove_pc_multi`` per k).  With the peer exchange ``out[k, j]`` is bit for bit
+    ``sharded_sif_embedding(table_t, vocab_w_t[k], ids_local, n_global, lo, npc=npcs[j])``'s result on padded
+    ids.  Every rank, an empty block included, must make the call with the same K, d and npcs."""
+    import sif_functions as sf
+
+    mark = timers or (lambda name: None)
+    npcs = sf.sweep_npcs(npcs)
+    emb, st = sf.sweep_embed(table_t, vocab_w_t, ids_local)
+    mark('embed')
+    out = sf.sweep_output(emb, npcs)
+    K, n_local, d = emb.shape
+    if n_global == 0:
+        return out, [[None] * len(npcs) for _ in range(K)], st
+    G = S0 = None
+    if any(npcs):
+        if comm == 'auto':
+            comm = default_comm(group)
+        G = sf.sweep_grams(emb, gram_mode)
+        mark('gram')
+        if n_global < d:
+            S0 = [[local_start_block(emb[k], n_global, lo, p, sf.start_block) if p else None for p in npcs]
+                  for k in range(K)]
+        exchange_sweep_(G, [b for row in S0 for b in row if b is not None] if S0 else (), comm, group)
+        mark('allreduce')
+    pcs = sf.sweep_solve_project(emb, G, npcs, n_global, out, S0=S0, mark=mark)
+    return out, pcs, st
+
+
 def cpu_reference_partition(X_blocks):
     """Host-side statement of the exchange step used by the CPU tests: the sum of per-shard
     Grams equals the Gram of the concatenation."""

@@ -11,6 +11,8 @@ removes several numbers of principal components: a sweep over SIF's ``a`` and ``
 
 There is no CPU fallback: without the built library or without a CUDA device these raise.
 """
+import ctypes as C
+
 import numpy as np
 import torch
 
@@ -244,23 +246,21 @@ def sif_embedding_device(table_t, vocab_w_t, ids_t, npc=1, gram_mode=nv.GRAM_AUT
     return (emb, pc) if return_pc else emb
 
 
-def sif_embedding_sweep(table_t, vocab_w_t, ids_t, npcs=(1,), gram_mode=nv.GRAM_AUTO):
-    """SIF embeddings for K word-weight vectors x P principal-component counts (a sweep over the smoothing
-    constant ``a`` of ``a / (a + p(w))`` and over ``npc``).  All arguments are on the device: table (V, d) f32,
-    vocab_w (K, V) f32, ids (N, L) int64 or ``RaggedIds``.  Returns float32 (K, P, N, d), P = ``len(npcs)``.
-
-    One ``mmb_sif_embed_multi`` call gathers every token's row once for all K weight vectors (``emb[k]`` is bit
-    for bit ``mmb_sif_embed`` with ``vocab_w[k]``); ``RaggedIds`` go through ``mmb_sif_embed_multi_ragged``
-    (``emb[k]`` is bit for bit ``mmb_sif_embed_ragged``, so ``out[k, j]`` is ``sif_embedding_ragged(table,
-    vocab_w[k], ids, npc=npcs[j])``), which walks no padding.  Then per k one Gram, and per (k, npc) one
-    ``pc_from_gram`` (with that k's own start block when N < d) and one projection.  ``npc = 0`` is the raw
-    weighted average.  With a single ``npc`` the projection runs in place: peak memory is the (K, N, d) output."""
+def sweep_npcs(npcs):
+    """``npcs`` as a tuple of ints in 0..22 (``ValueError`` otherwise)."""
     npcs = tuple(int(p) for p in npcs)
     if not npcs:
         raise ValueError('npcs must name at least one number of components')
     for p in npcs:
         if p < 0 or p + 10 > 32:
             raise ValueError('npc must be in 0..22')
+    return npcs
+
+
+def sweep_embed(table_t, vocab_w_t, ids_t):
+    """The sweep's embed stage: emb (K, N, d) float32 for the K rows of vocab_w (K, V) over one gather
+    (``mmb_sif_embed_multi``, or ``mmb_sif_embed_multi_ragged`` for ``RaggedIds``), and the status word, which
+    the caller checks.  Shape errors raise before any launch."""
     ragged = isinstance(ids_t, RaggedIds)
     if vocab_w_t.dim() != 2 or (not ragged and ids_t.dim() != 2):
         raise ValueError('vocab_w must be (K, V) and ids (n_samples, seq_len)')
@@ -281,22 +281,74 @@ def sif_embedding_sweep(table_t, vocab_w_t, ids_t, npcs=(1,), gram_mode=nv.GRAM_
     else:
         nv.check(lib.mmb_sif_embed_multi(nv.ptr(table_t), V, d, nv.ptr(vocab_w_t), K, nv.ptr(ids_t), n, L,
                                          nv.ptr(emb), nv.ptr(st), nv.ptr(ws), nbytes, nv.stream_ptr()))
-    nv.raise_on_status(st, V)
-    del ws
-    in_place = len(npcs) == 1
-    out = emb.unsqueeze(1) if in_place else torch.empty((K, len(npcs), n, d), dtype=torch.float32, device=dev)
+    return emb, st
+
+
+def sweep_grams(emb, gram_mode=nv.GRAM_AUTO):
+    """``G[k] = emb[k]^T emb[k]`` into one (K, d, d) float32 tensor (zeros when N = 0); one workspace serves
+    all K Grams (the same stream orders its uses)."""
+    K, n, d = emb.shape
     if n == 0:
-        return out
+        return torch.zeros((K, d, d), dtype=torch.float32, device=emb.device)
+    G = torch.empty((K, d, d), dtype=torch.float32, device=emb.device)
+    nbytes = lib.mmb_gram_workspace_bytes(n, d, gram_mode)
+    ws = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=emb.device)
     for k in range(K):
-        E = emb[k]
-        G = gram(E, gram_mode) if any(npcs) else None
-        for j, p in enumerate(npcs):
-            if p == 0:
-                if not in_place:
-                    out[k, j].copy_(E)
-                continue
-            pc = pc_from_gram(G, p, n, X_t=E)
-            project_out(E, pc, out=out[k, j])
+        nv.check(lib.mmb_gram(nv.ptr(emb[k]), n, d, nv.ptr(G[k]), nv.ptr(ws), nbytes, gram_mode, nv.stream_ptr()))
+    return G
+
+
+def sweep_output(emb, npcs):
+    """The (K, P, N, d) result: ``emb`` itself (as (K, 1, N, d)) when P = 1, so the projection runs in place."""
+    K, n, d = emb.shape
+    if len(npcs) == 1:
+        return emb.unsqueeze(1)
+    return torch.empty((K, len(npcs), n, d), dtype=torch.float32, device=emb.device)
+
+
+def sweep_solve_project(emb, G, npcs, n_rows, out, S0=None, mark=None):
+    """The sweep's last two stages.  Solve: ``pcs[k][j]`` = ``pc_from_gram(G[k], npcs[j], n_rows)`` (None for
+    npc = 0), with ``n_rows`` the global N; for N < d the start block is ``S0[k][j]`` when given (summed over
+    ranks by the caller), else ``emb[k]^T Omega`` of this device.  Project: one ``mmb_remove_pc_multi`` per k
+    writes ``out[k, j]`` for every j from one read of ``emb[k]``.  Returns ``pcs``."""
+    K, n, d = emb.shape
+    pcs = [[pc_from_gram(G[k], p, n_rows, X_t=emb[k], S0_t=None if S0 is None else S0[k][j]) if p else None
+            for j, p in enumerate(npcs)] for k in range(K)]
+    if mark:
+        mark('pc')
+    P = len(npcs)
+    if any(npcs) or P > 1:          # P = 1, npc = 0: out is emb, nothing to write
+        npc_arr = (C.c_int * P)(*npcs)
+        for k in range(K):
+            pc_arr = (C.c_void_p * P)(*[pc.data_ptr() if pc is not None else None for pc in pcs[k]])
+            out_arr = (C.c_void_p * P)(*[out[k, j].data_ptr() for j in range(P)])
+            nv.check(lib.mmb_remove_pc_multi(nv.ptr(emb[k]), n, d, P, pc_arr, npc_arr, out_arr, nv.stream_ptr()))
+    if mark:
+        mark('project')
+    return pcs
+
+
+def sif_embedding_sweep(table_t, vocab_w_t, ids_t, npcs=(1,), gram_mode=nv.GRAM_AUTO):
+    """SIF embeddings for K word-weight vectors x P principal-component counts (a sweep over the smoothing
+    constant ``a`` of ``a / (a + p(w))`` and over ``npc``).  All arguments are on the device: table (V, d) f32,
+    vocab_w (K, V) f32, ids (N, L) int64 or ``RaggedIds``.  Returns float32 (K, P, N, d), P = ``len(npcs)``.
+
+    One ``mmb_sif_embed_multi`` call gathers every token's row once for all K weight vectors (``emb[k]`` is bit
+    for bit ``mmb_sif_embed`` with ``vocab_w[k]``); ``RaggedIds`` go through ``mmb_sif_embed_multi_ragged``
+    (``emb[k]`` is bit for bit ``mmb_sif_embed_ragged``, so ``out[k, j]`` is ``sif_embedding_ragged(table,
+    vocab_w[k], ids, npc=npcs[j])``), which walks no padding.  Then per k one Gram, per (k, npc) one
+    ``pc_from_gram`` (with that k's own start block when N < d), and per k one ``mmb_remove_pc_multi`` that
+    writes all P columns from one read of ``emb[k]`` (``out[k, j]`` is bit for bit ``mmb_remove_pc`` with that
+    component).  ``npc = 0`` is the raw weighted average.  With a single ``npc`` the projection runs in place:
+    peak memory is the (K, N, d) output."""
+    npcs = sweep_npcs(npcs)
+    emb, st = sweep_embed(table_t, vocab_w_t, ids_t)
+    nv.raise_on_status(st, table_t.shape[0])
+    out = sweep_output(emb, npcs)
+    if emb.shape[1] == 0:
+        return out
+    G = sweep_grams(emb, gram_mode) if any(npcs) else None
+    sweep_solve_project(emb, G, npcs, emb.shape[1], out)
     return out
 
 
