@@ -160,7 +160,8 @@ MMB_API int mmb_gram(const float* X, int64_t N, int d, float* G, void* ws, size_
  * k = npc + 10): S0 = RandomState(0).normal(size=(d,k)) when N >= d (transposed = 0), or
  * X^T RandomState(0).normal(size=(N,k)) when N < d (transposed = 1); see
  * oracle/sif_oracle.py:compute_pc_from_gram.  pc is (npc, d) float32, unit rows, largest
- * |entry| of each row positive (sklearn svd_flip, u_based_decision=False).  One CTA, FP64.
+ * |entry| of each row positive (sklearn svd_flip, u_based_decision=False).  FP64, as a
+ * chain of n_iter + 3 kernels on `stream`.  Needs 1 <= d <= 512 and 1 <= npc <= k <= 32.
  * `ws` is scratch of at least mmb_pc_workspace_bytes(d, k) bytes.                      */
 MMB_API size_t mmb_pc_workspace_bytes(int d, int k);
 MMB_API int mmb_pc_from_gram(const float* G, int d, const double* S0, int k, int npc, int transposed,

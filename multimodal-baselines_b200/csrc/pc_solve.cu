@@ -8,285 +8,15 @@
 //            W = Y R^-1 with T = R^T R            (sklearn: right singular vectors of Q_x^T X)
 //   N <  d : components = Q * top eigenvectors of T   (sklearn works on X^T: Rayleigh-Ritz)
 //   rows unit-normalised, largest-|entry| of each row made positive (svd_flip, v-based).
-// The problem is d x k with d = 300 and k = npc + 10, so it runs as ONE CTA in FP64 (thread
-// i owns row i), entirely on the device: no host round trip between the Gram and the
-// projection pass (SURVEY.md H5).  orth() is CholeskyQR2 with rank-deficient columns dropped;
-// the k x k symmetric eigenproblems use cyclic Jacobi on one warp.
-#include <stdlib.h>
-
-#include "common.cuh"
-
-namespace mmb {
-
-constexpr int kPcMaxK = 32;
-
-struct PcSmem {
-  double S[kPcMaxK][kPcMaxK];   // small symmetric matrix / Cholesky factor R (upper)
-  double Vv[kPcMaxK][kPcMaxK];  // Jacobi eigenvectors
-  double lam[kPcMaxK];
-  double red[32];
-  int drop[kPcMaxK];
-  int order[kPcMaxK];
-  int flag;
-};
-
-// S[a][b] = sum_i A[i][a] * B[i][b] for a,b < k (A, B are d x k in global memory). Warps take
-// (a,b) pairs round-robin; lanes stride over rows; fixed order -> deterministic.
-__device__ void small_gram(PcSmem& sm, const double* A, const double* B, int d, int k, bool symmetric) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
-  for (int p = warp; p < k * k; p += nwarps) {
-    const int a = p / k, b = p % k;
-    if (symmetric && b < a) continue;
-    double s = 0.0;
-    for (int i = lane; i < d; i += 32) s = fma(A[(size_t)i * k + a], B[(size_t)i * k + b], s);
-    s = warp_sum(s);
-    if (lane == 0) {
-      sm.S[a][b] = s;
-      if (symmetric) sm.S[b][a] = s;
-    }
-  }
-  __syncthreads();
-}
-
-// In-place upper Cholesky S = R^T R (right-looking, warp 0, lane j owns column j); columns
-// whose pivot is not positive relative to the largest diagonal entry are dropped (they lie in
-// the span of earlier columns).  sm.lam[c] receives 1 / R[c][c] for apply_rinv.
-__device__ void cholesky_drop(PcSmem& sm, int k) {
-  if (threadIdx.x < 32) {
-    const int j = threadIdx.x;
-    double dmax = 0.0;
-    for (int c = 0; c < k; ++c) dmax = fmax(dmax, sm.S[c][c]);
-    for (int c = 0; c < k; ++c) {
-      const double piv = sm.S[c][c];
-      const bool bad = !(piv > 1e-26 * dmax) || !isfinite(piv);
-      const double rinv = bad ? 0.0 : rsqrt(piv);
-      __syncwarp();
-      if (j == c) {
-        sm.drop[c] = bad;
-        sm.S[c][c] = bad ? 1.0 : piv * rinv;   // sqrt(piv)
-        sm.lam[c] = bad ? 0.0 : rinv;
-      }
-      double rcj = 0.0;
-      if (j > c && j < k) {
-        rcj = sm.S[c][j] * rinv;               // row c of R (0 for a dropped column)
-        sm.S[c][j] = rcj;
-      }
-      __syncwarp();
-      if (j > c && j < k) {                    // trailing update of column j, rows c+1..j
-        for (int i = c + 1; i <= j; ++i) sm.S[i][j] -= sm.S[c][i] * rcj;
-      }
-      __syncwarp();
-    }
-  }
-  __syncthreads();
-}
-
-// row <- row * R^-1 (forward substitution on this thread's row); dropped columns become 0.
-template <int KMAX>
-__device__ void apply_rinv(const PcSmem& sm, double (&q)[KMAX], int k) {
-#pragma unroll
-  for (int c = 0; c < KMAX; ++c) {
-    if (c < k) {
-      double acc = q[c];
-#pragma unroll
-      for (int a = 0; a < KMAX; ++a)
-        if (a < c) acc -= q[a] * sm.S[a][c];
-      q[c] = acc * sm.lam[c];   // lam[c] = 1 / R[c][c], 0 for a dropped column
-    }
-  }
-}
-
-template <int KMAX>
-__device__ void store_row(double* M, const double (&q)[KMAX], int row, int d, int k) {
-  if (row < d) {
-#pragma unroll
-    for (int c = 0; c < KMAX; ++c)
-      if (c < k) M[(size_t)row * k + c] = q[c];
-  }
-  __syncthreads();
-}
-
-// CholeskyQR2 on the rows held in registers; Qg (global, d x k) is scratch and ends up
-// holding the orthonormalised block.
-template <int KMAX>
-__device__ void orth(PcSmem& sm, double (&q)[KMAX], double* Qg, int row, int d, int k, int passes) {
-  for (int pass = 0; pass < passes; ++pass) {
-    store_row<KMAX>(Qg, q, row, d, k);
-    small_gram(sm, Qg, Qg, d, k, true);
-    cholesky_drop(sm, k);
-    apply_rinv<KMAX>(sm, q, k);
-    __syncthreads();
-  }
-  store_row<KMAX>(Qg, q, row, d, k);
-}
-
-// y = (G Q)[row, :], G symmetric float32 (read column `row`, i.e. coalesced across threads).
-template <int KMAX>
-__device__ void gram_times(const float* __restrict__ G, const double* Qg, double (&y)[KMAX], int row,
-                           int d, int k) {
-#pragma unroll
-  for (int c = 0; c < KMAX; ++c) y[c] = 0.0;
-  if (row < d) {
-    for (int j = 0; j < d; ++j) {
-      const double g = (double)__ldg(G + (size_t)j * d + row);
-#pragma unroll
-      for (int c = 0; c < KMAX; ++c)
-        if (c < k) y[c] = fma(g, Qg[(size_t)j * k + c], y[c]);
-    }
-  }
-}
-
-// Cyclic Jacobi on sm.S (k x k symmetric, k <= 32) by warp 0; eigenvalues -> sm.lam,
-// eigenvectors (columns) -> sm.Vv; sm.order = indices by descending eigenvalue.
-__device__ void jacobi_eig(PcSmem& sm, int k) {
-  if (threadIdx.x < 32) {
-    const int l = threadIdx.x;
-    for (int c = 0; c < k; ++c)
-      if (l < k) sm.Vv[l][c] = (l == c) ? 1.0 : 0.0;
-    __syncwarp();
-    for (int sweep = 0; sweep < 16; ++sweep) {
-      double off = 0.0, dg = 0.0;
-      if (l < k) {
-        for (int c = 0; c < k; ++c) {
-          const double v = sm.S[l][c];
-          if (c > l) off += v * v;
-          if (c == l) dg += v * v;
-        }
-      }
-      off = warp_sum(off);
-      dg = warp_sum(dg);
-      if (!(off > 1e-27 * dg)) break;   // off-diagonal mass below ~3e-14 of the diagonal: converged
-      for (int p = 0; p < k - 1; ++p) {
-        for (int q = p + 1; q < k; ++q) {
-          const double apq = sm.S[p][q];
-          if (fabs(apq) > 1e-17 * sqrt(fabs(sm.S[p][p] * sm.S[q][q])) && fabs(apq) > 1e-300) {
-            const double app = sm.S[p][p], aqq = sm.S[q][q];
-            const double theta = (aqq - app) / (2.0 * apq);
-            const double t = (theta >= 0.0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
-            const double c = 1.0 / sqrt(t * t + 1.0), s = t * c;
-            __syncwarp();
-            if (l < k) {
-              const double vlp = sm.Vv[l][p], vlq = sm.Vv[l][q];
-              sm.Vv[l][p] = c * vlp - s * vlq;
-              sm.Vv[l][q] = s * vlp + c * vlq;
-              if (l != p && l != q) {
-                const double alp = sm.S[l][p], alq = sm.S[l][q];
-                const double nlp = c * alp - s * alq, nlq = s * alp + c * alq;
-                sm.S[l][p] = nlp; sm.S[p][l] = nlp;
-                sm.S[l][q] = nlq; sm.S[q][l] = nlq;
-              }
-            }
-            if (l == 0) {
-              sm.S[p][p] = app - t * apq;
-              sm.S[q][q] = aqq + t * apq;
-              sm.S[p][q] = 0.0;
-              sm.S[q][p] = 0.0;
-            }
-            __syncwarp();
-          }
-        }
-      }
-    }
-    if (l < k) sm.lam[l] = sm.S[l][l];
-    __syncwarp();
-    if (l == 0) {  // selection sort, descending, stable in index
-      bool used[kPcMaxK];
-      for (int c = 0; c < k; ++c) used[c] = false;
-      for (int r = 0; r < k; ++r) {
-        int best = -1;
-        for (int c = 0; c < k; ++c)
-          if (!used[c] && (best < 0 || sm.lam[c] > sm.lam[best])) best = c;
-        used[best] = true;
-        sm.order[r] = best;
-      }
-    }
-  }
-  __syncthreads();
-}
-
-template <int KMAX>
-__global__ void __launch_bounds__(512)
-    pc_from_gram_kernel(const float* __restrict__ G, int d, const double* __restrict__ S0, int k,
-                        int npc, int transposed, int n_iter, float* __restrict__ pc, double* ws) {
-  __shared__ PcSmem sm;
-  double* Qg = ws;                     // d x k
-  double* Yg = ws + (size_t)d * k;     // d x k
-  double* cbuf = Yg + (size_t)d * k;   // d
-  const int row = threadIdx.x;
-  double q[KMAX], y[KMAX];
-#pragma unroll
-  for (int c = 0; c < KMAX; ++c) q[c] = (row < d && c < k) ? S0[(size_t)row * k + c] : 0.0;
-  if (threadIdx.x < kPcMaxK) sm.drop[threadIdx.x] = 0;
-  __syncthreads();
-
-  // Only the span matters between multiplications, so one CholeskyQR pass keeps the block
-  // well enough conditioned there; the last one is repeated (CholeskyQR2) for orthonormality.
-  orth<KMAX>(sm, q, Qg, row, d, k, n_iter == 0 ? 2 : 1);
-  for (int it = 0; it < n_iter; ++it) {
-    gram_times<KMAX>(G, Qg, y, row, d, k);
-    __syncthreads();  // everyone has finished reading Qg
-#pragma unroll
-    for (int c = 0; c < KMAX; ++c) q[c] = y[c];
-    orth<KMAX>(sm, q, Qg, row, d, k, it + 1 == n_iter ? 2 : 1);
-  }
-  gram_times<KMAX>(G, Qg, y, row, d, k);
-  store_row<KMAX>(Yg, y, row, d, k);
-  small_gram(sm, Qg, Yg, d, k, false);   // T = Q^T Y
-  if (threadIdx.x < k) {                 // symmetrise
-    const int a = threadIdx.x;
-    for (int b = a + 1; b < k; ++b) {
-      const double m = 0.5 * (sm.S[a][b] + sm.S[b][a]);
-      sm.S[a][b] = m;
-      sm.S[b][a] = m;
-    }
-  }
-  __syncthreads();
-
-  // y becomes this thread's row of the basis the components are expressed in
-  if (transposed) {
-#pragma unroll
-    for (int c = 0; c < KMAX; ++c) y[c] = q[c];
-    jacobi_eig(sm, k);
-  } else {
-    cholesky_drop(sm, k);
-    apply_rinv<KMAX>(sm, y, k);
-    __syncthreads();
-    store_row<KMAX>(Yg, y, row, d, k);
-    small_gram(sm, Yg, Yg, d, k, true);  // W^T W
-    jacobi_eig(sm, k);
-  }
-
-  for (int c = 0; c < npc; ++c) {
-    const int sel = sm.order[c];
-    double v = 0.0;
-#pragma unroll
-    for (int a = 0; a < KMAX; ++a)
-      if (a < k) v = fma(y[a], sm.Vv[a][sel], v);
-    if (row < d) cbuf[row] = v;
-    __syncthreads();
-    if (threadIdx.x == 0) {  // norm + sklearn's sign rule (first arg-max of |v|)
-      double n2 = 0.0, best = -1.0;
-      int arg = 0;
-      for (int i = 0; i < d; ++i) {
-        const double x = cbuf[i];
-        n2 = fma(x, x, n2);
-        if (fabs(x) > best) { best = fabs(x); arg = i; }
-      }
-      const double sgn = cbuf[arg] < 0.0 ? -1.0 : 1.0;
-      sm.red[0] = sgn / sqrt(n2);
-    }
-    __syncthreads();
-    if (row < d) pc[(size_t)c * d + row] = (float)(v * sm.red[0]);
-    __syncthreads();
-  }
-}
-
-// ------------------------------------------------------------------------------------------
-// Grid-parallel variant ("pcm"): the same arithmetic as pc_from_gram_kernel above, organised for
-// latency.  The chain of 2 n_iter + 4 dependent steps is what every rank waits for between the
-// Gram all-reduce and the projection pass (SURVEY.md H5); measured on B200 the one-CTA kernel
-// spends 1.35 ms in it, instruction-issue bound (one CTA, mostly one warp).  Here the chain is
-// n_iter + 3 small kernels on the same stream:
+// The problem is d x k (d <= 512, k = npc + 10 <= 32).  It runs in FP64 entirely on the device:
+// no host round trip between the Gram and the projection pass (SURVEY.md H5).  orth() is
+// CholeskyQR with rank-deficient columns dropped, repeated (CholeskyQR2) where the result must be
+// orthonormal and not only span the right space.
+//
+// The chain of 2 n_iter + 4 dependent steps is what every rank waits for between the Gram
+// all-reduce and the projection pass, so it is organised for latency (run by one CTA, the chain is
+// instruction-issue bound and took 1.35 ms on a B200).  It runs as n_iter + 3 small kernels on one
+// stream:
 //   prep   : S0 -> column-major Y_0, per-CTA partials of Y_0^T Y_0;
 //   iter i : EVERY CTA sums the partials (fixed order), factorises the k x k matrix and forms
 //            Q_i = orth(Y_i) for all d rows redundantly -- no CTA ever waits for a serial CTA --
@@ -297,6 +27,11 @@ __global__ void __launch_bounds__(512)
 //            several warps), components, unit norm, sklearn's sign rule.
 // Kernel boundaries are the grid-wide barriers.  Everything is summed in a fixed order, so the
 // result is deterministic and identical on every rank.
+#include "common.cuh"
+
+namespace mmb {
+
+constexpr int kPcMaxK = 32;
 constexpr int kPcmRows = 8;        // rows of Y per CTA in the iteration kernels
 constexpr int kPcmThreads = 320;
 
@@ -478,12 +213,8 @@ template <int KMAX>
 __global__ void __launch_bounds__(kPcmThreads)
     pcm_iter_kernel(const float* __restrict__ G, int d, int k, int KP, int DP, int nb,
                     const double* __restrict__ Yprev, double* __restrict__ Ynext, double* __restrict__ Qout,
-                    const double* __restrict__ SpartIn, double* __restrict__ SpartOut, int passes, int last,
-                    long long* __restrict__ tlog) {
+                    const double* __restrict__ SpartIn, double* __restrict__ SpartOut, int passes, int last) {
   extern __shared__ __align__(16) unsigned char pcm_smem[];
-  int tl = 0;
-#define PCM_MARK() do { if (tlog && blockIdx.x == 0 && threadIdx.x == 0) tlog[tl++] = clock64(); } while (0)
-  PCM_MARK();
   PcmSmall& sm = *reinterpret_cast<PcmSmall*>(pcm_smem);
   double* Qt = reinterpret_cast<double*>(pcm_smem + ((sizeof(PcmSmall) + 15) & ~(size_t)15));   // [KP][DP]
   double* red = Qt + (size_t)KP * DP;                                // [JS][kPcmRows][KP]
@@ -514,9 +245,7 @@ __global__ void __launch_bounds__(kPcmThreads)
 #pragma unroll
   for (int c = 0; c < KMAX; ++c) q[c] = (c < k && myrow < d) ? Yprev[(size_t)c * DP + myrow] : 0.0;
   __syncthreads();
-  PCM_MARK();
   pcm_cholesky(sm, k, last ? 2 : 1);
-  PCM_MARK();
   // Q = Y R^-1 for all rows (redundantly in every CTA), column-major in shared memory
   if (myrow < DP) {
     pcm_solve_row<KMAX>(sm, q, k);
@@ -548,7 +277,6 @@ __global__ void __launch_bounds__(kPcmThreads)
     }
     __syncthreads();
   }
-  PCM_MARK();
   // Y rows of this CTA: tile = (row, 4 columns), j split over JS thread groups
   {
     const int t = threadIdx.x;
@@ -573,7 +301,6 @@ __global__ void __launch_bounds__(kPcmThreads)
     }
   }
   __syncthreads();
-  PCM_MARK();
   for (int i = threadIdx.x; i < kPcmRows * KP; i += kPcmThreads) {
     const int r = i / KP, c = i - r * KP, row = row0 + r;
     double s = 0.0;
@@ -598,8 +325,6 @@ __global__ void __launch_bounds__(kPcmThreads)
     }
     SpartOut[(size_t)blockIdx.x * KP * KP + a * KP + b] = s;
   }
-  PCM_MARK();
-#undef PCM_MARK
 }
 
 // Symmetric eigenproblem of sm.S (k <= 32), all warps of the CTA: Jacobi with the round-robin
@@ -771,11 +496,8 @@ template <int KMAX>
 __global__ void __launch_bounds__(kPcmThreads)
     pcm_final_kernel(int d, int k, int KP, int DP, int nb, int npc, int transposed,
                      const double* __restrict__ Y, const double* __restrict__ Q,
-                     const double* __restrict__ Tpart, float* __restrict__ pc, long long* __restrict__ tlog) {
+                     const double* __restrict__ Tpart, float* __restrict__ pc) {
   extern __shared__ __align__(16) unsigned char pcm_smem[];
-  int tl = 0;
-#define PCM_MARK() do { if (tlog && threadIdx.x == 0) tlog[tl++] = clock64(); } while (0)
-  PCM_MARK();
   PcmSmall& sm = *reinterpret_cast<PcmSmall*>(pcm_smem);
   double* Wt = reinterpret_cast<double*>(pcm_smem + ((sizeof(PcmSmall) + 15) & ~(size_t)15));   // [KP][DP]
   double* cvec = Wt + (size_t)KP * DP;                                                            // [DP]
@@ -794,7 +516,6 @@ __global__ void __launch_bounds__(kPcmThreads)
     }
   }
   __syncthreads();
-  PCM_MARK();
   if (transposed) {      // Rayleigh-Ritz vectors of G on span(Q)
     for (int i = threadIdx.x; i < KP * DP; i += kPcmThreads) Wt[i] = Q[i];
     __syncthreads();
@@ -811,12 +532,9 @@ __global__ void __launch_bounds__(kPcmThreads)
         if (c < KP) Wt[(size_t)c * DP + row] = q[c];
     }
     __syncthreads();
-    PCM_MARK();
     pcm_small_gram(sm, Wt, Wt, d, k, DP, true);
-    PCM_MARK();
     if (!(npc == 1 && k * k <= kPcmThreads && pcm_top1(sm, k))) pcm_jacobi(sm, k);
   }
-  PCM_MARK();
   for (int c = 0; c < npc; ++c) {
     const int sel = sm.order[c];
     for (int row = threadIdx.x; row < d; row += kPcmThreads) {
@@ -847,8 +565,6 @@ __global__ void __launch_bounds__(kPcmThreads)
     for (int row = threadIdx.x; row < d; row += kPcmThreads) pc[(size_t)c * d + row] = (float)(cvec[row] * sm.red[0]);
     __syncthreads();
   }
-  PCM_MARK();
-#undef PCM_MARK
 }
 
 struct PcmPlan {
@@ -868,7 +584,7 @@ static PcmPlan pcm_plan(int d, int k) {
   P.smem_iter = small + (P.blk + (size_t)(P.JS > 0 ? P.JS : 1) * kPcmRows * P.KP + kPcmRows * P.KP) * sizeof(double) +
                 (size_t)kPcmRows * d * sizeof(float);
   P.smem_final = small + (P.blk + P.DP) * sizeof(double);
-  P.ws_bytes = (3 * P.blk + 2 * P.spart) * sizeof(double) + 4096;   // + clock log (MMB_PC_TIMING)
+  P.ws_bytes = (3 * P.blk + 2 * P.spart) * sizeof(double);
   return P;
 }
 
@@ -879,9 +595,6 @@ static int pcm_run(const float* G, int d, const double* S0, int k, int npc, int 
   double* Yb[2] = {ws, ws + P.blk};
   double* Qg = ws + 2 * P.blk;
   double* Sp[2] = {ws + 3 * P.blk, ws + 3 * P.blk + P.spart};
-  // MMB_PC_TIMING=1: thread 0 of CTA 0 logs clock64() at phase boundaries (16 slots per kernel)
-  static const bool timing = getenv("MMB_PC_TIMING") && atoi(getenv("MMB_PC_TIMING")) != 0;
-  long long* tlog = timing ? (long long*)(ws + 3 * P.blk + 2 * P.spart) : nullptr;
   static bool attr_set = false;
   if (!attr_set) {
     MMB_CUDA(cudaFuncSetAttribute(pcm_iter_kernel<KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
@@ -907,7 +620,7 @@ static int pcm_run(const float* G, int d, const double* S0, int k, int npc, int 
     cfg.dynamicSmemBytes = P.smem_iter;
     MMB_CUDA(cudaLaunchKernelEx(&cfg, pcm_iter_kernel<KMAX>, G, d, k, P.KP, P.DP, P.nb, (const double*)Yb[cur],
                                 Yb[cur ^ 1], Qg, (const double*)Sp[cur], Sp[cur ^ 1], it == n_iter ? 2 : 1,
-                                it == n_iter ? 1 : 0, tlog ? tlog + 16 * (it < 8 ? it : 8) : (long long*)nullptr));
+                                it == n_iter ? 1 : 0));
     count_launch("pcm_iter");
   }
   const int fin = (n_iter + 1) & 1;
@@ -915,8 +628,7 @@ static int pcm_run(const float* G, int d, const double* S0, int k, int npc, int 
   cfg.blockDim = dim3(kPcmThreads);
   cfg.dynamicSmemBytes = P.smem_final;
   MMB_CUDA(cudaLaunchKernelEx(&cfg, pcm_final_kernel<KMAX>, d, k, P.KP, P.DP, P.nb, npc, transposed,
-                              (const double*)Yb[fin], (const double*)Qg, (const double*)Sp[fin], pc,
-                              tlog ? tlog + 16 * 10 : (long long*)nullptr));
+                              (const double*)Yb[fin], (const double*)Qg, (const double*)Sp[fin], pc));
   count_launch("pcm_final");
   return MMB_OK;
 }
@@ -936,11 +648,7 @@ __global__ void start_block_xt_kernel(const float* __restrict__ X, int64_t N, in
 
 using namespace mmb;
 
-extern "C" size_t mmb_pc_workspace_bytes(int d, int k) {
-  const size_t one_cta = ((size_t)2 * d * k + d) * sizeof(double);
-  const size_t grid = pcm_plan(d, k).ws_bytes;
-  return one_cta > grid ? one_cta : grid;
-}
+extern "C" size_t mmb_pc_workspace_bytes(int d, int k) { return pcm_plan(d, k).ws_bytes; }
 
 extern "C" int mmb_pc_from_gram(const float* G, int d, const double* S0, int k, int npc,
                                 int transposed, int n_iter, float* pc, void* ws, size_t ws_bytes,
@@ -950,22 +658,12 @@ extern "C" int mmb_pc_from_gram(const float* G, int d, const double* S0, int k, 
   MMB_REQUIRE(k > 0 && k <= kPcMaxK && npc > 0 && npc <= k, "need 0 < npc <= k <= 32");
   MMB_REQUIRE(ws_bytes >= mmb_pc_workspace_bytes(d, k), "workspace too small");
   MMB_REQUIRE(n_iter >= 0, "n_iter < 0");
-  // grid-parallel chain of small kernels (default); MMB_PC_SOLVER=0 selects the one-CTA kernel
-  static const bool one_cta = getenv("MMB_PC_SOLVER") && atoi(getenv("MMB_PC_SOLVER")) == 0;
-  const PcmPlan P = pcm_plan(d, k);
-  if (!one_cta && P.JS >= 1 && P.nb <= 64 && P.smem_iter <= 200 * 1024 && P.smem_final <= 200 * 1024) {
-    return k <= 16 ? pcm_run<16>(G, d, S0, k, npc, transposed, n_iter, pc, (double*)ws, as_stream(stream))
-                   : pcm_run<32>(G, d, S0, k, npc, transposed, n_iter, pc, (double*)ws, as_stream(stream));
-  }
-  const int threads = ((d + 31) / 32) * 32;
-  if (k <= 16)
-    pc_from_gram_kernel<16><<<1, threads, 0, as_stream(stream)>>>(G, d, S0, k, npc, transposed, n_iter,
-                                                                 pc, (double*)ws);
-  else
-    pc_from_gram_kernel<32><<<1, threads, 0, as_stream(stream)>>>(G, d, S0, k, npc, transposed, n_iter,
-                                                                 pc, (double*)ws);
-  MMB_LAUNCH_CHECK("pc_from_gram");
-  return MMB_OK;
+  // The checks above keep every launch of the chain within its limits: d <= 512 and k <= 32 give
+  // nb <= 64 CTAs (the partial sums read at most 64 slots), JS >= 5 j slices, and at most
+  // 186,576 B of dynamic shared memory in pcm_iter_kernel and 162,008 B in pcm_final_kernel
+  // (both under the 200 KiB pcm_run requests).
+  return k <= 16 ? pcm_run<16>(G, d, S0, k, npc, transposed, n_iter, pc, (double*)ws, as_stream(stream))
+                 : pcm_run<32>(G, d, S0, k, npc, transposed, n_iter, pc, (double*)ws, as_stream(stream));
 }
 
 extern "C" int mmb_start_block_xt(const float* X, int64_t N, int d, const double* Omega, int k,

@@ -17,7 +17,8 @@ The exchange has two implementations:
     NVLink peer memory (CUDA IPC buffers), fused into the kernel that finishes the Gram
     (``mmb_gram_allreduce_peer``) -- ranks add in rank order, so every rank holds identical bits;
   * ``torch.distributed.all_reduce`` (NCCL on GPUs, gloo on CPU): the fallback for any other
-    topology, and what tests/test_dist_cpu.py exercises for the partition / reduction arithmetic.
+    topology or backend, the path a caller selects with ``comm=None``, and what
+    tests/test_dist_cpu.py exercises for the partition / reduction arithmetic.
 """
 import ctypes as C
 import os
@@ -216,11 +217,12 @@ _DEFAULT_COMM = {}
 
 def default_comm(group=None):
     """The process-wide PeerComm of `group` (created on first use), or None when the exchange
-    should go through torch.distributed (no process group, one rank, non-NCCL backend, or
-    MMB_PEER_COMM=0)."""
+    goes through torch.distributed: no process group, one rank, a non-NCCL backend, more than
+    8 ranks or more than one host.  To use torch.distributed on purpose, pass ``comm=None`` to
+    the sharded entry points instead of the default ``'auto'``."""
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) < 2:
         return None
-    if os.environ.get('MMB_PEER_COMM', '1') == '0' or dist.get_backend(group) != 'nccl':
+    if dist.get_backend(group) != 'nccl':
         return None
     key = id(group)
     if key not in _DEFAULT_COMM:

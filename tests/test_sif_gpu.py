@@ -12,6 +12,7 @@ pytestmark = pytest.mark.gpu
 
 EMB_RTOL = 1e-5     # north_star: embeddings within 1e-5 relative
 PC_COS = 0.9999     # north_star: |cos| >= 0.9999 up to sign
+PC_SOLVE_TOL = 1e-12   # 1 - signed cos of mmb_pc_from_gram vs the oracle on the same Gram (~10x the B200 worst case)
 
 
 @pytest.fixture(scope='module')
@@ -93,6 +94,34 @@ def test_compute_pc_matches_sklearn(mods, golden_dir, tag, npc):
     rm = sf.remove_pc(X, npc)
     assert rm.dtype == np.float64
     assert np.max(np.abs(rm[:16] - g['%s_rm%d' % (tag, npc)])) < 2e-4 * np.abs(X).max()
+
+
+@pytest.mark.parametrize('d,n,npc', [(512, 2048, 22),   # k = 32 at the largest d
+                                     (512, 384, 22),    # k = 32, N < d: Rayleigh-Ritz on span(X^T Omega)
+                                     (8, 256, 2),       # tiny d: k = 12 > d, dependent columns dropped
+                                     (129, 1000, 3),    # odd d
+                                     (129, 1000, 1),    # npc = 1: the power-iteration fast path
+                                     (129, 64, 1)])     # npc = 1, N < d
+def test_pc_from_gram_matches_oracle(mods, d, n, npc):
+    """The component solve alone, across its (d, k) range, against the float64 oracle on the same
+    float32 Gram and start block.  X has singular values 0.9^i (floored at 0.9^40), so the leading
+    eigenvalues of G are well separated and each component is defined to the last bit of float32."""
+    import torch
+    nv, sf, sif = mods
+    rng = np.random.default_rng(d * 1000 + n + npc)
+    m = min(n, d)
+    P, _ = np.linalg.qr(rng.standard_normal((n, m)))
+    U, _ = np.linalg.qr(rng.standard_normal((d, m)))
+    X = (P * 0.9 ** np.minimum(np.arange(m), 40)) @ U.T
+    G = (X.T @ X).astype(np.float32)
+    S0 = X.T @ sf.start_block(n, npc) if n < d else sf.start_block(d, npc)
+    dev = torch.device('cuda')
+    pc = sf.pc_from_gram(torch.as_tensor(G, device=dev), npc, n, S0_t=torch.as_tensor(S0, device=dev))
+    got = pc.double().cpu().numpy()
+    want = so.compute_pc_from_gram(G.astype(np.float64), S0, npc, transposed=n < d)
+    assert got.shape == want.shape == (npc, d)
+    cos = np.sum(got * want, axis=1) / (np.linalg.norm(got, axis=1) * np.linalg.norm(want, axis=1))
+    assert np.all(1.0 - cos < PC_SOLVE_TOL), (d, n, npc, 1.0 - cos)
 
 
 @pytest.mark.parametrize('n,L,V,d', [(1, 1, 5, 300), (7, 33, 50, 300), (300, 64, 1000, 300),

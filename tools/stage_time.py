@@ -2,7 +2,7 @@
 slice of the bench workload, plus correctness of the Gram and the component solve against float64
 torch.  PROFILE_N sets the number of utterances (default 4 M); IDS=uniform draws the ids uniformly
 instead of from the bench's Zipf law.  Every output line is tagged with IDS and any MMB_* variable
-set, such as MMB_PC_SOLVER:   PROFILE_N=4000000 python tools/stage_time.py"""
+set, such as MMB_BENCH_V:   PROFILE_N=4000000 python tools/stage_time.py"""
 import os
 import sys
 
