@@ -204,6 +204,27 @@ MMB_API int mmb_sif_embedding_host(const float* table_dev, int64_t V, int d, con
                            const double* Omega_host, void* emb_host, int emb_f64,
                            float* pc_host, int gram_mode, int64_t chunk_rows);
 
+/* The SIF sweep (mmb_sif_embed_multi, then per k one Gram, per (k, npc) one component solve and per k one
+ * mmb_remove_pc_multi) with HOST buffers, as get_sentence_embeddings_sweep's NumPy caller sees it: x_host (N, L) in,
+ * out_host (K, P, N, d) out, float64 when out_f64 != 0 (each value the float32 result widened once), else float32.
+ * W_dev is (K, V) float32 on the device.  npcs and Omega_host are HOST arrays of P entries: Omega_host[j] is the
+ * seeded start block for npcs[j] (d x (npc + 10) when N >= d, N x (npc + 10) when N < d, float64), NULL when
+ * npcs[j] == 0.  out[k, j] is bit-identical to the device sweep's out[k, j] at every chunk_rows:
+ *   1. ids H2D in chunks of chunk_rows utterances (<= 0: 2^18), double-buffered, overlapped with the K-vector
+ *      embed of each chunk into a resident (K, N, d) float32 tensor (variant rule taken on the whole N);
+ *   2. per k one mmb_gram over the whole emb[k] (gram_mode resolved on N, as the device sweep does), then one
+ *      mmb_pc_from_gram per npc != 0 (start block mmb_start_block_xt(emb[k]) when N < d);
+ *   3. per k and chunk of at most chunk_rows rows, one projection writes all P sets from one read of the rows
+ *      into a (P, rows, d) staging buffer of the output type (at most 256 MB, so rows shrink as P grows),
+ *      overlapped with P plain D2H copies of the previous chunk into out_host[k, j, r0 : r1].
+ * Device memory: K * N * d * 4 bytes, plus two id buffers, two staging buffers and the Gram / solve scratch,
+ * none of which grows with P.  x_host and out_host should be pinned (mmb_host_alloc) for full PCIe rate.
+ * Synchronous.  N == 0 returns at once; a bad id is MMB_E_INDEX once every stream has drained.            */
+MMB_API int mmb_sif_embedding_sweep_host(const float* table_dev, int64_t V, int d, const float* W_dev, int K,
+                                         const int64_t* x_host, int64_t N, int64_t L, int P, const int* npcs,
+                                         const double* const* Omega_host, void* out_host, int out_f64,
+                                         int gram_mode, int64_t chunk_rows);
+
 /* The *_host entry points take their staging buffers from a private stream-ordered pool per device
  * that keeps freed blocks for the next call; this returns all but `keep_bytes` of them to the driver. */
 MMB_API int mmb_host_pipeline_trim(size_t keep_bytes);

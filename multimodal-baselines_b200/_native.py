@@ -62,6 +62,7 @@ SIGNATURES = {
     'mmb_sif_embedding_host': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _i, _p, _p, _i, _p, _i, _i64]),
     'mmb_sif_embedding_host_peer': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _i, _p, _p, _i, _p, _i, _i64, _i64, _i, _i,
                                          _p, C.c_uint64]),
+    'mmb_sif_embedding_sweep_host': (_i, [_p, _i64, _i, _p, _i, _p, _i64, _i64, _i, _p, _p, _p, _i, _i, _i64]),
     'mmb_host_pipeline_trim': (_i, [_sz]),
     'mmb_comm_abort': (_i, [_i, _i, _p, C.c_uint64, _p]),
     'mmb_comm_bytes': (_sz, []),

@@ -79,7 +79,7 @@ __global__ void f32_to_f64_kernel(const float* __restrict__ in, double* __restri
 
 using namespace mmb;
 
-extern "C" int mmb_version(void) { return 103; }
+extern "C" int mmb_version(void) { return 104; }
 
 extern "C" const char* mmb_last_error(void) { return g_err; }
 
@@ -148,6 +148,12 @@ namespace mmb {   // implemented in sif_embed.cu
 int sif_prescale(const float* table, int64_t V, int d, const float* vocab_w, void* ws, cudaStream_t st);
 int sif_embed_prescaled(const float* table, int64_t V, int d, const float* vocab_w, const void* ws, const int64_t* x,
                         int64_t N, int64_t L, float* emb, int* status, cudaStream_t st);
+// implemented in sif_embed_multi.cu / remove_pc.cu (used by mmb_sif_embedding_sweep_host)
+int sif_embed_multi_weights(const float* vocab_w, int64_t V, int d, int K, void* ws, cudaStream_t st);
+int sif_embed_multi_chunk(const float* table, int64_t V, int d, const void* ws, int K, const int64_t* x,
+                          int64_t rows, int64_t L, int64_t N_total, float* emb, int* status, cudaStream_t st);
+int remove_pc_multi(const float* X, int64_t N, int d, int P, const float* const* pc, const int* npc,
+                    void* const* out, bool f64, cudaStream_t st);
 }  // namespace mmb
 
 struct SifWs {
@@ -309,6 +315,73 @@ struct AbortGuard {
     if (armed) mmb_comm_abort(hc.rank, hc.world, hc.bufs, hc.epoch, (mmb_stream_t)st);
   }
 };
+
+// Rows per chunk of a *_host call: 2^18 by default (chunk_rows <= 0), at most N.
+int64_t host_chunk_rows(int64_t chunk_rows, int64_t N) {
+  if (chunk_rows <= 0) chunk_rows = 1 << 18;
+  if (chunk_rows > N) chunk_rows = N > 0 ? N : 1;
+  return chunk_rows;
+}
+
+// The copy streams start once the allocations and uploads enqueued on `comp` so far are done.
+int copy_streams_after_setup(Streams& S) {
+  cudaEvent_t allocs_done;
+  int rc = S.event(&allocs_done);
+  if (rc) return rc;
+  MMB_CUDA(cudaEventRecord(allocs_done, S.comp));
+  MMB_CUDA(cudaStreamWaitEvent(S.in, allocs_done, 0));
+  MMB_CUDA(cudaStreamWaitEvent(S.out, allocs_done, 0));
+  return MMB_OK;
+}
+
+// Phase 1 of the *_host calls: the ids H2D in chunks of chunk_rows utterances (stream `in`, the two id buffers in
+// turn) overlapped with the embed of the previous chunk (stream `comp`).  Per chunk, embed(ids_dev, r0, rows)
+// enqueues the embed on `comp`; once its id buffer is free again, after(c, r0, rows) enqueues what else the chunk
+// needs there.
+template <class Embed, class After>
+int stream_ids_in(Streams& S, DevBuf (&ids)[2], const int64_t* x_host, int64_t N, int64_t L, int64_t chunk_rows,
+                  Embed&& embed, After&& after) {
+  cudaEvent_t in_ready[2], buf_free[2];
+  int rc;
+  for (int b = 0; b < 2; ++b) {
+    if ((rc = S.event(&in_ready[b]))) return rc;
+    if ((rc = S.event(&buf_free[b]))) return rc;
+  }
+  const int64_t nchunks = ceil_div(N, chunk_rows);
+  for (int64_t c = 0; c < nchunks; ++c) {
+    const int b = (int)(c & 1);
+    const int64_t r0 = c * chunk_rows;
+    const int64_t rows = (N - r0) < chunk_rows ? (N - r0) : chunk_rows;
+    if (c >= 2) MMB_CUDA(cudaStreamWaitEvent(S.in, buf_free[b], 0));
+    MMB_CUDA(cudaMemcpyAsync(ids[b].p, x_host + r0 * L, (size_t)rows * L * sizeof(int64_t),
+                             cudaMemcpyHostToDevice, S.in));
+    MMB_CUDA(cudaEventRecord(in_ready[b], S.in));
+    MMB_CUDA(cudaStreamWaitEvent(S.comp, in_ready[b], 0));
+    if ((rc = embed((const int64_t*)ids[b].p, r0, rows))) return rc;
+    MMB_CUDA(cudaEventRecord(buf_free[b], S.comp));
+    if ((rc = after(c, r0, rows))) return rc;
+  }
+  return MMB_OK;
+}
+
+// The end of a *_host call: the status word read back behind everything on `comp`, all three streams drained, and
+// the status turned into its error code.
+int finish_host_call(Streams& S, const DevBuf& status, int64_t V) {
+  int h_status = 0;
+  MMB_CUDA(cudaMemcpyAsync(&h_status, status.p, sizeof(int), cudaMemcpyDeviceToHost, S.comp));
+  MMB_CUDA(cudaStreamSynchronize(S.comp));
+  MMB_CUDA(cudaStreamSynchronize(S.out));
+  MMB_CUDA(cudaStreamSynchronize(S.in));
+  if (h_status & MMB_STATUS_COMM_TIMEOUT) {
+    set_error("peer all-reduce timed out: a rank never raised its flag");
+    return MMB_E_COMM;
+  }
+  if (h_status & MMB_STATUS_BAD_INDEX) {
+    set_error("index out of bounds: a token id is outside [-%lld, %lld)", (long long)V, (long long)V);
+    return MMB_E_INDEX;
+  }
+  return MMB_OK;
+}
 }  // namespace
 
 static int sif_embedding_host_impl(const float* table_dev, int64_t V, int d, const float* vocab_w_dev,
@@ -323,8 +396,7 @@ static int sif_embedding_host_impl(const float* table_dev, int64_t V, int d, con
   const int64_t n_global = dist ? hc.n_global : N;
   MMB_REQUIRE(!dist || n_global >= d, "the multi-GPU host path needs N_global >= d (use sif_dist for tiny splits)");
   if (N == 0 && !(dist && npc > 0)) return MMB_OK;
-  if (chunk_rows <= 0) chunk_rows = 1 << 18;
-  if (chunk_rows > N) chunk_rows = N > 0 ? N : 1;
+  chunk_rows = host_chunk_rows(chunk_rows, N);
   const int64_t nchunks = ceil_div(N, chunk_rows);
   const int k = npc + 10;
 
@@ -362,49 +434,34 @@ static int sif_embedding_host_impl(const float* table_dev, int64_t V, int d, con
     if ((rc = scaled.alloc(scaled_bytes, S.comp))) return rc;
     if ((rc = sif_prescale(table_dev, V, d, vocab_w_dev, scaled.p, S.comp))) return rc;
   }
-  cudaEvent_t allocs_done;
-  if ((rc = S.event(&allocs_done))) return rc;
-  MMB_CUDA(cudaEventRecord(allocs_done, S.comp));
-  MMB_CUDA(cudaStreamWaitEvent(S.in, allocs_done, 0));
-  MMB_CUDA(cudaStreamWaitEvent(S.out, allocs_done, 0));
+  if ((rc = copy_streams_after_setup(S))) return rc;
 
   // phase 1: ids H2D (stream `in`) overlapped with the embed kernel (stream `comp`)
-  cudaEvent_t in_ready[2], buf_free[2];
-  for (int b = 0; b < 2; ++b) {
-    if ((rc = S.event(&in_ready[b]))) return rc;
-    if ((rc = S.event(&buf_free[b]))) return rc;
-  }
-  for (int64_t c = 0; c < nchunks; ++c) {
-    const int b = (int)(c & 1);
-    const int64_t r0 = c * chunk_rows;
-    const int64_t rows = (N - r0) < chunk_rows ? (N - r0) : chunk_rows;
-    if (c >= 2) MMB_CUDA(cudaStreamWaitEvent(S.in, buf_free[b], 0));
-    MMB_CUDA(cudaMemcpyAsync(ids[b].p, x_host + r0 * L, (size_t)rows * L * sizeof(int64_t),
-                             cudaMemcpyHostToDevice, S.in));
-    MMB_CUDA(cudaEventRecord(in_ready[b], S.in));
-    MMB_CUDA(cudaStreamWaitEvent(S.comp, in_ready[b], 0));
-    if (scaled_bytes)
-      rc = sif_embed_prescaled(table_dev, V, d, vocab_w_dev, scaled.p, (const int64_t*)ids[b].p, rows, L,
-                               (float*)emb.p + r0 * d, (int*)status.p, S.comp);
-    else
-      rc = mmb_sif_embed(table_dev, V, d, vocab_w_dev, (const int64_t*)ids[b].p, rows, L,
-                         (float*)emb.p + r0 * d, (int*)status.p, S.comp);
-    if (rc) return rc;
-    MMB_CUDA(cudaEventRecord(buf_free[b], S.comp));
-    if (chunked_gram) {
-      // The compute stream idles while the next chunk's ids cross PCIe: take the chunk's Gram now
-      // and add it to the running sum (chunk order -> deterministic), so that only the component
-      // solve separates the last H2D from the first D2H.
-      SifWs Lw = sif_ws_layout(N, d, npc);
-      char* base = (char*)ws.p;
-      float* G = (float*)(base + Lw.G);
-      rc = mmb_gram((const float*)emb.p + r0 * d, rows, d, (float*)gchunk.p, base + Lw.gram, Lw.pc - Lw.gram,
-                    gram_mode, S.comp);
-      if (rc) return rc;
-      accumulate_kernel<<<(d * d + 255) / 256, 256, 0, S.comp>>>(G, (const float*)gchunk.p, d * d, c == 0);
-      MMB_LAUNCH_CHECK("accumulate");
-    }
-  }
+  rc = stream_ids_in(
+      S, ids, x_host, N, L, chunk_rows,
+      [&](const int64_t* ids_dev, int64_t r0, int64_t rows) {
+        if (scaled_bytes)
+          return sif_embed_prescaled(table_dev, V, d, vocab_w_dev, scaled.p, ids_dev, rows, L,
+                                     (float*)emb.p + r0 * d, (int*)status.p, S.comp);
+        return mmb_sif_embed(table_dev, V, d, vocab_w_dev, ids_dev, rows, L, (float*)emb.p + r0 * d,
+                             (int*)status.p, S.comp);
+      },
+      [&](int64_t c, int64_t r0, int64_t rows) {
+        if (!chunked_gram) return (int)MMB_OK;
+        // The compute stream idles while the next chunk's ids cross PCIe: take the chunk's Gram now
+        // and add it to the running sum (chunk order -> deterministic), so that only the component
+        // solve separates the last H2D from the first D2H.
+        SifWs Lw = sif_ws_layout(N, d, npc);
+        char* base = (char*)ws.p;
+        float* G = (float*)(base + Lw.G);
+        int rc2 = mmb_gram((const float*)emb.p + r0 * d, rows, d, (float*)gchunk.p, base + Lw.gram,
+                           Lw.pc - Lw.gram, gram_mode, S.comp);
+        if (rc2) return rc2;
+        accumulate_kernel<<<(d * d + 255) / 256, 256, 0, S.comp>>>(G, (const float*)gchunk.p, d * d, c == 0);
+        MMB_LAUNCH_CHECK("accumulate");
+        return (int)MMB_OK;
+      });
+  if (rc) return rc;
   // phase 2: components from the Gram of the whole block (summed per chunk above, or taken here)
   float* pc_dev = (float*)pcv.p;
   if (npc > 0) {
@@ -469,22 +526,9 @@ static int sif_embedding_host_impl(const float* table_dev, int64_t V, int d, con
                                cudaMemcpyDeviceToHost, S.out));
     }
   }
-  int h_status = 0;
   if (pc_host && npc > 0)
     MMB_CUDA(cudaMemcpyAsync(pc_host, pc_dev, (size_t)npc * d * sizeof(float), cudaMemcpyDeviceToHost, S.comp));
-  MMB_CUDA(cudaMemcpyAsync(&h_status, status.p, sizeof(int), cudaMemcpyDeviceToHost, S.comp));
-  MMB_CUDA(cudaStreamSynchronize(S.comp));
-  MMB_CUDA(cudaStreamSynchronize(S.out));
-  MMB_CUDA(cudaStreamSynchronize(S.in));
-  if (h_status & MMB_STATUS_COMM_TIMEOUT) {
-    set_error("peer all-reduce timed out: a rank never raised its flag");
-    return MMB_E_COMM;
-  }
-  if (h_status & MMB_STATUS_BAD_INDEX) {
-    set_error("index out of bounds: a token id is outside [-%lld, %lld)", (long long)V, (long long)V);
-    return MMB_E_INDEX;
-  }
-  return MMB_OK;
+  return finish_host_call(S, status, V);
 }
 
 extern "C" int mmb_host_pipeline_trim(size_t keep_bytes) {
@@ -513,4 +557,151 @@ extern "C" int mmb_sif_embedding_host_peer(const float* table_dev, int64_t V, in
   hc.rank = rank; hc.world = world; hc.bufs = bufs; hc.epoch = epoch; hc.n_global = N_global;
   return sif_embedding_host_impl(table_dev, V, d, vocab_w_dev, x_host, N_local, L, npc, Omega_host, emb_host,
                                  emb_f64, pc_host, gram_mode, chunk_rows, hc);
+}
+
+// ---- the SIF sweep with host buffers ------------------------------------------------------------
+// One staging buffer of the projection holds at most this many bytes, whatever P is.
+static constexpr size_t kSweepStageBytes = (size_t)256 << 20;
+
+extern "C" int mmb_sif_embedding_sweep_host(const float* table_dev, int64_t V, int d, const float* W_dev, int K,
+                                            const int64_t* x_host, int64_t N, int64_t L, int P, const int* npcs,
+                                            const double* const* Omega_host, void* out_host, int out_f64,
+                                            int gram_mode, int64_t chunk_rows) {
+  MMB_REQUIRE(table_dev && W_dev && npcs && (x_host || N == 0) && (out_host || N == 0), "null pointer");
+  MMB_REQUIRE(N >= 0 && L >= 0 && d > 0 && d % 4 == 0 && d <= 1024, "bad size (d must be a multiple of 4, <= 1024)");
+  MMB_REQUIRE(V > 0 && V < (int64_t)1 << 31, "V out of range");
+  MMB_REQUIRE(K >= 1, "K must be >= 1");
+  MMB_REQUIRE(P >= 1, "P must be >= 1");
+  MMB_REQUIRE((uintptr_t)table_dev % 16 == 0, "table must be 16-byte aligned");
+  bool any_pc = false;
+  int npc_sum = 0;
+  for (int j = 0; j < P; ++j) {
+    MMB_REQUIRE(npcs[j] >= 0 && npcs[j] + 10 <= 32, "npc must be in [0, 22]");
+    MMB_REQUIRE(npcs[j] == 0 || (Omega_host && Omega_host[j]), "Omega is required when npc > 0");
+    any_pc |= npcs[j] > 0;
+    npc_sum += npcs[j];
+  }
+  if (N == 0) return MMB_OK;
+  chunk_rows = host_chunk_rows(chunk_rows, N);
+  const size_t esz = out_f64 ? sizeof(double) : sizeof(float);
+  // projection chunks: at most chunk_rows rows, and P rows of output per row within one staging buffer
+  const size_t prow_bytes = (size_t)P * d * esz;
+  int64_t out_rows = (int64_t)(kSweepStageBytes / prow_bytes);
+  if (out_rows < 1) out_rows = 1;
+  if (out_rows > chunk_rows) out_rows = chunk_rows;
+  const bool transposed = N < d;
+  const int64_t orows = transposed ? N : d;
+
+  Streams S;
+  int rc = S.init();
+  if (rc) return rc;
+  DevBuf ids[2], emb, wsm, status, G, gws, pcws, s0, pcv, omega, stage[2];
+  SyncGuard sync_guard{S};
+  const size_t ids_chunk = (size_t)chunk_rows * L * sizeof(int64_t);
+  if ((rc = ids[0].alloc(ids_chunk, S.comp))) return rc;
+  if ((rc = ids[1].alloc(ids_chunk, S.comp))) return rc;
+  if ((rc = emb.alloc((size_t)K * N * d * sizeof(float), S.comp))) return rc;
+  const size_t wsm_bytes = mmb_sif_embed_multi_workspace_bytes(V, K);
+  if ((rc = wsm.alloc(wsm_bytes, S.comp))) return rc;
+  if ((rc = status.alloc(sizeof(int), S.comp))) return rc;
+  MMB_CUDA(cudaMemsetAsync(status.p, 0, sizeof(int), S.comp));
+  for (int b = 0; b < 2; ++b)
+    if ((rc = stage[b].alloc((size_t)out_rows * prow_bytes, S.comp))) return rc;
+  // components: one Gram at a time, the P start blocks (uploaded once), the npc_sum rows of one k's components
+  std::vector<size_t> omega_off(P, 0), pc_off(P, 0);
+  size_t gws_bytes = 0, pcws_bytes = 0;
+  if (any_pc) {
+    size_t o = 0, q = 0;
+    for (int j = 0; j < P; ++j) {
+      omega_off[j] = o;
+      pc_off[j] = q;
+      if (!npcs[j]) continue;
+      o += (size_t)orows * (npcs[j] + 10);
+      q += (size_t)npcs[j] * d;
+      const size_t b = mmb_pc_workspace_bytes(d, npcs[j] + 10);
+      if (b > pcws_bytes) pcws_bytes = b;
+    }
+    gws_bytes = mmb_gram_workspace_bytes(N, d, gram_mode);
+    if ((rc = G.alloc((size_t)d * d * sizeof(float), S.comp))) return rc;
+    if ((rc = gws.alloc(gws_bytes, S.comp))) return rc;
+    if ((rc = pcws.alloc(pcws_bytes, S.comp))) return rc;
+    if ((rc = pcv.alloc(q * sizeof(float), S.comp))) return rc;
+    if ((rc = omega.alloc(o * sizeof(double), S.comp))) return rc;
+    if (transposed && (rc = s0.alloc((size_t)d * 32 * sizeof(double), S.comp))) return rc;
+    for (int j = 0; j < P; ++j)
+      if (npcs[j])
+        MMB_CUDA(cudaMemcpyAsync((double*)omega.p + omega_off[j], Omega_host[j],
+                                 (size_t)orows * (npcs[j] + 10) * sizeof(double), cudaMemcpyHostToDevice, S.comp));
+  }
+  if ((rc = sif_embed_multi_weights(W_dev, V, d, K, wsm.p, S.comp))) return rc;
+  if ((rc = copy_streams_after_setup(S))) return rc;
+
+  // phase 1: ids H2D (stream `in`) overlapped with the K-vector embed (stream `comp`) into the resident emb
+  float* E0 = (float*)emb.p;
+  rc = stream_ids_in(
+      S, ids, x_host, N, L, chunk_rows,
+      [&](const int64_t* ids_dev, int64_t r0, int64_t rows) {
+        return sif_embed_multi_chunk(table_dev, V, d, wsm.p, K, ids_dev, rows, L, N, E0 + r0 * d, (int*)status.p,
+                                     S.comp);
+      },
+      [](int64_t, int64_t, int64_t) { return (int)MMB_OK; });
+  if (rc) return rc;
+
+  // phases 2 and 3 per k: the Gram of the whole emb[k] and its components (as the device sweep takes them), then
+  // the projection of each chunk into a staging buffer (stream `comp`) overlapped with the D2H of the previous
+  // chunk (stream `out`); the next k's Gram runs while the last chunk of this k crosses PCIe
+  cudaEvent_t out_ready[2], out_free[2];
+  for (int b = 0; b < 2; ++b) {
+    if ((rc = S.event(&out_ready[b]))) return rc;
+    if ((rc = S.event(&out_free[b]))) return rc;
+  }
+  std::vector<const float*> pcs(P, nullptr);
+  std::vector<void*> outs(P, nullptr);
+  int64_t q = 0;                   // chunks projected so far, over all k
+  int64_t pend_k = 0, pend_r0 = 0, pend_rows = 0;
+  // the D2H of projected chunk q - 1: P copies from its staging buffer into out_host[k, j, r0 : r0 + rows]
+  auto copy_out = [&](int64_t qq, int64_t k, int64_t r0, int64_t rows) {
+    const int b = (int)(qq & 1);
+    MMB_CUDA(cudaStreamWaitEvent(S.out, out_ready[b], 0));
+    for (int j = 0; j < P; ++j)
+      MMB_CUDA(cudaMemcpyAsync((char*)out_host + (((size_t)k * P + j) * N + r0) * d * esz,
+                               (char*)stage[b].p + (size_t)j * rows * d * esz, (size_t)rows * d * esz,
+                               cudaMemcpyDeviceToHost, S.out));
+    MMB_CUDA(cudaEventRecord(out_free[b], S.out));
+    return (int)MMB_OK;
+  };
+  for (int k = 0; k < K; ++k) {
+    const float* E = E0 + (size_t)k * N * d;
+    if (any_pc) {
+      if ((rc = mmb_gram(E, N, d, (float*)G.p, gws.p, gws_bytes, gram_mode, S.comp))) return rc;
+      for (int j = 0; j < P; ++j) {
+        if (!npcs[j]) continue;
+        const int kk = npcs[j] + 10;
+        const double* S0 = (const double*)omega.p + omega_off[j];
+        if (transposed) {
+          if ((rc = mmb_start_block_xt(E, N, d, S0, kk, (double*)s0.p, S.comp))) return rc;
+          S0 = (const double*)s0.p;
+        }
+        float* pc = (float*)pcv.p + pc_off[j];
+        rc = mmb_pc_from_gram((const float*)G.p, d, S0, kk, npcs[j], transposed, 7, pc, pcws.p, pcws_bytes, S.comp);
+        if (rc) return rc;
+        pcs[j] = pc;
+      }
+    }
+    for (int64_t r0 = 0; r0 < N; r0 += out_rows, ++q) {
+      const int64_t rows = (N - r0) < out_rows ? (N - r0) : out_rows;
+      const int b = (int)(q & 1);
+      if (q >= 2) MMB_CUDA(cudaStreamWaitEvent(S.comp, out_free[b], 0));
+      for (int j = 0; j < P; ++j) outs[j] = (char*)stage[b].p + (size_t)j * rows * d * esz;
+      rc = remove_pc_multi(E + r0 * d, rows, d, P, pcs.data(), npcs, outs.data(), out_f64 != 0, S.comp);
+      if (rc) return rc;
+      MMB_CUDA(cudaEventRecord(out_ready[b], S.comp));
+      // enqueued after this chunk's projection, so that a D2H into pageable memory (which returns only when
+      // done) still overlaps it
+      if (q > 0 && (rc = copy_out(q - 1, pend_k, pend_r0, pend_rows))) return rc;
+      pend_k = k; pend_r0 = r0; pend_rows = rows;
+    }
+  }
+  if ((rc = copy_out(q - 1, pend_k, pend_r0, pend_rows))) return rc;
+  return finish_host_call(S, status, V);
 }

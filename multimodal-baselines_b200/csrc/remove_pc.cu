@@ -63,6 +63,20 @@ __device__ __forceinline__ void store_row(float4* out4, int64_t i, int d4, int l
   }
 }
 
+// The same row widened to float64 (one cvt per element): float4 k of the row becomes double2 2k and 2k + 1.
+template <int NCH>
+__device__ __forceinline__ void store_row(double2* out2, int64_t i, int d4, int lane, const float4 (&r)[NCH]) {
+#pragma unroll
+  for (int c = 0; c < NCH; ++c) {
+    const int k = lane + 32 * c;
+    if (k < d4) {
+      double2* p = out2 + ((size_t)i * d4 + k) * 2;
+      __stcs(p, make_double2((double)r[c].x, (double)r[c].y));
+      __stcs(p + 1, make_double2((double)r[c].z, (double)r[c].w));
+    }
+  }
+}
+
 template <int NCH>
 __global__ void __launch_bounds__(kRmWarps * 32)
     remove_pc_kernel(const float4* __restrict__ X4, int64_t N, int d4, const float4* __restrict__ pc4,
@@ -82,32 +96,33 @@ __global__ void __launch_bounds__(kRmWarps * 32)
 }
 
 // Several component sets against one read of X: out[j] = X - (X pc_j^T) pc_j for every set j of the group,
-// each bit for bit what remove_pc_kernel writes for that set alone (npc_j = 0 copies X).
+// each bit for bit what remove_pc_kernel writes for that set alone (npc_j = 0 copies X).  OutV is the output
+// vector type: float4 (float32 rows), or double2 (float64 rows: the float32 result, widened on the store).
 constexpr int kRmMultiSets = 8;                     // sets per launch
 constexpr size_t kRmMultiSmemBytes = 128 * 1024;    // components per launch: one set of 32 x 1024 floats fits
 
 struct RmSets {
   const float4* pc[kRmMultiSets];
-  float4* out[kRmMultiSets];
+  void* out[kRmMultiSets];
   int npc[kRmMultiSets];
   int off[kRmMultiSets];  // first float4 of set j's components in shared memory
   int n;
 };
 
-template <int NCH>
+template <int NCH, typename OutV>
 __global__ void __launch_bounds__(kRmWarps * 32)
     remove_pc_multi_kernel(const float4* X4, int64_t N, int d4, const RmSets sets) {
   extern __shared__ float4 spc[];
   // the per-set table goes to shared memory: indexing the parameter arrays with a run-time j would copy them
   // to local memory
-  __shared__ float4* s_out[kRmMultiSets];
+  __shared__ OutV* s_out[kRmMultiSets];
   __shared__ int s_npc[kRmMultiSets], s_off[kRmMultiSets];
 #pragma unroll
   for (int j = 0; j < kRmMultiSets; ++j) {
     if (j < sets.n) {
       for (int k = threadIdx.x; k < sets.npc[j] * d4; k += blockDim.x) spc[sets.off[j] + k] = sets.pc[j][k];
       if (threadIdx.x == 0) {
-        s_out[j] = sets.out[j];
+        s_out[j] = (OutV*)sets.out[j];
         s_npc[j] = sets.npc[j];
         s_off[j] = sets.off[j];
       }
@@ -168,8 +183,11 @@ extern "C" int mmb_remove_pc(const float* X, int64_t N, int d, const float* pc, 
   return MMB_OK;
 }
 
-extern "C" int mmb_remove_pc_multi(const float* X, int64_t N, int d, int P, const float* const* pc, const int* npc,
-                                   float* const* out, mmb_stream_t stream) {
+namespace mmb {
+
+// mmb_remove_pc_multi with out[j] float32 (f64 = false) or float64 (f64 = true, the host-buffer sweep's staging).
+int remove_pc_multi(const float* X, int64_t N, int d, int P, const float* const* pc, const int* npc,
+                    void* const* out, bool f64, cudaStream_t st) {
   // N == 0 touches no row, so X and out[j] may then be NULL (the data pointer of an empty tensor)
   MMB_REQUIRE(pc && npc && out && (X || N == 0), "null pointer");
   MMB_REQUIRE(d > 0 && d % 4 == 0 && d <= 1024, "d must be a multiple of 4, <= 1024");
@@ -185,7 +203,6 @@ extern "C" int mmb_remove_pc_multi(const float* X, int64_t N, int d, int P, cons
   int64_t blocks = ceil_div(N, kRmWarps);
   int64_t cap = (int64_t)sm_count() * 8;
   const int grid = (int)(blocks < cap ? blocks : cap);
-  cudaStream_t st = as_stream(stream);
   for (int j0 = 0; j0 < P;) {
     // a group: up to kRmMultiSets consecutive sets whose components fit kRmMultiSmemBytes (a single set always does)
     RmSets sets;
@@ -196,29 +213,43 @@ extern "C" int mmb_remove_pc_multi(const float* X, int64_t N, int d, int P, cons
       const size_t bytes = (size_t)npc[j] * d4 * sizeof(float4);
       if (sets.n > 0 && smem + bytes > kRmMultiSmemBytes) break;
       sets.pc[sets.n] = (const float4*)pc[j];
-      sets.out[sets.n] = (float4*)out[j];
+      sets.out[sets.n] = out[j];
       sets.npc[sets.n] = npc[j];
       sets.off[sets.n] = (int)(smem / sizeof(float4));
       smem += bytes;
       ++sets.n;
     }
-#define RMM_LAUNCH(NCH)                                                                                       \
-  do {                                                                                                        \
-    if (smem > 48 * 1024)                                                                                     \
-      MMB_CUDA(cudaFuncSetAttribute(remove_pc_multi_kernel<NCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                    (int)kRmMultiSmemBytes));                                                 \
-    remove_pc_multi_kernel<NCH><<<grid, kRmWarps * 32, smem, st>>>((const float4*)X, N, d4, sets);            \
+#define RMM_LAUNCH(NCH, OUTV)                                                                                       \
+  do {                                                                                                              \
+    if (smem > 48 * 1024)                                                                                           \
+      MMB_CUDA(cudaFuncSetAttribute(remove_pc_multi_kernel<NCH, OUTV>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                    (int)kRmMultiSmemBytes));                                                       \
+    remove_pc_multi_kernel<NCH, OUTV><<<grid, kRmWarps * 32, smem, st>>>((const float4*)X, N, d4, sets);            \
   } while (0)
-    switch (nch) {
-      case 1: RMM_LAUNCH(1); break;
-      case 2: RMM_LAUNCH(2); break;
-      case 3: RMM_LAUNCH(3); break;
-      case 4: RMM_LAUNCH(4); break;
-      default: RMM_LAUNCH(8);
+#define RMM_DISPATCH(OUTV)               \
+  switch (nch) {                         \
+    case 1: RMM_LAUNCH(1, OUTV); break;  \
+    case 2: RMM_LAUNCH(2, OUTV); break;  \
+    case 3: RMM_LAUNCH(3, OUTV); break;  \
+    case 4: RMM_LAUNCH(4, OUTV); break;  \
+    default: RMM_LAUNCH(8, OUTV);        \
+  }
+    if (f64) {
+      RMM_DISPATCH(double2)
+    } else {
+      RMM_DISPATCH(float4)
     }
+#undef RMM_DISPATCH
 #undef RMM_LAUNCH
     MMB_LAUNCH_CHECK("remove_pc_multi");
     j0 += sets.n;
   }
   return MMB_OK;
+}
+
+}  // namespace mmb
+
+extern "C" int mmb_remove_pc_multi(const float* X, int64_t N, int d, int P, const float* const* pc, const int* npc,
+                                   float* const* out, mmb_stream_t stream) {
+  return remove_pc_multi(X, N, d, P, pc, npc, (void* const*)out, false, as_stream(stream));
 }

@@ -138,12 +138,13 @@ __device__ __forceinline__ void accumulate_chunk_multi(RowAcc<NCH> (&acc)[KG], i
 }
 
 // Warp per utterance, the next chunk's ids in flight (sif_embed_warp_prefetch_kernel for KG vectors).  emb4 is the
-// group's first output; output k of the group is at emb4 + k * N * d4, for k < kn (the rest is padding).
+// group's first output; output k of the group is at emb4 + k * kstride * d4, for k < kn (the rest is padding).
+// kstride is the row count of one output slice: N for a whole batch, the call's total N for one chunk of it.
 template <int NCH, int KG, int UNROLL, int MINB, bool WIDE>
 __global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
     sif_embed_multi_warp_kernel(const float4* __restrict__ table4, int V, int d4, const float* __restrict__ wg,
                                 const int64_t* __restrict__ ids, int64_t N, int64_t L, int kn,
-                                float4* __restrict__ emb4, int* __restrict__ status) {
+                                float4* __restrict__ emb4, int64_t kstride, int* __restrict__ status) {
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = (int64_t)blockIdx.x * kEmbedWarps + (threadIdx.x >> 5);
   const int64_t nwarps = (int64_t)gridDim.x * kEmbedWarps;
@@ -169,19 +170,19 @@ __global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
     }
 #pragma unroll
     for (int k = 0; k < KG; ++k)
-      if (k < kn) store_row<NCH>(emb4 + ((size_t)k * N + i) * d4, acc[k], cnt[k], lane, d4);
+      if (k < kn) store_row<NCH>(emb4 + ((size_t)k * kstride + i) * d4, acc[k], cnt[k], lane, d4);
   }
   if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, MMB_STATUS_BAD_INDEX);
 }
 
 // The CTA-per-utterance epilogue: per output k the warp partials go through shared memory and are summed in warp
 // order, then divided by the utterance's count (sif_embed_cta_kernel, one k at a time so the shared footprint is the
-// single-vector kernel's).  Output k of utterance i is row (k * N + i) of emb4.
+// single-vector kernel's).  Output k of utterance i is row (k * kstride + i) of emb4.
 template <int NCH, int KG>
 __device__ __forceinline__ void cta_store_multi(float4 (&part)[kEmbedWarps][NCH * 32], int (&part_cnt)[kEmbedWarps],
                                                 const RowAcc<NCH> (&acc)[KG], const int (&cnt)[KG], int kn,
                                                 typename Live<NCH>::type tail, int lane, int warp, int d4,
-                                                float4* __restrict__ emb4, int64_t N, int64_t i) {
+                                                float4* __restrict__ emb4, int64_t kstride, int64_t i) {
 #pragma unroll
   for (int k = 0; k < KG; ++k) {
     if (k >= kn) break;
@@ -200,7 +201,7 @@ __device__ __forceinline__ void cta_store_multi(float4 (&part)[kEmbedWarps][NCH 
 #pragma unroll
     for (int w = 0; w < kEmbedWarps; ++w) total += part_cnt[w];
     const float div = (float)total;
-    float4* out = emb4 + ((size_t)k * N + i) * d4;
+    float4* out = emb4 + ((size_t)k * kstride + i) * d4;
     for (int e = threadIdx.x; e < d4; e += blockDim.x) {
       float4 s = part[0][e];
 #pragma unroll
@@ -221,7 +222,7 @@ template <int NCH, int KG, int UNROLL>
 __global__ void __launch_bounds__(kEmbedWarps * 32, 1)
     sif_embed_multi_cta_kernel(const float4* __restrict__ table4, int V, int d4, const float* __restrict__ wg,
                                const int64_t* __restrict__ ids, int64_t N, int64_t L, int kn,
-                               float4* __restrict__ emb4, int* __restrict__ status) {
+                               float4* __restrict__ emb4, int64_t kstride, int* __restrict__ status) {
   __shared__ float4 part[kEmbedWarps][NCH * 32];
   __shared__ int part_cnt[kEmbedWarps];
   const int lane = threadIdx.x & 31;
@@ -239,7 +240,7 @@ __global__ void __launch_bounds__(kEmbedWarps * 32, 1)
     for (int64_t base = 32 * (int64_t)warp; base < L; base += 32 * kEmbedWarps)
       accumulate_chunk_multi<NCH, KG, UNROLL, true, false>(acc, cnt, lane_base, V, row_bytes, tail, wg, row_ids, base,
                                                            L, lane, bad, 0);
-    cta_store_multi<NCH, KG>(part, part_cnt, acc, cnt, kn, tail, lane, warp, d4, emb4, N, i);
+    cta_store_multi<NCH, KG>(part, part_cnt, acc, cnt, kn, tail, lane, warp, d4, emb4, kstride, i);
   }
   if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, MMB_STATUS_BAD_INDEX);
 }
@@ -339,13 +340,13 @@ __global__ void __launch_bounds__(kEmbedWarps * 32, 1)
   if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, MMB_STATUS_BAD_INDEX);
 }
 
-// One gather pass: kn (<= KG) vectors whose weights are the (V, KG) block wg, outputs from emb.  With offsets (ragged
-// ids, d <= 512) ids are the CSR tokens and L is L_pad.
+// One gather pass: kn (<= KG) vectors whose weights are the (V, KG) block wg, output k at emb + k * kstride * d.
+// With offsets (ragged ids, d <= 512; kstride == N) ids are the CSR tokens and L is L_pad.
 template <int NCH, int KG>
 static int launch_multi_group(const float* table, int64_t V, int d, const float* wg, const int64_t* ids,
                               const int64_t* offsets, int64_t N, int64_t L, int64_t pad_id, int kn, float* emb,
-                              int* status, bool few_long, bool wide, int grid, cudaStream_t st, char* kname,
-                              size_t kname_len) {
+                              int64_t kstride, int* status, bool few_long, bool wide, int grid, cudaStream_t st,
+                              char* kname, size_t kname_len) {
   const int d4 = d / 4;
   // 64 accumulator registers (KG * NCH = 16): one row in flight instead of two (spills otherwise); d > 512 also
   // takes the whole register file (one CTA per SM), as the single-vector kernel's one-row configuration spills.
@@ -373,53 +374,81 @@ static int launch_multi_group(const float* table, int64_t V, int d, const float*
   }
   if (few_long) {
     sif_embed_multi_cta_kernel<NCH, KG, UNROLL><<<grid, kEmbedWarps * 32, 0, st>>>(
-        (const float4*)table, (int)V, d4, wg, ids, N, L, kn, (float4*)emb, status);
+        (const float4*)table, (int)V, d4, wg, ids, N, L, kn, (float4*)emb, kstride, status);
     snprintf(kname, kname_len, "sif_embed_multi_cta_kernel<%d,%d,%d>", NCH, KG, UNROLL);
   } else if (wide) {
     sif_embed_multi_warp_kernel<NCH, KG, UNROLL, MINB, true><<<grid, kEmbedWarps * 32, 0, st>>>(
-        (const float4*)table, (int)V, d4, wg, ids, N, L, kn, (float4*)emb, status);
+        (const float4*)table, (int)V, d4, wg, ids, N, L, kn, (float4*)emb, kstride, status);
     snprintf(kname, kname_len, "sif_embed_multi_warp_kernel<%d,%d,%d,%d,true>", NCH, KG, UNROLL, MINB);
   } else {
     sif_embed_multi_warp_kernel<NCH, KG, UNROLL, MINB, false><<<grid, kEmbedWarps * 32, 0, st>>>(
-        (const float4*)table, (int)V, d4, wg, ids, N, L, kn, (float4*)emb, status);
+        (const float4*)table, (int)V, d4, wg, ids, N, L, kn, (float4*)emb, kstride, status);
     snprintf(kname, kname_len, "sif_embed_multi_warp_kernel<%d,%d,%d,%d,false>", NCH, KG, UNROLL, MINB);
   }
   MMB_LAUNCH_CHECK("sif_embed_multi");
   return MMB_OK;
 }
 
+// Group layout of K vectors: ngroups passes of KG, the last with last_n vectors in last_w (a power of two) columns.
+struct MultiGroups {
+  int ngroups, last_n, last_w;
+};
+static MultiGroups multi_groups(int K, int KG) {
+  MultiGroups g;
+  g.ngroups = (K + KG - 1) / KG;
+  g.last_n = K - (g.ngroups - 1) * KG;
+  g.last_w = 1;
+  while (g.last_w < g.last_n) g.last_w *= 2;
+  return g;
+}
+
+// The weight re-layout into ws (multi_weights_kernel): once per call, before any gather.
 template <int NCH>
-static int launch_multi(const float* table, int64_t V, int d, const float* vocab_w, int K, const int64_t* ids,
-                        const int64_t* offsets, int64_t N, int64_t L, int64_t pad_id, float* emb, int* status,
-                        float* ws, cudaStream_t st) {
+static int multi_weights(const float* vocab_w, int64_t V, int K, float* ws, cudaStream_t st) {
   constexpr int KG = multi_group(NCH);
+  const MultiGroups g = multi_groups(K, KG);
   const int sms = sm_count();
-  const int ngroups = (K + KG - 1) / KG;
-  const int last_n = K - (ngroups - 1) * KG;
-  int last_w = 1;
-  while (last_w < last_n) last_w *= 2;
-  const int64_t total = ((int64_t)(ngroups - 1) * KG + last_w) * V;
+  const int64_t total = ((int64_t)(g.ngroups - 1) * KG + g.last_w) * V;
   const int64_t pblocks = ceil_div(total, 256);
   const int pgrid = (int)(pblocks < (int64_t)sms * 16 ? pblocks : (int64_t)sms * 16);
-  multi_weights_kernel<<<pgrid, 256, 0, st>>>(vocab_w, V, K, KG, ngroups, last_w, total, ws);
+  multi_weights_kernel<<<pgrid, 256, 0, st>>>(vocab_w, V, K, KG, g.ngroups, g.last_w, total, ws);
   MMB_LAUNCH_CHECK("sif_multi_weights");
+  return MMB_OK;
+}
 
-  // launch_embed's (and mmb_sif_embed_ragged's) variant rule and grid (sif_embed.cu)
-  const bool few_long = (L >= 256) && (N < (int64_t)sms * 16);
-  const bool wide = (uint64_t)V * (uint64_t)(d / 4) * 16u >= ((uint64_t)1 << 32);
-  const int64_t cap = (int64_t)sms * 8;
-  const int64_t blocks = few_long ? N : ceil_div(N, kEmbedWarps);
+// launch_embed's (and mmb_sif_embed_ragged's) variant rule (sif_embed.cu), taken on the batch's total N: a chunk
+// of a batch runs the variant of the whole batch, so its rows have the bits of the one-call result.
+struct MultiVariant {
+  bool few_long, wide;
+};
+static MultiVariant multi_variant(int64_t V, int d, int64_t N_total, int64_t L) {
+  MultiVariant v;
+  v.few_long = (L >= 256) && (N_total < (int64_t)sm_count() * 16);
+  v.wide = (uint64_t)V * (uint64_t)(d / 4) * 16u >= ((uint64_t)1 << 32);
+  return v;
+}
+
+// The gather of utterances [0, N) of ids for all K vectors (weights laid out in ws by multi_weights): output k of
+// utterance i is row k * kstride + i of emb.
+template <int NCH>
+static int multi_gather(const float* table, int64_t V, int d, const float* ws, int K, const int64_t* ids,
+                        const int64_t* offsets, int64_t N, int64_t L, int64_t pad_id, float* emb, int64_t kstride,
+                        int* status, MultiVariant var, cudaStream_t st) {
+  constexpr int KG = multi_group(NCH);
+  const MultiGroups gl = multi_groups(K, KG);
+  const int64_t cap = (int64_t)sm_count() * 8;
+  const int64_t blocks = var.few_long ? N : ceil_div(N, kEmbedWarps);
   const int grid = (int)(blocks < cap ? blocks : cap);
   char kname[96] = "";
-  for (int g = 0; g < ngroups; ++g) {
-    const int kn = g + 1 < ngroups ? KG : last_n;
-    const int kw = g + 1 < ngroups ? KG : last_w;
+  for (int g = 0; g < gl.ngroups; ++g) {
+    const int kn = g + 1 < gl.ngroups ? KG : gl.last_n;
+    const int kw = g + 1 < gl.ngroups ? KG : gl.last_w;
     const float* wg = ws + (size_t)g * KG * V;
-    float* out = emb + (size_t)g * KG * N * d;
+    float* out = emb + (size_t)g * KG * kstride * d;
     int rc = MMB_OK;
-#define MULTI_GROUP(W) \
-  rc = launch_multi_group<NCH, W>(table, V, d, wg, ids, offsets, N, L, pad_id, kn, out, status, few_long, wide, \
-                                  grid, st, kname, sizeof(kname))
+#define MULTI_GROUP(W)                                                                                       \
+  rc = launch_multi_group<NCH, W>(table, V, d, wg, ids, offsets, N, L, pad_id, kn, out, kstride, status,       \
+                                  var.few_long, var.wide, grid, st, kname, sizeof(kname))
     if (kw == 1) MULTI_GROUP(1);
     else if (kw == 2) MULTI_GROUP(2);
     else if constexpr (KG >= 4) {
@@ -431,6 +460,42 @@ static int launch_multi(const float* table, int64_t V, int d, const float* vocab
   }
   note_kernel(1, kname);
   return MMB_OK;
+}
+
+template <int NCH>
+static int launch_multi(const float* table, int64_t V, int d, const float* vocab_w, int K, const int64_t* ids,
+                        const int64_t* offsets, int64_t N, int64_t L, int64_t pad_id, float* emb, int* status,
+                        float* ws, cudaStream_t st) {
+  const int rc = multi_weights<NCH>(vocab_w, V, K, ws, st);
+  if (rc) return rc;
+  return multi_gather<NCH>(table, V, d, ws, K, ids, offsets, N, L, pad_id, emb, N, status,
+                           multi_variant(V, d, N, L), st);
+}
+
+// The chunked form for the host-buffer sweep (api.cu): sif_embed_multi_weights once per call, then one
+// sif_embed_multi_chunk per chunk of `rows` utterances, whose outputs go to rows [r0, r0 + rows) of a
+// (K, N_total, d) tensor (emb = its base + r0 * d).  Arguments are checked by the caller.
+int sif_embed_multi_weights(const float* vocab_w, int64_t V, int d, int K, void* ws, cudaStream_t st) {
+  switch ((d / 4 + 31) / 32) {
+    case 1: return multi_weights<1>(vocab_w, V, K, (float*)ws, st);
+    case 2: return multi_weights<2>(vocab_w, V, K, (float*)ws, st);
+    case 3: return multi_weights<3>(vocab_w, V, K, (float*)ws, st);
+    case 4: return multi_weights<4>(vocab_w, V, K, (float*)ws, st);
+    default: return multi_weights<8>(vocab_w, V, K, (float*)ws, st);
+  }
+}
+
+int sif_embed_multi_chunk(const float* table, int64_t V, int d, const void* ws, int K, const int64_t* x,
+                          int64_t rows, int64_t L, int64_t N_total, float* emb, int* status, cudaStream_t st) {
+  const MultiVariant var = multi_variant(V, d, N_total, L);
+  const float* w = (const float*)ws;
+  switch ((d / 4 + 31) / 32) {
+    case 1: return multi_gather<1>(table, V, d, w, K, x, nullptr, rows, L, 0, emb, N_total, status, var, st);
+    case 2: return multi_gather<2>(table, V, d, w, K, x, nullptr, rows, L, 0, emb, N_total, status, var, st);
+    case 3: return multi_gather<3>(table, V, d, w, K, x, nullptr, rows, L, 0, emb, N_total, status, var, st);
+    case 4: return multi_gather<4>(table, V, d, w, K, x, nullptr, rows, L, 0, emb, N_total, status, var, st);
+    default: return multi_gather<8>(table, V, d, w, K, x, nullptr, rows, L, 0, emb, N_total, status, var, st);
+  }
 }
 
 }  // namespace mmb

@@ -2,8 +2,9 @@
 ``get_sentence_embeddings``, the call ``simplesif.main`` makes per split (reference
 simplesif.py:296-311).  The embedding itself runs through ``mmb_sif_embedding_host`` /
 ``mmb_sif_embedding`` of libmmb_b200.so.  ``get_sentence_embeddings_sweep`` (no reference counterpart) does the
-same for K word-weight vectors and several numbers of removed components in one gather (``mmb_sif_embed_multi``;
-``mmb_sif_embed_multi_ragged`` for ``RaggedIds``).
+same for K word-weight vectors and several numbers of removed components in one gather
+(``mmb_sif_embedding_sweep_host`` for NumPy ids; ``mmb_sif_embed_multi`` / ``mmb_sif_embed_multi_ragged`` for ids
+on the device).
 """
 import ctypes as C
 import os
@@ -14,7 +15,7 @@ import torch
 import _native as nv
 from _native import lib
 from sif_functions import Params, seq2weight, SIF_embedding, start_block, sif_embedding_device  # noqa: F401
-from sif_functions import sif_embedding_sweep  # noqa: F401
+from sif_functions import sif_embedding_sweep, sweep_npcs  # noqa: F401
 from sif_functions import RaggedIds, sif_embedding_ragged, to_ragged  # noqa: F401
 
 # ---- word weights a / (a + p(w)) (host-side file handling; the arithmetic that matters runs in the kernels) ----
@@ -135,20 +136,26 @@ def get_sentence_embeddings(word_embeddings, weights, text, out=None):
     return out
 
 
-def get_sentence_embeddings_sweep(word_embeddings, weights, text, npcs=(1,)):
+def get_sentence_embeddings_sweep(word_embeddings, weights, text, npcs=(1,), out=None):
     """``get_sentence_embeddings`` for K word-weight vectors at once (e.g. ``get_word_weights(file, a)`` for
     several ``a``) and P numbers of removed principal components: ``out[k, j]`` is the SIF embedding with
     ``weights[k]`` and ``npcs[j]`` components removed (0 = the raw weighted average).  The table rows are
-    gathered once for all K vectors (``sif_functions.sif_embedding_sweep``).
+    gathered once for all K vectors.
 
     ``weights`` is a (K, V) array or a sequence of K vectors; a vector shorter than the table is padded with
-    zeros, and an id beyond it raises ``IndexError``, as in ``get_sentence_embeddings``.  NumPy in -> float64
-    (K, P, N, d) NumPy out; CUDA tensors or ``RaggedIds`` in -> float32 CUDA tensor out.  The ids are uploaded
-    once and the result downloaded once.  For ``RaggedIds`` the ids are those of the padded matrix they stand
-    for: the tokens, and ``pad_id`` when an utterance is shorter than ``L_pad``."""
+    zeros, and an id beyond it raises ``IndexError``, as in ``get_sentence_embeddings``.  CUDA tensors or
+    ``RaggedIds`` in -> float32 CUDA tensor out (``sif_functions.sif_embedding_sweep``).  NumPy in -> float64
+    (K, P, N, d) NumPy out through ``mmb_sif_embedding_sweep_host``: the ids stream to the device in chunks, only
+    the K embeddings stay resident there, and each projected chunk is written straight into the host result,
+    bit for bit the device sweep's values.  ``out`` may be a preallocated C-contiguous (K, P, N, d) float64 or
+    float32 host array (e.g. ``_native.PinnedArray(...).array``, for full PCIe rate) to receive the result; it is
+    returned.  For ``RaggedIds`` the ids are those of the padded matrix they stand for: the tokens, and
+    ``pad_id`` when an utterance is shorter than ``L_pad``."""
     dev = nv.require_cuda()
     ragged = isinstance(text, RaggedIds)
     as_np = not (ragged or (isinstance(text, torch.Tensor) and text.is_cuda))
+    if out is not None and not as_np:
+        raise ValueError('out= takes host ids; with CUDA ids or RaggedIds the result is a CUDA tensor')
     table_t = nv.to_device(word_embeddings, torch.float32, dev)
     V, d = table_t.shape
     if isinstance(weights, torch.Tensor):
@@ -161,7 +168,6 @@ def get_sentence_embeddings_sweep(word_embeddings, weights, text, npcs=(1,)):
         ids = np.ascontiguousarray(np.asarray(text), dtype=np.int64)
         if ids.ndim != 2:
             raise ValueError('text must be (n_samples, seq_len)')
-        ids_t = nv.to_device(ids, torch.int64, dev)
         id_max = int(ids.max()) if ids.size else None
     elif ragged:
         ids_t = text
@@ -181,5 +187,21 @@ def get_sentence_embeddings_sweep(word_embeddings, weights, text, npcs=(1,)):
                 raise IndexError('index %d is out of bounds for axis 0 with size %d' % (id_max, w_t.numel()))
             w_t = torch.cat([w_t, w_t.new_zeros(V - w_t.numel())])
         rows.append(w_t[:V])
-    out = sif_embedding_sweep(table_t, torch.stack(rows).contiguous(), ids_t, npcs=npcs)
-    return out.double().cpu().numpy() if as_np else out
+    W_t = torch.stack(rows).contiguous()
+    if not as_np:
+        return sif_embedding_sweep(table_t, W_t, ids_t, npcs=npcs)
+    npcs = sweep_npcs(npcs)
+    K, P = W_t.shape[0], len(npcs)
+    n, L = ids.shape
+    if out is None:
+        out = np.empty((K, P, n, d), dtype=np.float64)
+    if (tuple(out.shape) != (K, P, n, d) or not out.flags['C_CONTIGUOUS']
+            or out.dtype not in (np.float64, np.float32)):
+        raise ValueError('out must be a C-contiguous (%d, %d, %d, %d) float64 or float32 array' % (K, P, n, d))
+    omegas = [np.ascontiguousarray(start_block(d if n >= d else n, p)) if p else None for p in npcs]
+    omega_arr = (C.c_void_p * P)(*[o.ctypes.data if o is not None else None for o in omegas])
+    torch.cuda.current_stream().synchronize()      # table / weights uploads are done
+    nv.check(lib.mmb_sif_embedding_sweep_host(nv.ptr(table_t), V, d, nv.ptr(W_t), K, nv.np_ptr(ids), n, L, P,
+                                              (C.c_int * P)(*npcs), omega_arr, nv.np_ptr(out),
+                                              int(out.dtype == np.float64), nv.GRAM_AUTO, 0))
+    return out
