@@ -107,6 +107,16 @@ MMB_API int mmb_sif_embed_ws(const float* table, int64_t V, int d, const float* 
                              int64_t N, int64_t L, float* emb, int* status, void* ws, size_t ws_bytes,
                              mmb_stream_t stream);
 
+/* SIF embedding with GIVEN components (TruncatedSVD.transform's counterpart of compute_pc's fit: remove_pc,
+ * sif_functions.py:69-81, with pc fitted elsewhere): mmb_sif_embed_ws (ws as there; NULL -> the general kernel)
+ * followed by mmb_remove_pc(pc, npc), in one pass, bit for bit -- the warp that finishes a row subtracts its
+ * projection before the row is stored.  pc: npc x d float32 on the device, 16-byte aligned; npc in [0, 32]; npc = 0
+ * is the plain embed.  out (N, d) float32, 16-byte aligned.  mmb_last_kernel(0) names the embed kernel, followed
+ * by " +pc f32" when npc > 0 (with npc = 0 the plain kernel runs, under its plain name).                        */
+MMB_API int mmb_sif_transform(const float* table, int64_t V, int d, const float* vocab_w, const int64_t* x,
+                              int64_t N, int64_t L, const float* pc, int npc, float* out, int* status,
+                              void* ws, size_t ws_bytes, mmb_stream_t stream);
+
 /* SIF sweep: seq2weight + get_weighted_average (sif_functions.py:8-15, 28-56) for K vocabulary-weight vectors
  * over one gather of the table rows.  vocab_w is (K, V) row-major; emb is (K, N, d), so every emb[k] is a dense
  * (N, d) matrix that mmb_gram / mmb_remove_pc take as it is.  emb[k] is bit-identical to mmb_sif_embed with
@@ -224,6 +234,30 @@ MMB_API int mmb_sif_embedding_sweep_host(const float* table_dev, int64_t V, int 
                                          const int64_t* x_host, int64_t N, int64_t L, int P, const int* npcs,
                                          const double* const* Omega_host, void* out_host, int out_f64,
                                          int gram_mode, int64_t chunk_rows);
+
+/* mmb_sif_transform from host buffers: ids H2D || fused kernel || D2H, chunk by chunk (chunk_rows <= 0: 2^18),
+ * with two id buffers and two staging buffers of the output type on the device and nothing of size N -- no row
+ * depends on the whole batch, so chunk c + 1's ids cross H2D while chunk c is embedded and chunk c - 1 crosses D2H.
+ * pc_host: npc x d float32 on the host, npc in [0, 32].  out_host (N, d): float64 when out_f64 != 0 (the float32
+ * result widened once), else float32.  The kernel variant (pre-scaled, CTA per utterance, wide table) is decided
+ * on the WHOLE N, as mmb_sif_embedding_sweep_host does, so the result equals mmb_sif_transform on all N rows (with
+ * ws of mmb_sif_embed_workspace_bytes) at every chunk_rows.  Synchronous; a bad id is MMB_E_INDEX.  The kernel
+ * name (mmb_last_kernel(0)) ends in " +pc f32" (npc > 0), " +pc f64" (float64 out, any npc) or nothing.      */
+MMB_API int mmb_sif_transform_host(const float* table_dev, int64_t V, int d, const float* vocab_w_dev,
+                                   const int64_t* x_host, int64_t N, int64_t L, const float* pc_host, int npc,
+                                   void* out_host, int out_f64, int64_t chunk_rows);
+
+/* Components only (compute_pc, sif_functions.py:58-67, on the SIF embedding): ids H2D || embed of a chunk -> its
+ * Gram added to the running sum in chunk order -> one solve.  Device memory is two id chunks + one embedding chunk
+ * + the Gram / solve scratch (+ the pre-scaled table for large batches), whatever N is.  N < d runs as one chunk
+ * (the start block X^T Omega needs every row).  Omega_host as for mmb_sif_embedding_host; pc_host: npc x d
+ * float32, npc in [1, 22]; d <= 512; N >= 1.  The kernel variant is decided on the whole N, so pc_host equals
+ * mmb_sif_embedding_host's at the same chunk_rows wherever each chunk of that call runs the whole batch's variant:
+ * it decides the CTA-per-utterance rule (L >= 256, N < 16 SMs) per chunk, so a short last chunk of long
+ * utterances may run another kernel there.  With chunk_rows >= N it equals mmb_sif_embedding's pc.  Synchronous. */
+MMB_API int mmb_sif_fit_host(const float* table_dev, int64_t V, int d, const float* vocab_w_dev,
+                             const int64_t* x_host, int64_t N, int64_t L, int npc, const double* Omega_host,
+                             float* pc_host, int gram_mode, int64_t chunk_rows);
 
 /* The *_host entry points take their staging buffers from a private stream-ordered pool per device
  * that keeps freed blocks for the next call; this returns all but `keep_bytes` of them to the driver. */

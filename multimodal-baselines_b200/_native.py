@@ -42,6 +42,7 @@ SIGNATURES = {
     'mmb_sif_embed': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _p, _p, _p]),
     'mmb_sif_embed_workspace_bytes': (_sz, [_i64, _i, _i64, _i64]),
     'mmb_sif_embed_ws': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _p, _p, _p, _sz, _p]),
+    'mmb_sif_transform': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _p, _i, _p, _p, _p, _sz, _p]),
     'mmb_sif_embed_multi_workspace_bytes': (_sz, [_i64, _i]),
     'mmb_sif_embed_multi': (_i, [_p, _i64, _i, _p, _i, _p, _i64, _i64, _p, _p, _p, _sz, _p]),
     'mmb_sif_embed_multi_ragged': (_i, [_p, _i64, _i, _p, _i, _p, _p, _i64, _i64, _i64, _p, _p, _p, _sz, _p]),
@@ -63,6 +64,8 @@ SIGNATURES = {
     'mmb_sif_embedding_host_peer': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _i, _p, _p, _i, _p, _i, _i64, _i64, _i, _i,
                                          _p, C.c_uint64]),
     'mmb_sif_embedding_sweep_host': (_i, [_p, _i64, _i, _p, _i, _p, _i64, _i64, _i, _p, _p, _p, _i, _i, _i64]),
+    'mmb_sif_transform_host': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _p, _i, _p, _i, _i64]),
+    'mmb_sif_fit_host': (_i, [_p, _i64, _i, _p, _p, _i64, _i64, _i, _p, _p, _i, _i64]),
     'mmb_host_pipeline_trim': (_i, [_sz]),
     'mmb_comm_abort': (_i, [_i, _i, _p, C.c_uint64, _p]),
     'mmb_comm_bytes': (_sz, []),

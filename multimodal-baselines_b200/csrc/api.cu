@@ -79,7 +79,7 @@ __global__ void f32_to_f64_kernel(const float* __restrict__ in, double* __restri
 
 using namespace mmb;
 
-extern "C" int mmb_version(void) { return 104; }
+extern "C" int mmb_version(void) { return 105; }
 
 extern "C" const char* mmb_last_error(void) { return g_err; }
 
@@ -148,6 +148,9 @@ namespace mmb {   // implemented in sif_embed.cu
 int sif_prescale(const float* table, int64_t V, int d, const float* vocab_w, void* ws, cudaStream_t st);
 int sif_embed_prescaled(const float* table, int64_t V, int d, const float* vocab_w, const void* ws, const int64_t* x,
                         int64_t N, int64_t L, float* emb, int* status, cudaStream_t st);
+int sif_transform_chunk(const float* table, int64_t V, int d, const float* vocab_w, const void* scaled,
+                        const int64_t* x, int64_t N, int64_t L, int64_t N_total, const float* pc, int npc, void* out,
+                        bool f64, int* status, cudaStream_t st);
 // implemented in sif_embed_multi.cu / remove_pc.cu (used by mmb_sif_embedding_sweep_host)
 int sif_embed_multi_weights(const float* vocab_w, int64_t V, int d, int K, void* ws, cudaStream_t st);
 int sif_embed_multi_chunk(const float* table, int64_t V, int d, const void* ws, int K, const int64_t* x,
@@ -382,6 +385,32 @@ int finish_host_call(Streams& S, const DevBuf& status, int64_t V) {
   }
   return MMB_OK;
 }
+
+// The Gram of chunk c (rows of emb_chunk) added to the running sum G, in chunk order (deterministic): G is the
+// first chunk's Gram, then G += each next one.  gchunk: d x d scratch.
+int add_chunk_gram(const float* emb_chunk, int64_t rows, int d, int64_t c, float* G, float* gchunk, void* gram_ws,
+                   size_t gram_ws_bytes, int gram_mode, cudaStream_t st) {
+  int rc = mmb_gram(emb_chunk, rows, d, gchunk, gram_ws, gram_ws_bytes, gram_mode, st);
+  if (rc) return rc;
+  accumulate_kernel<<<(d * d + 255) / 256, 256, 0, st>>>(G, gchunk, d * d, c == 0);
+  MMB_LAUNCH_CHECK("accumulate");
+  return MMB_OK;
+}
+
+// The components from the Gram G of n_global rows, in the workspace layout of sif_ws_layout: the start block (X^T
+// Omega when n_global < d, from the N rows of emb, which are then every row) and the solve into pc_dev.
+int components_from_gram(const float* G, const float* emb, int64_t N, int64_t n_global, int d, int npc,
+                         const double* omega_dev, char* ws_base, const SifWs& Lw, float* pc_dev, cudaStream_t st) {
+  const int k = npc + 10;
+  const double* S0 = omega_dev;
+  const int transposed = n_global < d;
+  if (transposed) {
+    int rc = mmb_start_block_xt(emb, N, d, omega_dev, k, (double*)(ws_base + Lw.s0), st);
+    if (rc) return rc;
+    S0 = (const double*)(ws_base + Lw.s0);
+  }
+  return mmb_pc_from_gram(G, d, S0, k, npc, transposed, 7, pc_dev, ws_base + Lw.pc, Lw.s0 - Lw.pc, st);
+}
 }  // namespace
 
 static int sif_embedding_host_impl(const float* table_dev, int64_t V, int d, const float* vocab_w_dev,
@@ -449,17 +478,12 @@ static int sif_embedding_host_impl(const float* table_dev, int64_t V, int d, con
       [&](int64_t c, int64_t r0, int64_t rows) {
         if (!chunked_gram) return (int)MMB_OK;
         // The compute stream idles while the next chunk's ids cross PCIe: take the chunk's Gram now
-        // and add it to the running sum (chunk order -> deterministic), so that only the component
-        // solve separates the last H2D from the first D2H.
+        // and add it to the running sum, so that only the component solve separates the last H2D
+        // from the first D2H.
         SifWs Lw = sif_ws_layout(N, d, npc);
         char* base = (char*)ws.p;
-        float* G = (float*)(base + Lw.G);
-        int rc2 = mmb_gram((const float*)emb.p + r0 * d, rows, d, (float*)gchunk.p, base + Lw.gram,
-                           Lw.pc - Lw.gram, gram_mode, S.comp);
-        if (rc2) return rc2;
-        accumulate_kernel<<<(d * d + 255) / 256, 256, 0, S.comp>>>(G, (const float*)gchunk.p, d * d, c == 0);
-        MMB_LAUNCH_CHECK("accumulate");
-        return (int)MMB_OK;
+        return add_chunk_gram((const float*)emb.p + r0 * d, rows, d, c, (float*)(base + Lw.G), (float*)gchunk.p,
+                              base + Lw.gram, Lw.pc - Lw.gram, gram_mode, S.comp);
       });
   if (rc) return rc;
   // phase 2: components from the Gram of the whole block (summed per chunk above, or taken here)
@@ -482,15 +506,8 @@ static int sif_embedding_host_impl(const float* table_dev, int64_t V, int d, con
       if (rc) return rc;
       abort_guard.armed = false;   // this rank has taken part in the exchange
     }
-    const double* S0 = (const double*)omega.p;
-    const int transposed = n_global < d;
-    if (transposed) {
-      rc = mmb_start_block_xt((const float*)emb.p, N, d, (const double*)omega.p, k,
-                              (double*)(base + Lw.s0), S.comp);
-      if (rc) return rc;
-      S0 = (const double*)(base + Lw.s0);
-    }
-    rc = mmb_pc_from_gram(G, d, S0, k, npc, transposed, 7, pc_dev, base + Lw.pc, Lw.s0 - Lw.pc, S.comp);
+    rc = components_from_gram(G, (const float*)emb.p, N, n_global, d, npc, (const double*)omega.p, base, Lw, pc_dev,
+                              S.comp);
     if (rc) return rc;
   }
   // phase 3: projection (stream `comp`) overlapped with the D2H of finished chunks (`out`)
@@ -703,5 +720,139 @@ extern "C" int mmb_sif_embedding_sweep_host(const float* table_dev, int64_t V, i
     }
   }
   if ((rc = copy_out(q - 1, pend_k, pend_r0, pend_rows))) return rc;
+  return finish_host_call(S, status, V);
+}
+
+// ---- SIF fit / transform with host buffers -----------------------------------------------------------------
+extern "C" int mmb_sif_transform_host(const float* table_dev, int64_t V, int d, const float* vocab_w_dev,
+                                      const int64_t* x_host, int64_t N, int64_t L, const float* pc_host, int npc,
+                                      void* out_host, int out_f64, int64_t chunk_rows) {
+  MMB_REQUIRE(table_dev && vocab_w_dev && (x_host || N == 0) && (out_host || N == 0), "null pointer");
+  MMB_REQUIRE(N >= 0 && L >= 0 && d > 0 && d % 4 == 0 && d <= 1024, "bad size (d must be a multiple of 4, <= 1024)");
+  MMB_REQUIRE(npc >= 0 && npc <= 32, "npc must be in [0, 32]");
+  MMB_REQUIRE(pc_host || npc == 0, "null pointer");
+  if (N == 0) return MMB_OK;
+  chunk_rows = host_chunk_rows(chunk_rows, N);
+  const size_t esz = out_f64 ? sizeof(double) : sizeof(float);
+
+  Streams S;
+  int rc = S.init();
+  if (rc) return rc;
+  DevBuf ids[2], stage[2], status, pcv, scaled;
+  SyncGuard sync_guard{S};
+  const size_t ids_chunk = (size_t)chunk_rows * L * sizeof(int64_t);
+  for (int b = 0; b < 2; ++b) {
+    if ((rc = ids[b].alloc(ids_chunk, S.comp))) return rc;
+    if ((rc = stage[b].alloc((size_t)chunk_rows * d * esz, S.comp))) return rc;
+  }
+  if ((rc = status.alloc(sizeof(int), S.comp))) return rc;
+  MMB_CUDA(cudaMemsetAsync(status.p, 0, sizeof(int), S.comp));
+  if (npc > 0) {
+    if ((rc = pcv.alloc((size_t)npc * d * sizeof(float), S.comp))) return rc;
+    MMB_CUDA(cudaMemcpyAsync(pcv.p, pc_host, (size_t)npc * d * sizeof(float), cudaMemcpyHostToDevice, S.comp));
+  }
+  // the kernel variant of the WHOLE batch: the pre-scaled table once, and N as the CTA-per-utterance rule's N
+  const size_t scaled_bytes = mmb_sif_embed_workspace_bytes(V, d, N, L);
+  if (scaled_bytes) {
+    if ((rc = scaled.alloc(scaled_bytes, S.comp))) return rc;
+    if ((rc = sif_prescale(table_dev, V, d, vocab_w_dev, scaled.p, S.comp))) return rc;
+  }
+  if ((rc = copy_streams_after_setup(S))) return rc;
+
+  // ids H2D (stream `in`) || the fused embed + projection of a chunk into a staging buffer (`comp`) || the D2H of the
+  // previous chunk (`out`): nothing depends on the whole batch, so the three run at once
+  cudaEvent_t out_ready[2], out_free[2];
+  for (int b = 0; b < 2; ++b) {
+    if ((rc = S.event(&out_ready[b]))) return rc;
+    if ((rc = S.event(&out_free[b]))) return rc;
+  }
+  auto copy_out = [&](int64_t c) {
+    const int b = (int)(c & 1);
+    const int64_t r0 = c * chunk_rows;
+    const int64_t rows = (N - r0) < chunk_rows ? (N - r0) : chunk_rows;
+    MMB_CUDA(cudaStreamWaitEvent(S.out, out_ready[b], 0));
+    MMB_CUDA(cudaMemcpyAsync((char*)out_host + (size_t)r0 * d * esz, stage[b].p, (size_t)rows * d * esz,
+                             cudaMemcpyDeviceToHost, S.out));
+    MMB_CUDA(cudaEventRecord(out_free[b], S.out));
+    return (int)MMB_OK;
+  };
+  rc = stream_ids_in(
+      S, ids, x_host, N, L, chunk_rows,
+      [&](const int64_t* ids_dev, int64_t r0, int64_t rows) {
+        const int64_t c = r0 / chunk_rows;
+        const int b = (int)(c & 1);
+        if (c >= 2) MMB_CUDA(cudaStreamWaitEvent(S.comp, out_free[b], 0));
+        return sif_transform_chunk(table_dev, V, d, vocab_w_dev, scaled_bytes ? scaled.p : nullptr, ids_dev, rows, L,
+                                   N, (const float*)pcv.p, npc, stage[b].p, out_f64 != 0, (int*)status.p, S.comp);
+      },
+      [&](int64_t c, int64_t, int64_t) {
+        MMB_CUDA(cudaEventRecord(out_ready[c & 1], S.comp));
+        // the D2H of the previous chunk, enqueued after this chunk's kernel, so that a copy into pageable memory
+        // (which returns only when done) still overlaps it
+        return c > 0 ? copy_out(c - 1) : (int)MMB_OK;
+      });
+  if (rc) return rc;
+  if ((rc = copy_out(ceil_div(N, chunk_rows) - 1))) return rc;
+  return finish_host_call(S, status, V);
+}
+
+extern "C" int mmb_sif_fit_host(const float* table_dev, int64_t V, int d, const float* vocab_w_dev,
+                                const int64_t* x_host, int64_t N, int64_t L, int npc, const double* Omega_host,
+                                float* pc_host, int gram_mode, int64_t chunk_rows) {
+  MMB_REQUIRE(table_dev && vocab_w_dev && x_host && Omega_host && pc_host, "null pointer");
+  MMB_REQUIRE(N >= 1 && L >= 0 && d > 0 && d % 4 == 0 && d <= 512,
+              "bad size (N >= 1; d must be a multiple of 4, <= 512)");
+  MMB_REQUIRE(npc >= 1 && npc + 10 <= 32, "npc must be in [1, 22]");
+  // N < d: the start block X^T Omega needs every row at once
+  chunk_rows = N < d ? N : host_chunk_rows(chunk_rows, N);
+  const int64_t nchunks = ceil_div(N, chunk_rows);
+  const int k = npc + 10;
+  const int64_t orows = N >= d ? d : N;
+
+  Streams S;
+  int rc = S.init();
+  if (rc) return rc;
+  DevBuf ids[2], emb, ws, omega, status, pcv, gchunk, scaled;
+  SyncGuard sync_guard{S};
+  const size_t ids_chunk = (size_t)chunk_rows * L * sizeof(int64_t);
+  if ((rc = ids[0].alloc(ids_chunk, S.comp))) return rc;
+  if ((rc = ids[1].alloc(ids_chunk, S.comp))) return rc;
+  if ((rc = emb.alloc((size_t)chunk_rows * d * sizeof(float), S.comp))) return rc;
+  if ((rc = status.alloc(sizeof(int), S.comp))) return rc;
+  MMB_CUDA(cudaMemsetAsync(status.p, 0, sizeof(int), S.comp));
+  const SifWs Lw = sif_ws_layout(N, d, npc);
+  if ((rc = ws.alloc(Lw.total, S.comp))) return rc;
+  if ((rc = omega.alloc((size_t)orows * k * sizeof(double), S.comp))) return rc;
+  if ((rc = pcv.alloc((size_t)npc * d * sizeof(float), S.comp))) return rc;
+  if (nchunks > 1 && (rc = gchunk.alloc((size_t)d * d * sizeof(float), S.comp))) return rc;
+  MMB_CUDA(cudaMemcpyAsync(omega.p, Omega_host, (size_t)orows * k * sizeof(double), cudaMemcpyHostToDevice, S.comp));
+  const size_t scaled_bytes = mmb_sif_embed_workspace_bytes(V, d, N, L);
+  if (scaled_bytes) {
+    if ((rc = scaled.alloc(scaled_bytes, S.comp))) return rc;
+    if ((rc = sif_prescale(table_dev, V, d, vocab_w_dev, scaled.p, S.comp))) return rc;
+  }
+  if ((rc = copy_streams_after_setup(S))) return rc;
+
+  // ids H2D (stream `in`) || embed of a chunk, then its Gram added to the running sum (`comp`); one embedding chunk
+  // suffices because the Gram of chunk c runs on `comp` before the embed of chunk c + 1
+  char* base = (char*)ws.p;
+  float* G = (float*)(base + Lw.G);
+  rc = stream_ids_in(
+      S, ids, x_host, N, L, chunk_rows,
+      [&](const int64_t* ids_dev, int64_t, int64_t rows) {
+        return sif_transform_chunk(table_dev, V, d, vocab_w_dev, scaled_bytes ? scaled.p : nullptr, ids_dev, rows, L,
+                                   N, nullptr, 0, emb.p, false, (int*)status.p, S.comp);
+      },
+      [&](int64_t c, int64_t, int64_t rows) {
+        if (nchunks == 1)
+          return mmb_gram((const float*)emb.p, rows, d, G, base + Lw.gram, Lw.pc - Lw.gram, gram_mode, S.comp);
+        return add_chunk_gram((const float*)emb.p, rows, d, c, G, (float*)gchunk.p, base + Lw.gram, Lw.pc - Lw.gram,
+                              gram_mode, S.comp);
+      });
+  if (rc) return rc;
+  rc = components_from_gram(G, (const float*)emb.p, N, N, d, npc, (const double*)omega.p, base, Lw, (float*)pcv.p,
+                            S.comp);
+  if (rc) return rc;
+  MMB_CUDA(cudaMemcpyAsync(pc_host, pcv.p, (size_t)npc * d * sizeof(float), cudaMemcpyDeviceToHost, S.comp));
   return finish_host_call(S, status, V);
 }

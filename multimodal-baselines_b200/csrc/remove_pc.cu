@@ -3,7 +3,7 @@
 //   npc  > 1: XX = X - (X pc^T) pc            (line 80; all projections taken from X itself)
 // HBM-bound streaming pass: one warp per row, the row lives in registers as float4 (read
 // once, written once = 2*d*4 bytes per utterance), the components sit in shared memory.
-#include "common.cuh"
+#include "pc_rows.cuh"
 
 namespace mmb {
 
@@ -19,61 +19,6 @@ __device__ __forceinline__ void load_row(const float4* X4, int64_t i, int d4, in
     const int k = lane + 32 * c;
     x[c] = k < d4 ? ld_stream(X4 + (size_t)i * d4 + k) : make_float4(0.f, 0.f, 0.f, 0.f);
     r[c] = x[c];
-  }
-}
-
-// r -= sum_p dot(x, pc[p]) pc[p] with every dot taken from x (pc: npc x d4 in shared memory); r enters as x.
-template <int NCH>
-__device__ __forceinline__ void subtract_pcs(const float4 (&x)[NCH], float4 (&r)[NCH], const float4* spc, int npc,
-                                             int d4, int lane) {
-  for (int p = 0; p < npc; ++p) {
-    float dot = 0.f;
-#pragma unroll
-    for (int c = 0; c < NCH; ++c) {
-      const int k = lane + 32 * c;
-      if (k < d4) {
-        const float4 v = spc[p * d4 + k];
-        dot = fmaf(x[c].x, v.x, dot);
-        dot = fmaf(x[c].y, v.y, dot);
-        dot = fmaf(x[c].z, v.z, dot);
-        dot = fmaf(x[c].w, v.w, dot);
-      }
-    }
-    dot = warp_sum(dot);
-#pragma unroll
-    for (int c = 0; c < NCH; ++c) {
-      const int k = lane + 32 * c;
-      if (k < d4) {
-        const float4 v = spc[p * d4 + k];
-        r[c].x = fmaf(-dot, v.x, r[c].x);
-        r[c].y = fmaf(-dot, v.y, r[c].y);
-        r[c].z = fmaf(-dot, v.z, r[c].z);
-        r[c].w = fmaf(-dot, v.w, r[c].w);
-      }
-    }
-  }
-}
-
-template <int NCH>
-__device__ __forceinline__ void store_row(float4* out4, int64_t i, int d4, int lane, const float4 (&r)[NCH]) {
-#pragma unroll
-  for (int c = 0; c < NCH; ++c) {
-    const int k = lane + 32 * c;
-    if (k < d4) st_stream(out4 + (size_t)i * d4 + k, r[c]);
-  }
-}
-
-// The same row widened to float64 (one cvt per element): float4 k of the row becomes double2 2k and 2k + 1.
-template <int NCH>
-__device__ __forceinline__ void store_row(double2* out2, int64_t i, int d4, int lane, const float4 (&r)[NCH]) {
-#pragma unroll
-  for (int c = 0; c < NCH; ++c) {
-    const int k = lane + 32 * c;
-    if (k < d4) {
-      double2* p = out2 + ((size_t)i * d4 + k) * 2;
-      __stcs(p, make_double2((double)r[c].x, (double)r[c].y));
-      __stcs(p + 1, make_double2((double)r[c].z, (double)r[c].w));
-    }
   }
 }
 
@@ -163,20 +108,21 @@ extern "C" int mmb_remove_pc(const float* X, int64_t N, int d, const float* pc, 
   const int grid = (int)(blocks < cap ? blocks : cap);
   const size_t smem = (size_t)npc * d4 * sizeof(float4);
   cudaStream_t st = as_stream(stream);
-#define RM_LAUNCH(NCH)                                                                          \
-  remove_pc_kernel<NCH><<<grid, kRmWarps * 32, smem, st>>>((const float4*)X, N, d4, (const float4*)pc, \
-                                                          npc, (float4*)out)
+  // more than 48 KB of components (npc * d > 12288, e.g. npc = 32 at d >= 388) needs the opt-in at every NCH
+#define RM_LAUNCH(NCH)                                                                                       \
+  do {                                                                                                       \
+    if (smem > 48 * 1024)                                                                                    \
+      MMB_CUDA(cudaFuncSetAttribute(remove_pc_kernel<NCH>, cudaFuncAttributeMaxDynamicSharedMemorySize,      \
+                                    (int)smem));                                                             \
+    remove_pc_kernel<NCH><<<grid, kRmWarps * 32, smem, st>>>((const float4*)X, N, d4, (const float4*)pc,     \
+                                                            npc, (float4*)out);                              \
+  } while (0)
   switch (nch) {
     case 1: RM_LAUNCH(1); break;
     case 2: RM_LAUNCH(2); break;
     case 3: RM_LAUNCH(3); break;
     case 4: RM_LAUNCH(4); break;
-    default: {
-      if (smem > 48 * 1024)
-        MMB_CUDA(cudaFuncSetAttribute(remove_pc_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)smem));
-      RM_LAUNCH(8);
-    }
+    default: RM_LAUNCH(8);
   }
 #undef RM_LAUNCH
   MMB_LAUNCH_CHECK("remove_pc");

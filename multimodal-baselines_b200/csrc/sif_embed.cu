@@ -18,9 +18,62 @@
 //   * ids outside [-V, V) are NumPy's IndexError: the kernel skips them and raises
 //     MMB_STATUS_BAD_INDEX, which the Python shim turns into IndexError;
 //   * an all-zero-weight row divides by zero -> NaN row.
+#include "pc_rows.cuh"
 #include "sif_rows.cuh"
 
 namespace mmb {
+
+// Epilogue of the embed kernels: the finished row as it is (kPlain), or minus its projection on npc given
+// components (mmb_sif_transform), stored as float32 (kProjF32) or widened to float64 (kProjF64; npc may be 0).
+// The components are read from global memory through the read-only path: npc * d * 4 bytes (1.2 KB at npc = 1,
+// d = 300) stay in L1 next to the gathered rows, and the gather's L1 share -- a capacity number -- loses no shared
+// memory carve-out to them.
+enum class Epi { kPlain, kProjF32, kProjF64 };
+template <Epi E> struct EpiOut { typedef float4 type; };
+template <> struct EpiOut<Epi::kProjF64> { typedef double2 type; };
+
+// CTAs per SM (__launch_bounds__ minimum) of the projecting instantiations: the plain kernel's 4 (64 registers) where
+// the epilogue fits that budget without spilling, else the most CTAs per SM at which ptxas -v reports no spill (3:
+// 80 registers, 2: 128; DESIGN section 4).  The d > 512 warp kernel keeps its 2.  The CTA kernel's plain form sets no
+// minimum and ptxas holds it near 64 registers; its projecting forms ask for 2 CTAs per SM (128 registers), or 1.
+constexpr int proj_minb(Epi E, int f32, int f64) { return E == Epi::kPlain ? 4 : E == Epi::kProjF32 ? f32 : f64; }
+constexpr int prefetch_minb(Epi E, int nch) {
+  return proj_minb(E, nch <= 2 ? 4 : 2, nch <= 1 ? 4 : nch == 2 ? 3 : 2);
+}
+constexpr int prescaled_minb(Epi E, int nch) { return proj_minb(E, nch <= 3 ? 4 : 3, 4); }
+constexpr int wide_minb(Epi E, int nch) {
+  return proj_minb(E, nch <= 2 ? 4 : nch == 3 ? 3 : 2, nch <= 1 ? 4 : nch <= 3 ? 3 : 2);
+}
+constexpr int cta_minb(Epi E, int nch) { return E == Epi::kPlain ? 0 : (nch <= 2 ? 2 : 1); }
+
+// Row i of the output.  Projected: x = acc / cnt exactly as store_row forms it (absent chunks 0, as remove_pc's
+// load_row reads them), then remove_pc's own subtract_pcs and store, so the row is bit for bit the embed followed
+// by mmb_remove_pc.
+template <Epi E, int NCH>
+__device__ __forceinline__ void finish_row(typename EpiOut<E>::type* __restrict__ out, int64_t i,
+                                           const RowAcc<NCH>& acc, int cnt, int lane, int d4,
+                                           const float4* __restrict__ pc4, int npc) {
+  if constexpr (E == Epi::kPlain) {
+    store_row<NCH>(out + (size_t)i * d4, acc, cnt, lane, d4);
+  } else {
+    const float div = (float)cnt;
+    float4 x[NCH];
+#pragma unroll
+    for (int c = 0; c < NCH; ++c) {
+      x[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (lane + 32 * c < d4) {
+        unpack2(acc.a[c][0], x[c].x, x[c].y);
+        unpack2(acc.a[c][1], x[c].z, x[c].w);
+        x[c].x = __fdiv_rn(x[c].x, div);
+        x[c].y = __fdiv_rn(x[c].y, div);
+        x[c].z = __fdiv_rn(x[c].z, div);
+        x[c].w = __fdiv_rn(x[c].w, div);
+      }
+    }
+    subtract_pcs_inplace<NCH>(x, pc4, npc, d4, lane);
+    store_row<NCH>(out, i, d4, lane, x);
+  }
+}
 
 // A1: the stand-alone lookup (the reference materialises this matrix; the fused kernel
 // below does not).
@@ -150,12 +203,13 @@ __device__ __forceinline__ int accumulate_chunk(RowAcc<NCH>& acc, const char* __
 // Warp-per-utterance variant (large N).
 // The same kernel with the ids of the NEXT chunk (same utterance, or the warp's next utterance) requested
 // before the current chunk's rows are walked.
-template <int NCH, int UNROLL, int MINB>
+template <int NCH, int UNROLL, int MINB, Epi E = Epi::kPlain>
 __global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
     sif_embed_warp_prefetch_kernel(const float4* __restrict__ table4, int V, int d4, const float* __restrict__ wsrc,
                                    const int64_t* __restrict__ ids, int64_t N, int64_t L,
-                                   float4* __restrict__ emb4, int* __restrict__ status,
-                                   const int* __restrict__ only_if_flag = nullptr) {
+                                   typename EpiOut<E>::type* __restrict__ emb4, int* __restrict__ status,
+                                   const int* __restrict__ only_if_flag = nullptr,
+                                   const float4* __restrict__ pc4 = nullptr, int npc = 0) {
   // launched behind sif_embed_prescaled_kernel: work only if that one stood down (flag bit 0 set)
   if (only_if_flag && !(__ldg(only_if_flag) & 1)) return;
   const int lane = threadIdx.x & 31;
@@ -181,17 +235,18 @@ __global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
       cnt += accumulate_chunk<NCH, false, UNROLL, false, true>(acc, lane_base, V, row_bytes, tail, wsrc, row_ids,
                                                                nullptr, base, L, lane, bad, id);
     }
-    store_row<NCH>(emb4 + (size_t)i * d4, acc, cnt, lane, d4);
+    finish_row<E, NCH>(emb4, i, acc, cnt, lane, d4, pc4, npc);
   }
   if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, MMB_STATUS_BAD_INDEX);
 }
 
-template <int NCH, bool EXPLICIT_W, int UNROLL, int MINB, bool WIDE>
+template <int NCH, bool EXPLICIT_W, int UNROLL, int MINB, bool WIDE, Epi E = Epi::kPlain>
 __global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
     sif_embed_warp_kernel(const float4* __restrict__ table4, int V, int d4,
                           const float* __restrict__ wsrc, const int64_t* __restrict__ ids,
-                          int64_t N, int64_t L, float4* __restrict__ emb4,
-                          int* __restrict__ status) {
+                          int64_t N, int64_t L, typename EpiOut<E>::type* __restrict__ emb4,
+                          int* __restrict__ status, const float4* __restrict__ pc4 = nullptr, int npc = 0) {
+  static_assert(E == Epi::kPlain || !EXPLICIT_W, "the projecting epilogue serves the fused-lookup embed only");
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = (int64_t)blockIdx.x * kEmbedWarps + (threadIdx.x >> 5);
   const int64_t nwarps = (int64_t)gridDim.x * kEmbedWarps;
@@ -208,7 +263,7 @@ __global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
     for (int64_t base = 0; base < L; base += 32)
       cnt += accumulate_chunk<NCH, EXPLICIT_W, UNROLL, WIDE>(acc, lane_base, V, row_bytes, tail, wsrc, row_ids,
                                                              row_w, base, L, lane, bad);
-    store_row<NCH>(emb4 + (size_t)i * d4, acc, cnt, lane, d4);
+    finish_row<E, NCH>(emb4, i, acc, cnt, lane, d4, pc4, npc);
   }
   if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, MMB_STATUS_BAD_INDEX);
 }
@@ -248,11 +303,12 @@ __global__ void __launch_bounds__(256)
   if (zero && lane == 0) atomicOr(flags, 1);
 }
 
-template <int NCH, int UNROLL, int MINB>
+template <int NCH, int UNROLL, int MINB, Epi E = Epi::kPlain>
 __global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
     sif_embed_prescaled_kernel(const float4* __restrict__ tp4, int V, int d4, const int* __restrict__ flags,
-                               const int64_t* __restrict__ ids, int64_t N, int64_t L, float4* __restrict__ emb4,
-                               int* __restrict__ status) {
+                               const int64_t* __restrict__ ids, int64_t N, int64_t L,
+                               typename EpiOut<E>::type* __restrict__ emb4, int* __restrict__ status,
+                               const float4* __restrict__ pc4 = nullptr, int npc = 0) {
   if (__ldg(flags) & 1) return;        // a zero vocabulary weight: the general kernel behind this one runs
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = (int64_t)blockIdx.x * kEmbedWarps + (threadIdx.x >> 5);
@@ -318,7 +374,7 @@ __global__ void __launch_bounds__(kEmbedWarps * 32, MINB)
         }
       }
     }
-    store_row<NCH>(emb4 + (size_t)i * d4, acc, cnt, lane, d4);
+    finish_row<E, NCH>(emb4, i, acc, cnt, lane, d4, pc4, npc);
   }
   if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, MMB_STATUS_BAD_INDEX);
 }
@@ -461,12 +517,16 @@ __global__ void __launch_bounds__(1024)
 // order, so the result is still deterministic.
 // With `offsets` (ragged ids, see sif_embed_ragged_kernel) utterance i is ids[offsets[i] .. offsets[i+1]) followed
 // by L - length copies of pad_id, whose closed-form term warp 0 adds.
-template <int NCH, bool EXPLICIT_W>
-__global__ void __launch_bounds__(kEmbedWarps * 32)
+// Projecting epilogue: the summed row goes back to part[0] and warp 0 reads it in the warp kernels' lane + 32 c
+// layout, so that the dot products run in remove_pc's order (the CTA's own thread layout would change it).
+template <int NCH, bool EXPLICIT_W, Epi E = Epi::kPlain>
+__global__ void __launch_bounds__(kEmbedWarps * 32, cta_minb(E, NCH))
     sif_embed_cta_kernel(const float4* __restrict__ table4, int V, int d4,
                          const float* __restrict__ wsrc, const int64_t* __restrict__ ids, int64_t N,
-                         int64_t L, float4* __restrict__ emb4, int* __restrict__ status,
-                         const int64_t* __restrict__ offsets = nullptr, int64_t pad_id = 0) {
+                         int64_t L, typename EpiOut<E>::type* __restrict__ emb4, int* __restrict__ status,
+                         const int64_t* __restrict__ offsets = nullptr, int64_t pad_id = 0,
+                         const float4* __restrict__ pc4 = nullptr, int npc = 0) {
+  static_assert(E == Epi::kPlain || !EXPLICIT_W, "the projecting epilogue serves the fused-lookup embed only");
   __shared__ float4 part[kEmbedWarps][NCH * 32];
   __shared__ int part_cnt[kEmbedWarps];
   const int lane = threadIdx.x & 31;
@@ -523,25 +583,54 @@ __global__ void __launch_bounds__(kEmbedWarps * 32)
       }
       s.x = __fdiv_rn(s.x, div); s.y = __fdiv_rn(s.y, div);
       s.z = __fdiv_rn(s.z, div); s.w = __fdiv_rn(s.w, div);
-      st_stream(emb4 + (size_t)i * d4 + k, s);
+      if constexpr (E == Epi::kPlain) st_stream(emb4 + (size_t)i * d4 + k, s);
+      else part[0][k] = s;           // only this thread reads or writes column k of part[] in this loop
+    }
+    if constexpr (E != Epi::kPlain) {
+      __syncthreads();
+      if (warp == 0) {
+        float4 x[NCH];
+#pragma unroll
+        for (int c = 0; c < NCH; ++c)
+          x[c] = lane + 32 * c < d4 ? part[0][lane + 32 * c] : make_float4(0.f, 0.f, 0.f, 0.f);
+        subtract_pcs_inplace<NCH>(x, pc4, npc, d4, lane);
+        store_row<NCH>(emb4, i, d4, lane, x);
+      }
     }
     __syncthreads();
   }
   if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, MMB_STATUS_BAD_INDEX);
 }
 
-template <int NCH, bool EXPLICIT_W>
+// " +pc f32" / " +pc f64" after the kernel name of a projecting instantiation (mmb_last_kernel(0))
+template <Epi E>
+static void note_embed(char (&kname)[96]) {
+  if constexpr (E != Epi::kPlain)
+    strncat(kname, E == Epi::kProjF32 ? " +pc f32" : " +pc f64", sizeof(kname) - strlen(kname) - 1);
+  note_kernel(0, kname);
+}
+
+// The variant (CTA per utterance or warp per utterance) is decided on N_total, the batch that N rows are a chunk
+// of, so that every chunk of a chunked call runs the kernel the whole batch would.
+template <int NCH, bool EXPLICIT_W, Epi E = Epi::kPlain>
 static int launch_embed(const float* table, int64_t V, int d, const float* wsrc, const int64_t* ids,
-                        int64_t N, int64_t L, float* emb, int* status, cudaStream_t st) {
+                        int64_t N, int64_t L, void* emb, int* status, cudaStream_t st, int64_t N_total,
+                        const float* pc = nullptr, int npc = 0) {
+  typedef typename EpiOut<E>::type OutV;
   const int sms = sm_count();
   const int d4 = d / 4;
-  const bool few_long = (L >= 256) && (N < (int64_t)sms * 16);
+  const bool few_long = (L >= 256) && (N_total < (int64_t)sms * 16);
+  const float4* pc4 = (const float4*)pc;
   char kname[96] = "";
   if (few_long) {
     snprintf(kname, sizeof(kname), "sif_embed_cta_kernel<%d,%s>", NCH, EXPLICIT_W ? "true" : "false");
     int grid = (int)(N < (int64_t)sms * 8 ? N : (int64_t)sms * 8);
-    sif_embed_cta_kernel<NCH, EXPLICIT_W><<<grid, kEmbedWarps * 32, 0, st>>>(
-        (const float4*)table, (int)V, d4, wsrc, ids, N, L, (float4*)emb, status);
+    if constexpr (E == Epi::kPlain)
+      sif_embed_cta_kernel<NCH, EXPLICIT_W><<<grid, kEmbedWarps * 32, 0, st>>>(
+          (const float4*)table, (int)V, d4, wsrc, ids, N, L, (float4*)emb, status);
+    else
+      sif_embed_cta_kernel<NCH, EXPLICIT_W, E><<<grid, kEmbedWarps * 32, 0, st>>>(
+          (const float4*)table, (int)V, d4, wsrc, ids, N, L, (OutV*)emb, status, nullptr, 0, pc4, npc);
   } else {
     // Persistent-style grid: a multiple of the SM count, grid-stride over utterances.
     const int64_t blocks = ceil_div(N, kEmbedWarps);
@@ -552,8 +641,8 @@ static int launch_embed(const float* table, int64_t V, int d, const float* wsrc,
     const bool wide = (uint64_t)V * (uint64_t)d4 * 16u >= ((uint64_t)1 << 32);
 #define EMBED_LAUNCH(U, B, W)                                                                \
   do {                                                                                       \
-    sif_embed_warp_kernel<NCH, EXPLICIT_W, U, B, W><<<grid, kEmbedWarps * 32, 0, st>>>(      \
-        (const float4*)table, (int)V, d4, wsrc, ids, N, L, (float4*)emb, status);            \
+    sif_embed_warp_kernel<NCH, EXPLICIT_W, U, B, W, E><<<grid, kEmbedWarps * 32, 0, st>>>(   \
+        (const float4*)table, (int)V, d4, wsrc, ids, N, L, (OutV*)emb, status, pc4, npc);    \
     snprintf(kname, sizeof(kname), "sif_embed_warp_kernel<%d,%s,%d,%d,%s>", NCH,             \
              EXPLICIT_W ? "true" : "false", U, B, W ? "true" : "false");                     \
   } while (0)
@@ -563,28 +652,28 @@ static int launch_embed(const float* table, int64_t V, int d, const float* wsrc,
       if (wide) EMBED_LAUNCH(1, 2, true);
       else EMBED_LAUNCH(1, 2, false);
     } else if (wide) {
-      EMBED_LAUNCH(2, 4, true);
+      EMBED_LAUNCH(2, wide_minb(E, NCH), true);
     } else if constexpr (!EXPLICIT_W) {
       // fused lookup: ids of the next chunk prefetched; measured on B200, 4 M utterances: 11.83 ms
       // without the prefetch -> 11.56 ms; also prefetching the next chunk's weight lookups (two chunks
       // ahead) spills at the 64-register budget and takes 16.5 ms -- not kept
-      sif_embed_warp_prefetch_kernel<NCH, 2, 4><<<grid, kEmbedWarps * 32, 0, st>>>(
-          (const float4*)table, (int)V, d4, wsrc, ids, N, L, (float4*)emb, status);
-      snprintf(kname, sizeof(kname), "sif_embed_warp_prefetch_kernel<%d,2,4>", NCH);
+      sif_embed_warp_prefetch_kernel<NCH, 2, prefetch_minb(E, NCH), E><<<grid, kEmbedWarps * 32, 0, st>>>(
+          (const float4*)table, (int)V, d4, wsrc, ids, N, L, (OutV*)emb, status, nullptr, pc4, npc);
+      snprintf(kname, sizeof(kname), "sif_embed_warp_prefetch_kernel<%d,2,%d>", NCH, prefetch_minb(E, NCH));
     } else {
       EMBED_LAUNCH(2, 4, false);
     }
 #undef EMBED_LAUNCH
   }
   MMB_LAUNCH_CHECK("sif_embed");
-  note_kernel(0, kname);
+  note_embed<E>(kname);
   return MMB_OK;
 }
 
-template <bool EXPLICIT_W>
+template <bool EXPLICIT_W, Epi E = Epi::kPlain>
 static int dispatch_embed(const float* table, int64_t V, int d, const float* wsrc,
-                          const int64_t* ids, int64_t N, int64_t L, float* emb, int* status,
-                          cudaStream_t st) {
+                          const int64_t* ids, int64_t N, int64_t L, void* emb, int* status,
+                          cudaStream_t st, int64_t N_total, const float* pc = nullptr, int npc = 0) {
   MMB_REQUIRE(d > 0 && d % 4 == 0 && d <= 1024, "d must be a multiple of 4, <= 1024");
   MMB_REQUIRE(V > 0 && V < (int64_t)1 << 31, "V out of range");
   MMB_REQUIRE(N >= 0 && L >= 0, "negative size");
@@ -594,11 +683,11 @@ static int dispatch_embed(const float* table, int64_t V, int d, const float* wsr
   if (N == 0) return MMB_OK;
   const int nch = (d / 4 + 31) / 32;
   switch (nch) {
-    case 1: return launch_embed<1, EXPLICIT_W>(table, V, d, wsrc, ids, N, L, emb, status, st);
-    case 2: return launch_embed<2, EXPLICIT_W>(table, V, d, wsrc, ids, N, L, emb, status, st);
-    case 3: return launch_embed<3, EXPLICIT_W>(table, V, d, wsrc, ids, N, L, emb, status, st);
-    case 4: return launch_embed<4, EXPLICIT_W>(table, V, d, wsrc, ids, N, L, emb, status, st);
-    default: return launch_embed<8, EXPLICIT_W>(table, V, d, wsrc, ids, N, L, emb, status, st);
+    case 1: return launch_embed<1, EXPLICIT_W, E>(table, V, d, wsrc, ids, N, L, emb, status, st, N_total, pc, npc);
+    case 2: return launch_embed<2, EXPLICIT_W, E>(table, V, d, wsrc, ids, N, L, emb, status, st, N_total, pc, npc);
+    case 3: return launch_embed<3, EXPLICIT_W, E>(table, V, d, wsrc, ids, N, L, emb, status, st, N_total, pc, npc);
+    case 4: return launch_embed<4, EXPLICIT_W, E>(table, V, d, wsrc, ids, N, L, emb, status, st, N_total, pc, npc);
+    default: return launch_embed<8, EXPLICIT_W, E>(table, V, d, wsrc, ids, N, L, emb, status, st, N_total, pc, npc);
   }
 }
 
@@ -624,13 +713,13 @@ extern "C" int mmb_seq2weight(const int64_t* seq, const float* mask, const float
 extern "C" int mmb_weighted_average(const float* table, int64_t V, int d, const int64_t* x,
                                     const float* w, int64_t N, int64_t L, float* emb, int* status,
                                     mmb_stream_t stream) {
-  return dispatch_embed<true>(table, V, d, w, x, N, L, emb, status, as_stream(stream));
+  return dispatch_embed<true>(table, V, d, w, x, N, L, emb, status, as_stream(stream), N);
 }
 
 extern "C" int mmb_sif_embed(const float* table, int64_t V, int d, const float* vocab_w,
                              const int64_t* x, int64_t N, int64_t L, float* emb, int* status,
                              mmb_stream_t stream) {
-  return dispatch_embed<false>(table, V, d, vocab_w, x, N, L, emb, status, as_stream(stream));
+  return dispatch_embed<false>(table, V, d, vocab_w, x, N, L, emb, status, as_stream(stream), N);
 }
 
 // ---- ragged (CSR) ids, SURVEY.md 8f N3 -----------------------------------------------------------------
@@ -720,24 +809,29 @@ int sif_prescale(const float* table, int64_t V, int d, const float* vocab_w, voi
 }
 
 // The embed pass on a pre-scaled table (ws from sif_prescale) with the general kernel standing by.
-int sif_embed_prescaled(const float* table, int64_t V, int d, const float* vocab_w, const void* ws, const int64_t* x,
-                        int64_t N, int64_t L, float* emb, int* status, cudaStream_t st) {
+template <Epi E = Epi::kPlain>
+static int embed_prescaled(const float* table, int64_t V, int d, const float* vocab_w, const void* ws,
+                           const int64_t* x, int64_t N, int64_t L, void* emb, int* status, cudaStream_t st,
+                           const float* pc = nullptr, int npc = 0) {
+  typedef typename EpiOut<E>::type OutV;
   if (N == 0) return MMB_OK;
   const int d4 = d / 4;
   const int* flags = (const int*)ws;
   const float4* tp4 = (const float4*)((const char*)ws + 256);
+  const float4* pc4 = (const float4*)pc;
   const int sms = sm_count();
   const int64_t blocks = ceil_div(N, kEmbedWarps);
   const int grid = (int)(blocks < (int64_t)sms * 8 ? blocks : (int64_t)sms * 8);
+  char kname[96] = "";
 #define PRESCALED_LAUNCH(NCH)                                                                                  \
   do {                                                                                                         \
-    sif_embed_prescaled_kernel<NCH, 2, 4><<<grid, kEmbedWarps * 32, 0, st>>>(tp4, (int)V, d4, flags, x, N, L,  \
-                                                                             (float4*)emb, status);            \
+    sif_embed_prescaled_kernel<NCH, 2, prescaled_minb(E, NCH), E><<<grid, kEmbedWarps * 32, 0, st>>>(          \
+        tp4, (int)V, d4, flags, x, N, L, (OutV*)emb, status, pc4, npc);                                        \
     MMB_LAUNCH_CHECK("sif_embed_prescaled");                                                                   \
-    sif_embed_warp_prefetch_kernel<NCH, 2, 4><<<grid, kEmbedWarps * 32, 0, st>>>(                              \
-        (const float4*)table, (int)V, d4, vocab_w, x, N, L, (float4*)emb, status, flags);                      \
+    sif_embed_warp_prefetch_kernel<NCH, 2, prefetch_minb(E, NCH), E><<<grid, kEmbedWarps * 32, 0, st>>>(       \
+        (const float4*)table, (int)V, d4, vocab_w, x, N, L, (OutV*)emb, status, flags, pc4, npc);              \
     MMB_LAUNCH_CHECK("sif_embed_general_standby");                                                             \
-    note_kernel(0, "sif_embed_prescaled_kernel<" #NCH ",2,4>");                                               \
+    snprintf(kname, sizeof(kname), "sif_embed_prescaled_kernel<%d,2,%d>", NCH, prescaled_minb(E, NCH));       \
   } while (0)
   switch ((d4 + 31) / 32) {
     case 1: PRESCALED_LAUNCH(1); break;
@@ -746,7 +840,43 @@ int sif_embed_prescaled(const float* table, int64_t V, int d, const float* vocab
     default: PRESCALED_LAUNCH(4); break;
   }
 #undef PRESCALED_LAUNCH
+  note_embed<E>(kname);
   return MMB_OK;
+}
+
+int sif_embed_prescaled(const float* table, int64_t V, int d, const float* vocab_w, const void* ws, const int64_t* x,
+                        int64_t N, int64_t L, float* emb, int* status, cudaStream_t st) {
+  return embed_prescaled(table, V, d, vocab_w, ws, x, N, L, emb, status, st);
+}
+
+static int check_pc(const float* pc, int npc) {
+  MMB_REQUIRE(npc >= 0 && npc <= 32, "npc must be in [0, 32]");
+  MMB_REQUIRE(pc || npc == 0, "null pointer");
+  MMB_REQUIRE((uintptr_t)pc % 16 == 0, "pc must be 16-byte aligned");
+  return MMB_OK;
+}
+
+// mmb_sif_transform on N rows of a batch of N_total: the embed with the projection on npc given components (npc x d
+// float32 on the device) as its epilogue, out (N, d) float32, or float64 when f64.  scaled: the pre-scaled table of
+// sif_prescale for the whole batch, or NULL for the general kernels.
+int sif_transform_chunk(const float* table, int64_t V, int d, const float* vocab_w, const void* scaled,
+                        const int64_t* x, int64_t N, int64_t L, int64_t N_total, const float* pc, int npc, void* out,
+                        bool f64, int* status, cudaStream_t st) {
+  if (int rc = check_pc(pc, npc)) return rc;
+  if (scaled) {
+    if (N == 0) return MMB_OK;
+    MMB_REQUIRE(table && vocab_w && x && out && status, "null pointer");
+    MMB_REQUIRE(((uintptr_t)table % 16 == 0) && ((uintptr_t)out % 16 == 0) && ((uintptr_t)scaled % 16 == 0),
+                "table / out / ws must be 16-byte aligned");
+    if (f64) return embed_prescaled<Epi::kProjF64>(table, V, d, vocab_w, scaled, x, N, L, out, status, st, pc, npc);
+    if (npc) return embed_prescaled<Epi::kProjF32>(table, V, d, vocab_w, scaled, x, N, L, out, status, st, pc, npc);
+    return embed_prescaled(table, V, d, vocab_w, scaled, x, N, L, out, status, st);
+  }
+  if (f64)
+    return dispatch_embed<false, Epi::kProjF64>(table, V, d, vocab_w, x, N, L, out, status, st, N_total, pc, npc);
+  if (npc)
+    return dispatch_embed<false, Epi::kProjF32>(table, V, d, vocab_w, x, N, L, out, status, st, N_total, pc, npc);
+  return dispatch_embed<false>(table, V, d, vocab_w, x, N, L, out, status, st, N_total);
 }
 }  // namespace mmb
 
@@ -762,4 +892,20 @@ extern "C" int mmb_sif_embed_ws(const float* table, int64_t V, int d, const floa
   int rc = sif_prescale(table, V, d, vocab_w, ws, as_stream(stream));
   if (rc) return rc;
   return sif_embed_prescaled(table, V, d, vocab_w, ws, x, N, L, emb, status, as_stream(stream));
+}
+
+extern "C" int mmb_sif_transform(const float* table, int64_t V, int d, const float* vocab_w, const int64_t* x,
+                                 int64_t N, int64_t L, const float* pc, int npc, float* out, int* status, void* ws,
+                                 size_t ws_bytes, mmb_stream_t stream) {
+  cudaStream_t st = as_stream(stream);
+  const size_t need = mmb_sif_embed_workspace_bytes(V, d, N, L);
+  const bool scaled = need != 0 && ws != nullptr && ws_bytes >= need && N > 0;
+  if (int rc = check_pc(pc, npc)) return rc;
+  if (scaled) {
+    MMB_REQUIRE(table && vocab_w && (uintptr_t)table % 16 == 0 && (uintptr_t)ws % 16 == 0,
+                "table / ws must be non-null and 16-byte aligned");
+    const int rc = sif_prescale(table, V, d, vocab_w, ws, st);
+    if (rc) return rc;
+  }
+  return sif_transform_chunk(table, V, d, vocab_w, scaled ? ws : nullptr, x, N, L, N, pc, npc, out, false, status, st);
 }

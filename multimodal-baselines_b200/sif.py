@@ -4,7 +4,9 @@ simplesif.py:296-311).  The embedding itself runs through ``mmb_sif_embedding_ho
 ``mmb_sif_embedding`` of libmmb_b200.so.  ``get_sentence_embeddings_sweep`` (no reference counterpart) does the
 same for K word-weight vectors and several numbers of removed components in one gather
 (``mmb_sif_embedding_sweep_host`` for NumPy ids; ``mmb_sif_embed_multi`` / ``mmb_sif_embed_multi_ragged`` for ids
-on the device).
+on the device).  ``fit_sentence_components`` and ``transform_sentence_embeddings`` split the same call into
+TruncatedSVD's fit and transform: components fitted on one set of utterances (``mmb_sif_fit_host``), then removed
+from the embeddings of any other (``mmb_sif_transform_host`` / ``mmb_sif_transform``, one fused pass).
 """
 import ctypes as C
 import os
@@ -15,6 +17,7 @@ import torch
 import _native as nv
 from _native import lib
 from sif_functions import Params, seq2weight, SIF_embedding, start_block, sif_embedding_device  # noqa: F401
+from sif_functions import sif_transform_device  # noqa: F401
 from sif_functions import sif_embedding_sweep, sweep_npcs  # noqa: F401
 from sif_functions import RaggedIds, sif_embedding_ragged, to_ragged  # noqa: F401
 
@@ -94,6 +97,29 @@ def get_sentence_word_weights(text, weights):
     return seq2weight(text, np.ones(np.shape(text)), weights)
 
 
+def _prepare(word_embeddings, weights, text, dev):
+    """``(table_t, w_t, ids)`` for the single-vector calls: the table and the weight vector as float32 CUDA tensors,
+    and the ids as they came, a C-contiguous int64 NumPy array or a contiguous CUDA tensor, either (N, L).  A weight
+    vector shorter than the table is padded with zeros; an id beyond it raises ``IndexError``, as NumPy's
+    ``weights[ids]`` would."""
+    if isinstance(text, torch.Tensor) and text.is_cuda:
+        ids = text.contiguous()
+    else:
+        ids = np.ascontiguousarray(np.asarray(text), dtype=np.int64)
+    if ids.ndim != 2:
+        raise ValueError('text must be (n_samples, seq_len)')
+    table_t = nv.to_device(word_embeddings, torch.float32, dev)
+    w_t = nv.to_device(weights if isinstance(weights, torch.Tensor) else np.asarray(weights).reshape(-1),
+                       torch.float32, dev).reshape(-1)
+    V = table_t.shape[0]
+    if w_t.numel() < V:
+        id_max = int(ids.max()) if ids.shape[0] * ids.shape[1] else None     # only here: a pass over the ids
+        if id_max is not None and id_max >= w_t.numel():
+            raise IndexError('index %d is out of bounds for axis 0 with size %d' % (id_max, w_t.numel()))
+        w_t = torch.cat([w_t, w_t.new_zeros(V - w_t.numel())])
+    return table_t, w_t, ids
+
+
 def get_sentence_embeddings(word_embeddings, weights, text, out=None):
     """reference sif.py:84-94 -- SIF embedding of every utterance with the first principal
     component removed (``RMPC = 1``, line 88).
@@ -114,17 +140,9 @@ def get_sentence_embeddings(word_embeddings, weights, text, out=None):
         w_t = nv.to_device(weights, torch.float32, dev).reshape(-1)
         return sif_embedding_device(table_t, w_t, text.contiguous(), npc=RMPC)
 
-    ids = np.ascontiguousarray(np.asarray(text), dtype=np.int64)
-    if ids.ndim != 2:
-        raise ValueError('text must be (n_samples, seq_len)')
+    table_t, w_t, ids = _prepare(word_embeddings, weights, text, dev)
     n, L = ids.shape
-    table_t = nv.to_device(word_embeddings, torch.float32, dev)
-    w_t = nv.to_device(np.asarray(weights).reshape(-1), torch.float32, dev)
     V, d = table_t.shape
-    if w_t.numel() < V:
-        if ids.size and ids.max() >= w_t.numel():
-            raise IndexError('index %d is out of bounds for axis 0 with size %d' % (ids.max(), w_t.numel()))
-        w_t = torch.cat([w_t, w_t.new_zeros(V - w_t.numel())])
     if out is None:
         out = np.empty((n, d), dtype=np.float64)
     assert out.shape == (n, d) and out.flags['C_CONTIGUOUS'] and out.dtype in (np.float64, np.float32)
@@ -204,4 +222,69 @@ def get_sentence_embeddings_sweep(word_embeddings, weights, text, npcs=(1,), out
     nv.check(lib.mmb_sif_embedding_sweep_host(nv.ptr(table_t), V, d, nv.ptr(W_t), K, nv.np_ptr(ids), n, L, P,
                                               (C.c_int * P)(*npcs), omega_arr, nv.np_ptr(out),
                                               int(out.dtype == np.float64), nv.GRAM_AUTO, 0))
+    return out
+
+
+def fit_sentence_components(word_embeddings, weights, text, npc=1):
+    """The first half of ``get_sentence_embeddings`` as an estimator's fit: the ``npc`` principal components
+    (reference sif_functions.py:58-67, ``TruncatedSVD.fit``) of the SIF embeddings of ``text``, for
+    ``transform_sentence_embeddings`` to remove from these or any other utterances' embeddings.
+
+    NumPy ids -> float64 (npc, d) NumPy array, like ``compute_pc`` (``mmb_sif_fit_host``: the ids stream to the
+    device in chunks and only the Gram stays there, so N is not bounded by device memory); CUDA ids -> the float32
+    (npc, d) CUDA tensor ``mmb_sif_embedding`` computes.  npc in 1..22."""
+    dev = nv.require_cuda()
+    if isinstance(text, RaggedIds):
+        raise ValueError('fit_sentence_components takes padded (N, L) ids, not RaggedIds')
+    npc = int(npc)
+    if npc < 1 or npc + 10 > 32:
+        raise ValueError('npc must be in 1..22')
+    table_t, w_t, ids = _prepare(word_embeddings, weights, text, dev)
+    n, L = ids.shape
+    V, d = table_t.shape
+    if n == 0:
+        raise ValueError('fitting components needs at least one utterance')
+    if isinstance(ids, torch.Tensor):
+        return sif_embedding_device(table_t, w_t, ids, npc=npc, return_pc=True)[1]
+    omega = np.ascontiguousarray(start_block(d if n >= d else n, npc))
+    pc = np.empty((npc, d), dtype=np.float32)
+    torch.cuda.current_stream().synchronize()      # table / weights uploads are done
+    nv.check(lib.mmb_sif_fit_host(nv.ptr(table_t), V, d, nv.ptr(w_t), nv.np_ptr(ids), n, L, npc, nv.np_ptr(omega),
+                                  nv.np_ptr(pc), nv.GRAM_AUTO, 0))
+    return pc.astype(np.float64)
+
+
+def transform_sentence_embeddings(word_embeddings, weights, text, components, out=None):
+    """The second half of ``get_sentence_embeddings`` as an estimator's transform: the SIF embedding of every
+    utterance of ``text`` minus its projection on ``components`` (reference sif_functions.py:69-81 with the
+    components given), embedded and projected in one pass.  ``components`` is a float32 or float64 (npc, d) array
+    or tensor, npc in 0..32 (0: the plain weighted average), rounded to float32 -- exact for what
+    ``fit_sentence_components`` returns, so ``transform_sentence_embeddings(We, w, X,
+    fit_sentence_components(We, w, X))`` is ``get_sentence_embeddings(We, w, X)`` bit for bit.
+
+    NumPy ids -> float64 (N, d) NumPy out (``mmb_sif_transform_host``: ids in, embedding and D2H overlap chunk by
+    chunk, and nothing of size N is kept on the device).  ``out`` may be a preallocated C-contiguous (N, d) float64
+    or float32 host array (e.g. ``_native.PinnedArray(...).array``, for full PCIe rate); it is filled and returned.
+    CUDA ids -> float32 (N, d) CUDA tensor (``sif_functions.sif_transform_device``)."""
+    dev = nv.require_cuda()
+    if isinstance(text, RaggedIds):
+        raise ValueError('transform_sentence_embeddings takes padded (N, L) ids, not RaggedIds')
+    table_t, w_t, ids = _prepare(word_embeddings, weights, text, dev)
+    n, L = ids.shape
+    V, d = table_t.shape
+    pc_t = nv.to_device(components, torch.float32, dev)
+    if pc_t.dim() != 2 or pc_t.shape[1] != d or pc_t.shape[0] > 32:
+        raise ValueError('components must be (npc, %d) with npc in 0..32, got %s' % (d, tuple(pc_t.shape)))
+    if isinstance(ids, torch.Tensor):
+        if out is not None:
+            raise ValueError('out= takes host ids; with CUDA ids the result is a CUDA tensor')
+        return sif_transform_device(table_t, w_t, ids, pc_t)
+    if out is None:
+        out = np.empty((n, d), dtype=np.float64)
+    if tuple(out.shape) != (n, d) or not out.flags['C_CONTIGUOUS'] or out.dtype not in (np.float64, np.float32):
+        raise ValueError('out must be a C-contiguous (%d, %d) float64 or float32 array' % (n, d))
+    pc = pc_t.cpu().numpy()
+    torch.cuda.current_stream().synchronize()      # table / weights uploads are done
+    nv.check(lib.mmb_sif_transform_host(nv.ptr(table_t), V, d, nv.ptr(w_t), nv.np_ptr(ids), n, L, nv.np_ptr(pc),
+                                        pc.shape[0], nv.np_ptr(out), int(out.dtype == np.float64), 0))
     return out

@@ -21,7 +21,8 @@ from _native import lib
 
 __all__ = ['seq2weight', 'Params', 'get_weighted_average', 'compute_pc', 'remove_pc',
            'SIF_embedding', 'start_block', 'gram', 'pc_from_gram', 'project_out',
-           'sif_embedding_device', 'sif_embedding_sweep', 'RaggedIds', 'to_ragged', 'sif_embedding_ragged']
+           'sif_embedding_device', 'sif_transform_device', 'sif_embedding_sweep', 'RaggedIds', 'to_ragged',
+           'sif_embedding_ragged']
 
 
 def _is_np(*xs):
@@ -244,6 +245,30 @@ def sif_embedding_device(table_t, vocab_w_t, ids_t, npc=1, gram_mode=nv.GRAM_AUT
     if check:
         nv.raise_on_status(st, V)
     return (emb, pc) if return_pc else emb
+
+
+def sif_transform_device(table_t, vocab_w_t, ids_t, pc_t, out=None, check=True):
+    """The SIF embedding with GIVEN components (``mmb_sif_transform``): embed and remove the projection on ``pc_t``
+    in one pass, bit for bit ``mmb_sif_embed_ws`` followed by ``project_out``.  All arguments are CUDA tensors:
+    table (V, d) f32, vocab_w (V,) f32, ids (N, L) int64, pc (npc, d) f32 with npc in 0..32 (0: the plain embed).
+    The pre-scale workspace is sized as in ``sif_embedding_device``, so both run the same embed kernel.  Returns
+    ``out``, an (N, d) float32 CUDA tensor."""
+    n, L = ids_t.shape
+    V, d = table_t.shape
+    npc = pc_t.shape[0]
+    dev = table_t.device
+    if out is None:
+        out = torch.empty((n, d), dtype=torch.float32, device=dev)
+    elif tuple(out.shape) != (n, d) or out.dtype != torch.float32 or out.device != dev or not out.is_contiguous():
+        raise ValueError('out must be a contiguous (%d, %d) float32 tensor on %s' % (n, d, dev))
+    st = _status(dev)
+    nbytes = lib.mmb_sif_embed_workspace_bytes(V, d, n, L)     # large batches: scratch for the pre-scaled table
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=dev) if nbytes else None
+    nv.check(lib.mmb_sif_transform(nv.ptr(table_t), V, d, nv.ptr(vocab_w_t), nv.ptr(ids_t), n, L, nv.ptr(pc_t), npc,
+                                   nv.ptr(out), nv.ptr(st), nv.ptr(ws), nbytes, nv.stream_ptr()))
+    if check:
+        nv.raise_on_status(st, V)
+    return out
 
 
 def sweep_npcs(npcs):
